@@ -29,6 +29,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the benchmark writes nothing into the tree it runs from (which may be read-only)
 # This script's stdout is ONE JSON line.  Libraries write to file descriptor 1 behind Python's back (NCCL prints its version
 # banner there at VERSION level, whatever the environment says), so descriptor 1 is pointed at stderr for the whole run
 # and the line goes to a private copy of the original stdout.
@@ -419,6 +420,30 @@ def plane_crcs(planes):
     return [zlib.crc32(np.ascontiguousarray(p).tobytes()) for p in planes]
 
 
+DUMP_BYTES = 64 * 10**6
+
+
+def dump_outputs(f, num_slots, width, height, out_dir):
+    """Write the filtered pictures of slots [0, num_slots) as out_dir/{y,cb,cr}.npy, float32 [slot, row, column].  Whole
+    pictures when all of them fit in DUMP_BYTES; otherwise the same seeded sample of chroma rows of every picture, with the two
+    luma rows of each, so that two builds run with the same arguments can be compared sample for sample."""
+    bytes_per_chroma_row = 4 * (2 * width + 2 * (width // 2))
+    n = min(height // 2, (DUMP_BYTES - 4096) // (bytes_per_chroma_row * num_slots))
+    if n < 1:
+        raise SystemExit(f"bench.py: {num_slots} pictures of {width}x{height} do not fit --dump-outputs' {DUMP_BYTES} bytes")
+    rows = np.sort(np.random.default_rng(0).choice(height // 2, n, replace=False))
+    luma_rows = np.stack([2 * rows, 2 * rows + 1], axis=1).reshape(-1)
+    out = {"y": [], "cb": [], "cr": []}
+    for s in range(num_slots):
+        pic = f.download(s)
+        out["y"].append(pic["y"][luma_rows].astype(np.float32))
+        out["cb"].append(pic["cb"][rows].astype(np.float32))
+        out["cr"].append(pic["cr"][rows].astype(np.float32))
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in out.items():
+        np.save(os.path.join(out_dir, k + ".npy"), np.stack(a))
+
+
 def bands_record(args, wl, rank, world, local, dist, torch, v):
     """BASELINE config 4: every rank owns a band of CTU rows of ONE picture (vvcsoftware_vtm_b200.bands), uploads its own rows,
     pulls 16 halo rows per side from its neighbours' input planes (CUDA IPC mapping, device-to-device over NVLink P2P, one copy
@@ -432,7 +457,7 @@ def bands_record(args, wl, rank, world, local, dist, torch, v):
     side = load_sideinfo("intra_8k_bands")
     side_on = all_on_sideinfo(side)
     B = args.bands_batch
-    steps = max(3, min(args.steps, 20))
+    steps = args.steps
     f = bands.make_band_context(w, h, 10, 10, 7, rank, world, local, num_slots=B)
     y0, y1 = f.own_row0, f.own_row0 + f.own_rows
     # synthetic planes: a 4K texture tiled 2 x 2 (every rank builds the picture and keeps its own rows)
@@ -620,7 +645,7 @@ def streams_record(args, rank, world, local, dist, torch, v):
     side = [pic for st in mine for pic in sets[st % len(sets)]]
     B = len(side)
     total_pics = sum(len(sets[st % len(sets)]) for st in range(wl["streams"]))
-    steps = max(3, min(args.steps, 20))
+    steps = args.steps
     planes = synth_planes(w, h, 4, seed=3000 + rank)
     f = v.InLoopFilter(w, h, 10, 10, 7, device=local, num_slots=B)
     pins = [[torch.from_numpy(np.ascontiguousarray(p)).pin_memory() for p in trip] for trip in planes]
@@ -792,6 +817,8 @@ def run_b200(args, wl):
     ms_on, kt_on, _, msi_on = measure(all_on_sideinfo(side), args.steps)      # worst case: every CTU filtered by every stage
     ms_total, ktimes, launches, msi_total = measure(side, args.steps)         # the stream's own decisions (headline)
     clk = clocks.finish()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(f, B, w, h, args.dump_outputs)   # before the encoder-statistics runs below overwrite the slots' results
     value = world * B * args.steps * mpx / (ms_total * 1e-3)
     value_on = world * B * args.steps * mpx / (ms_on * 1e-3)
 
@@ -820,7 +847,7 @@ def run_b200(args, wl):
         f.alf_stats(0, B)
     f.sync()
     f.set_timing(True)
-    for _ in range(max(3, args.steps // 4)):
+    for _ in range(args.steps):
         f.alf_stats(0, B)
     kt_alf_stats = f.kernel_times()["alf_stats"]
     f.set_timing(False)
@@ -957,9 +984,15 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--quick", action="store_true", help="kernel A/B runs: no CPU baseline, no drop-in leg, no bands_8k / streams_64 sub-records")
     ap.add_argument("--bands-batch", type=int, default=16, help="resident 8K pictures per step of the band configuration")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the filtered pictures of the last step as DIR/{y,cb,cr}.npy "
+                                                         "(float32 [picture, row, column]; a fixed sample of rows when the batch exceeds 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.workload = args.workload or default_workload()
     wl = WORKLOADS[args.workload]
+    if args.dump_outputs and (args.impl != "b200" or wl.get("bands")):
+        ap.error("--dump-outputs needs --impl b200 and a workload filtered as whole pictures")
     if args.impl == "reference":
         run_reference(args, wl)
     elif wl.get("bands"):
