@@ -260,6 +260,34 @@ int ilf_alf_stats(ilf_ctx* ctx, int first_slot, int num_slots);
 int ilf_get_alf_stats(ilf_ctx* ctx, int slot, int64_t* out);
 
 /* ---------------------------------------------------------------------------------------------
+ * Encoder deblocking parameter search on the device-resident picture (SURVEY.md 8f): serves
+ * EncGOP::applyDeblockingFilterParameterSelection (EncoderLib/EncGOP.cpp:2550-2574, switched on by DeblockingFilterMetric), which
+ * deblocks the same reconstruction once per (beta offset, tc offset) candidate and keeps the pair of least distortion
+ * (xFindDistortionFrame, :3970).  ilf_deblock_search scores K candidates of every slot in one pass that reads the picture and the
+ * original once and writes no picture; ilf_get_deblock_search copies a slot's K x 3 sums to the host:
+ *   out[k][c] = sum over the samples of plane c (Y, Cb, Cr) of ((D_k - O)^2 >> shift[c > 0])
+ * The shift applies to every sample, as xFindDistortionFrame does; the caller passes the reference's shift
+ * (DISTORTION_PRECISION_ADJUSTMENT of its bit depth).  O is the original of ilf_set_original.  D_k is exactly what ilf_deblock
+ * produces from the slot's UPLOADED picture with the slot's deblocking side information, the beta_offset_div2 / tc_offset_div2 of
+ * EVERY slice replaced by candidate k (the reference sets the same offsets on all slices, :2560-2566); chroma QP offsets,
+ * mv_threshold, ctu_slice, grids and motion stay as set.  Offsets are any int8_t; the table index clamps as in deblocking (:626-634).
+ * The search reads buffer 0, so stages run since the upload do not change its result, and it writes no picture plane:
+ * ilf_download / ilf_run after a search give what they gave before it.
+ * Errors: ILF_ERR_ARG for a bad slot range, num_cands outside 1..ILF_DEBLOCK_SEARCH_MAX, NULL pointers or a shift outside 0..31;
+ * ILF_ERR_STATE for a slot without an upload, without deblocking side information or without ilf_set_original since its upload,
+ * and on band contexts.  Ordering: the search waits for the slots' uploads and side information, runs on the context's stream and
+ * is waited for by the slots' next uploads.  ilf_get_deblock_search synchronises and returns the K of the slot's last search
+ * (ILF_ERR_STATE before any search, ILF_ERR_ARG when max_cands < K).
+ * ------------------------------------------------------------------------------------------- */
+typedef struct {
+  int8_t beta_offset_div2, tc_offset_div2;
+} ilf_deblock_candidate;
+#define ILF_DEBLOCK_SEARCH_MAX 64
+int ilf_deblock_search(ilf_ctx* ctx, int first_slot, int num_slots, const ilf_deblock_candidate* cands, int num_cands,
+                       const int32_t shift[2] /* luma, chroma */);
+int ilf_get_deblock_search(ilf_ctx* ctx, int slot, uint64_t* out /* [K][3] */, int max_cands);
+
+/* ---------------------------------------------------------------------------------------------
  * Post-filter consumers on the device-resident picture (SURVEY.md 8f): what the decoder does with a picture right after the
  * in-loop filters.
  *   ilf_picture_hash       the two decoded-picture-hash methods that are not inherently serial, calcCRC and calcChecksum

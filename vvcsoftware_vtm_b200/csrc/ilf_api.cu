@@ -100,6 +100,8 @@ struct Slot {
   long long* stats = nullptr;  // [num_ctus][3][5][64]
   long long* alf_stats = nullptr;  // [num_ctus][ILF_ALF_STATS_WORDS]
   bool has_org = false;
+  bool org_since_upload = false;   // ilf_set_original was called after the slot's last upload (ilf_deblock_search)
+  int search_k = 0;                // candidates of the slot's last ilf_deblock_search (0: none yet)
   int16_t* pinned = nullptr;   // host staging for pageable planes on the way up, one picture; allocated on first use
   int16_t* pinned_down = nullptr;  // ... and on the way down
   uint8_t* pinned_side = nullptr;  // host staging for side information
@@ -168,6 +170,7 @@ struct ilf_ctx {
   CopyPool copy_pool;
   uint32_t* hash_scratch = nullptr;   // ilf_picture_hash
   int* db_work = nullptr;             // tile queues of the deblocking kernel: two ints per stream (the compute stream, then the lanes)
+  unsigned long long* search_out = nullptr;   // ilf_deblock_search: [num_slots][ILF_DEBLOCK_SEARCH_MAX][3], allocated by the first search
   cudaEvent_t chunk_ev[COPY_CHUNKS_MAX] = {};   // download: chunk i has reached the staging buffer
 };
 
@@ -472,6 +475,7 @@ int ilf_destroy(ilf_ctx* ctx) {
   cudaFree(ctx->slots_dev);
   cudaFree(ctx->hash_scratch);
   cudaFree(ctx->db_work);
+  cudaFree(ctx->search_out);
   for (auto& t : ctx->timed) { cudaEventDestroy(t.a); cudaEventDestroy(t.b); }
   for (cudaEvent_t e : ctx->free_events) cudaEventDestroy(e);
   for (cudaStream_t st : {ctx->s_up, ctx->stream, ctx->s_down, ctx->lane[0], ctx->lane[1], ctx->lane[2], ctx->lane[3]}) if (st) cudaStreamDestroy(st);
@@ -569,6 +573,7 @@ static int upload_rows(ilf_ctx* ctx, int slot, const int16_t* y, ptrdiff_t sy, c
   s.h2d_pending = true;
   s.uploaded = true;
   s.has_db = s.has_sao = s.has_alf = false;
+  s.org_since_upload = false;
   s.result_buf[0] = s.result_buf[1] = s.result_buf[2] = 0;
   return ILF_OK;
 }
@@ -1254,6 +1259,7 @@ int ilf_set_original(ilf_ctx* ctx, int slot, const int16_t* y, ptrdiff_t sy, con
   CU(ctx, cudaMemcpyAsync(s.stats_avail, ctu_avail, ctx->num_ctus, cudaMemcpyHostToDevice, ctx->s_up));
   if (!is_pinned(ctu_avail)) CU(ctx, cudaStreamSynchronize(ctx->s_up));  // the caller may reuse ctu_avail
   s.has_org = true;
+  s.org_since_upload = true;
   return push_desc(ctx, slot);
 }
 
@@ -1353,6 +1359,70 @@ int ilf_get_alf_stats(ilf_ctx* ctx, int slot, int64_t* out) {
   return ILF_OK;
 }
 
+// ---------------------------------------------------------------------------------------------------------------
+// Encoder deblocking parameter search (include/ilf_b200.h; EncGOP::applyDeblockingFilterParameterSelection)
+// ---------------------------------------------------------------------------------------------------------------
+int ilf_deblock_search(ilf_ctx* ctx, int first_slot, int num_slots, const ilf_deblock_candidate* cands, int num_cands, const int32_t shift[2]) {
+  if (!ctx) return ILF_ERR_ARG;
+  if (first_slot < 0 || num_slots < 1 || first_slot + num_slots > (int)ctx->slots.size()) return fail(ctx, ILF_ERR_ARG, "slot range [%d,+%d) out of range", first_slot, num_slots);
+  if (!cands || !shift) return fail(ctx, ILF_ERR_ARG, "null pointer");
+  if (num_cands < 1 || num_cands > ILF_DEBLOCK_SEARCH_MAX) return fail(ctx, ILF_ERR_ARG, "num_cands %d outside 1..%d", num_cands, ILF_DEBLOCK_SEARCH_MAX);
+  if (shift[0] < 0 || shift[0] > 31 || shift[1] < 0 || shift[1] > 31) return fail(ctx, ILF_ERR_ARG, "shift (%d, %d) outside 0..31", shift[0], shift[1]);
+  if (ctx->is_band) return fail(ctx, ILF_ERR_STATE, "not available on band contexts");
+  for (int i = first_slot; i < first_slot + num_slots; i++) {
+    const Slot& s = ctx->slots[i];
+    if (!s.uploaded || !s.has_db || !s.org_since_upload)
+      return fail(ctx, ILF_ERR_STATE, "slot %d: the search needs ilf_upload, then ilf_set_deblock_info and ilf_set_original", i);
+  }
+  CU(ctx, cudaSetDevice(ctx->cfg.device));
+  constexpr size_t ROW = (size_t)ILF_DEBLOCK_SEARCH_MAX * 3;
+  if (!ctx->search_out) CU(ctx, cudaMalloc(&ctx->search_out, ctx->slots.size() * ROW * sizeof(unsigned long long)));
+  for (int i = first_slot; i < first_slot + num_slots; i++) {
+    Slot& s = ctx->slots[i];
+    if (s.h2d_pending) { CU(ctx, cudaStreamWaitEvent(ctx->stream, s.ev_up, 0)); s.h2d_pending = false; }
+    if (int rc = order_after_run(ctx, s, ctx->stream)) return rc;
+  }
+  CU(ctx, cudaMemsetAsync(ctx->search_out + first_slot * ROW, 0, num_slots * ROW * sizeof(unsigned long long), ctx->stream));
+  for (int c0 = first_slot; c0 < first_slot + num_slots; c0 += MAX_BATCH) {
+    const int cn = std::min(MAX_BATCH, first_slot + num_slots - c0);
+    // one launch per motion-vector representation present (none / int16 / int32 are different kernels)
+    for (int mode = 0; mode < 3; mode++) {
+      BatchCtl ctl;
+      int m = 0;
+      for (int i = 0; i < cn; i++) {
+        if (ctx->slots[c0 + i].mv_mode != mode) continue;
+        ctl.v[m] = 0;   // every plane from buffer 0, the uploaded picture
+        ctl.slot[m] = (uint8_t)i;
+        m++;
+      }
+      if (!m) continue;
+      launch_deblock_search(ctx->g, ctx->slots_dev, c0, m, ctl, mode, cands, num_cands, shift[0], shift[1], ctx->search_out, ctx->stream);
+      ctx->launches++;
+      CU(ctx, cudaGetLastError());
+    }
+  }
+  cudaEvent_t done = ctx->next_run_event(0);
+  CU(ctx, cudaEventRecord(done, ctx->stream));
+  for (int i = first_slot; i < first_slot + num_slots; i++) {
+    ctx->slots[i].ev_run = done;
+    ctx->slots[i].run_stream = ctx->stream;
+    ctx->slots[i].search_k = num_cands;
+  }
+  return ILF_OK;
+}
+
+int ilf_get_deblock_search(ilf_ctx* ctx, int slot, uint64_t* out, int max_cands) {
+  if (int rc = check_slot(ctx, slot)) return rc;
+  if (!out) return fail(ctx, ILF_ERR_ARG, "null output");
+  const Slot& s = ctx->slots[slot];
+  if (!s.search_k) return fail(ctx, ILF_ERR_STATE, "slot %d: no deblocking search yet", slot);
+  if (max_cands < s.search_k) return fail(ctx, ILF_ERR_ARG, "max_cands %d < %d candidates of the last search", max_cands, s.search_k);
+  CU(ctx, cudaSetDevice(ctx->cfg.device));
+  CU(ctx, cudaMemcpyAsync(out, ctx->search_out + (size_t)slot * ILF_DEBLOCK_SEARCH_MAX * 3, (size_t)s.search_k * 3 * sizeof(uint64_t), cudaMemcpyDeviceToHost, ctx->stream));
+  CU(ctx, cudaStreamSynchronize(ctx->stream));
+  return s.search_k;
+}
+
 int ilf_set_timing(ilf_ctx* ctx, int enable) {
   if (!ctx) return ILF_ERR_ARG;
   CU(ctx, cudaSetDevice(ctx->cfg.device));
@@ -1381,6 +1451,7 @@ int ilf_slot_input_planes(ilf_ctx* ctx, int slot, void* planes[3], int32_t pitch
   Slot& s = ctx->slots[slot];
   for (int p = 0; p < 3; p++) { planes[p] = plane_ptr(ctx, s, 0, p); pitch[p] = p ? ctx->g.pitch_c : ctx->g.pitch_y; }
   s.uploaded = true;  // the caller fills the planes on the device
+  s.org_since_upload = false;
   s.result_buf[0] = s.result_buf[1] = s.result_buf[2] = 0;
   return ILF_OK;
 }

@@ -158,6 +158,9 @@ inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, s
 
 // One launch covers `num_slots` <= MAX_BATCH grid layers; layer z works on slot first_slot + ctl.slot[z] under control word ctl.v[z].
 void launch_deblock(const Geom& g, const SlotDev* slots, int first_slot, int num_slots, const BatchCtl& ctl, int mv_mode, int* work, cudaStream_t st);
+// ilf_deblock_search: adds sum((D_k - O)^2 >> shift) of every candidate k and plane to out[(first_slot + ctl.slot[z]) * 192 + 3 k + plane].
+void launch_deblock_search(const Geom& g, const SlotDev* slots, int first_slot, int num_slots, const BatchCtl& ctl, int mv_mode, const ilf_deblock_candidate* cands,
+                           int num_cands, int shift_luma, int shift_chroma, unsigned long long* out, cudaStream_t st);
 void launch_sao(const Geom& g, const SlotDev* slots, int first_slot, int num_slots, const BatchCtl& ctl, cudaStream_t st);
 void launch_alf(const Geom& g, const SlotDev* slots, int first_slot, int num_slots, const BatchCtl& ctl, int planes /* bit 0 luma, bit 1 chroma */, cudaStream_t st);
 void launch_sao_stats(const Geom& g, const SlotDev* slots, int first_slot, int num_slots, const BatchCtl& ctl, cudaStream_t st);

@@ -513,4 +513,380 @@ void launch_deblock(const Geom& g, const SlotDev* slots, int first_slot, int num
   else launch_deblock_mv<2>(g, slots, first_slot, num_slots, ctl, work, st);
 }
 
+// ---------------------------------------------------------------------------------------------------------------------------
+// Deblocking offset search (ilf_deblock_search; EncGOP::applyDeblockingFilterParameterSelection).  The same tiles, boxes and
+// device functions as deblock_kernel, but a tile is deblocked K times, once per (beta, tc) offset candidate, and nothing is
+// stored: the horizontal-pass tasks compare their filtered block with the original and only sums of squared differences leave.
+//   - per tile, what does not depend on the offsets (edge flag, bS, QP, no-filter sides, chroma QP) is derived once into a
+//     compact record per segment; a thread owns the same four segments (one per phase) for every candidate, so the records stay
+//     in its registers, and so does the horizontal-pass task's block of the original;
+//   - per candidate: the staged samples are copied into a work buffer (two buffers alternate, so the copy of candidate k + 1 needs
+//     no barrier behind the horizontal pass of k), vertical edges, a barrier, horizontal edges + distortion;
+//   - a tile without any filtered segment has the same distortion for every candidate: it is measured once (`common`);
+//   - sums: a thread's block fits uint32 (32 x 4095^2 < 2^32), a warp's sum does not: 64-bit warp reduction, then per-warp rows
+//     [candidate][plane] in shared memory (one writer each, no atomics), flushed to global memory with one 64-bit atomicAdd per
+//     entry when the CTA moves on to another slot and at exit.
+// The CTAs walk the tiles of a launch statically (tile blockIdx.x + i * gridDim.x): there is no work counter to share with
+// deblocking launches on other streams.  A tile's K passes hide the fetch of the next tile, which is issued once the last
+// candidate's copy is done.
+namespace {
+
+constexpr int SEARCH_MAX = ILF_DEBLOCK_SEARCH_MAX;
+constexpr int SEARCH_THREADS = 160;   // the task split of deblock_kernel: 136 / 144 vertical tasks, 128 + 128 horizontal tasks on warps 0..3
+constexpr int SEARCH_WARPS_H = 4;     // warps with horizontal tasks (luma: all four; Cb: warps 0, 1; Cr: warps 2, 3)
+constexpr int SEARCH_MIN_CTAS = 4;    // 95 registers, no spills; about 55 KB of shared memory per CTA also fits four (123 registers, 3 CTAs, unbounded)
+
+struct SearchCands {
+  ilf_deblock_candidate c[SEARCH_MAX];
+  int n;
+  int shift_luma, shift_chroma;
+};
+
+// The sample part of a stage (its first bytes: luma, then both chroma planes, same layout), copied once per candidate.
+struct SearchWork {
+  int16_t y[TH][BW];
+  int16_t c[2][CTH][BCW];
+};
+static_assert(sizeof(SearchWork) % 128 == 0 && sizeof(SearchWork) % 16 == 0, "work buffers are copied with 16-byte moves and stay 128-byte aligned");
+
+struct SearchShared {
+  unsigned long long acc[SEARCH_WARPS_H][SEARCH_MAX][3];   // per warp: [candidate][Y, Cb, Cr]
+  unsigned long long common[SEARCH_WARPS_H][3];            // tiles without a filtered segment: the same for every candidate
+  uint64_t full;                                           // the stage's barrier
+  ilf_deblock_params prm;                                  // of the slot being searched
+  uint8_t tc[66 + 2], beta[64], chroma_scale[70 + 2];
+};
+
+template <int MV> __host__ __device__ constexpr int search_smem() {
+  return stage_stride<MV>() + 2 * (int)sizeof(SearchWork) + (int)sizeof(SearchShared);
+}
+
+// Offset-independent part of a luma segment (luma_edge_params up to the tables): 0 = not filtered, else
+// bS | no_p << 2 | no_q << 3 | (QP & 0xFF) << 8.
+template <int MV>
+__device__ __forceinline__ uint32_t luma_edge_record(const Tile<MV>& t, int thr, int qr, int qc, int pr, int pc, bool vertical) {
+  const uint32_t iq = t.info(qr, qc), ip = t.info(pr, pc);
+  if (!(iq & (vertical ? ILF_BI_EDGE_V : ILF_BI_EDGE_H))) return 0;
+  const int bs = boundary_strength<MV>(t, iq, ip, qr, qc, pr, pc, vertical ? ILF_BI_TU_V : ILF_BI_TU_H, thr);
+  if (!bs) return 0;
+  const int qp = ((int)(int8_t)(ip >> 8) + (int)(int8_t)(iq >> 8) + 1) >> 1;
+  return (uint32_t)bs | ((ip & ILF_BI_NOFILT) ? 4u : 0u) | ((iq & ILF_BI_NOFILT) ? 8u : 0u) | ((uint32_t)(qp & 0xFF) << 8);
+}
+
+// tc / beta of a luma record under one candidate's offsets (LoopFilter.cpp:626-634).
+__device__ __forceinline__ EdgeParams luma_edge_apply(uint32_t rec, const SearchShared& sh, int beta_off, int tc_off, int scale) {
+  EdgeParams ep;
+  const int bs = rec & 3, qp = (int)(int8_t)(rec >> 8);
+  ep.bs = bs;
+  ep.tc = sh.tc[clip3i(0, 65, qp + 2 * (bs - 1) + 2 * tc_off)] * scale;
+  ep.beta = sh.beta[clip3i(0, 63, qp + 2 * beta_off)] * scale;
+  ep.no_p = (rec & 4) != 0;
+  ep.no_q = (rec & 8) != 0;
+  return ep;
+}
+
+// Offset-independent part of a chroma segment (chroma_tc up to the table): 0 = not filtered, else
+// 1 | no_p << 1 | no_q << 2 | (chroma QP after the mapping) << 16.
+__device__ __forceinline__ uint32_t chroma_edge_record(uint32_t iq, uint32_t ip, const SearchShared& sh, bool vertical, int comp) {
+  if (!(iq & (vertical ? ILF_BI_EDGE_V : ILF_BI_EDGE_H))) return 0;
+  if (!((iq | ip) & ILF_BI_INTRA)) return 0;
+  int qp = (((int)(int8_t)(ip >> 8) + (int)(int8_t)(iq >> 8) + 1) >> 1) + (comp == 0 ? sh.prm.cb_qp_offset : sh.prm.cr_qp_offset);
+  if (qp >= 70) qp -= 6;
+  else if (qp >= 0) qp = sh.chroma_scale[qp];
+  return 1u | ((ip & ILF_BI_NOFILT) ? 2u : 0u) | ((iq & ILF_BI_NOFILT) ? 4u : 0u) | ((uint32_t)qp << 16);
+}
+
+__device__ __forceinline__ int chroma_edge_tc(uint32_t rec, const SearchShared& sh, int tc_off, int bd_chroma) {
+  return sh.tc[clip3i(0, 65, ((int)rec >> 16) + 2 + 2 * tc_off)] * (1 << (bd_chroma - 8));
+}
+
+// The chroma filter of one line across an edge (xPelFilterChroma, LoopFilter.cpp:918-957): p1 p0 | q0 q1 -> p0, q0.
+__device__ __forceinline__ void filter_chroma_line(int p1, int& p0, int& q0, int q1, int tc, bool no_p, bool no_q, int max_c) {
+  const int delta = clip3i(-tc, tc, (((q0 - p0) << 2) + p1 - q1 + 4) >> 3);
+  const int np = clip3i(0, max_c, p0 + delta), nq = clip3i(0, max_c, q0 - delta);
+  if (!no_p) p0 = np;
+  if (!no_q) q0 = nq;
+}
+
+__device__ __forceinline__ uint32_t sq_shift(int a, int b, int s) { const int d = a - b; return (uint32_t)(d * d) >> s; }
+
+// Squared differences of a luma task's block (8 rows of 4 samples; row i counts when bit i of `rows`) against the original.
+__device__ __forceinline__ uint32_t dist_luma(const uint2 (&r)[8], const uint2 (&o)[8], unsigned rows, int s) {
+  uint32_t acc = 0;
+#pragma unroll
+  for (int i = 0; i < 8; i++) {
+    if (!((rows >> i) & 1)) continue;
+    int a0, a1, a2, a3, b0, b1, b2, b3;
+    unpack2(r[i].x, a0, a1); unpack2(r[i].y, a2, a3); unpack2(o[i].x, b0, b1); unpack2(o[i].y, b2, b3);
+    acc += sq_shift(a0, b0, s) + sq_shift(a1, b1, s) + sq_shift(a2, b2, s) + sq_shift(a3, b3, s);
+  }
+  return acc;
+}
+__device__ __forceinline__ uint32_t dist_chroma(const uint32_t (&r)[8], const uint32_t (&o)[8], unsigned rows, int s) {
+  uint32_t acc = 0;
+#pragma unroll
+  for (int i = 0; i < 8; i++) {
+    if (!((rows >> i) & 1)) continue;
+    int a0, a1, b0, b1;
+    unpack2(r[i], a0, a1); unpack2(o[i], b0, b1);
+    acc += sq_shift(a0, b0, s) + sq_shift(a1, b1, s);
+  }
+  return acc;
+}
+
+__device__ __forceinline__ unsigned long long warp_sum(uint32_t v) {
+  unsigned long long s = v;
+#pragma unroll
+  for (int o = 16; o; o >>= 1) s += __shfl_xor_sync(0xFFFFFFFFu, s, o);
+  return s;
+}
+
+// out[slot][candidate][plane]: slot = first_slot + bc.slot[z] (absolute), rows of SEARCH_MAX x 3 words, zeroed by the caller.
+template <int MV>
+__global__ void __launch_bounds__(SEARCH_THREADS, SEARCH_MIN_CTAS) deblock_search_kernel(Geom g, const SlotDev* __restrict__ slots, int first_slot, BatchCtl bc, int num_slots,
+                                                                      SearchCands cands, unsigned long long* __restrict__ out) {
+  extern __shared__ __align__(128) unsigned char smem[];
+  constexpr int STRIDE = stage_stride<MV>();
+  Stage<MV>* const st = reinterpret_cast<Stage<MV>*>(smem);
+  SearchWork* const work = reinterpret_cast<SearchWork*>(smem + STRIDE);
+  SearchShared& sh = *reinterpret_cast<SearchShared*>(smem + STRIDE + 2 * sizeof(SearchWork));
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int rows = g.rows, crow = g.rows >> 1, cw = g.width >> 1;
+  const int ntx = (g.width + TW - 1) / TW, bands = (g.rows + 4 + TH - 1) / TH;
+  const int per_pic = ntx * bands, total = per_pic * num_slots;
+  const int K = cands.n;
+  int id = blockIdx.x;
+  if (id >= total) return;
+
+  // the boxes of `tile` into the stage, all issued by one thread (the K passes over a tile hide the fetch)
+  auto issue = [&](int tile) {
+    const int z = tile / per_pic, r = tile - z * per_pic, ty = r / ntx, tx = r - ty * ntx;
+    const SlotDev& sd = slots[first_slot + bc.slot[z]];
+    const bool ctree = sd.info_c != nullptr;
+    const int y0 = ty * TH - 4, cy0 = ty * CTH - 2, uy0 = ty * UH - 1;
+    ring::mbar_expect_tx(&sh.full, (uint32_t)stage_tx_bytes<MV>(ctree));
+    ring::tma_load_3d(&st->y[0][0], &sd.tm_db[0], &sh.full, tx * TW - 8, y0, 0);   // buffer 0: the uploaded picture
+    ring::tma_load_3d(&st->c[0][0][0], &sd.tm_db[1], &sh.full, tx * CTW - 8, cy0, 0);
+    ring::tma_load_3d(&st->c[1][0][0], &sd.tm_db[2], &sh.full, tx * CTW - 8, cy0, 0);
+    ring::tma_load_3d(&st->info[0][0], &sd.tm_info, &sh.full, tx * UW - 4, uy0, 0);
+    if (ctree) ring::tma_load_3d(&st->info_c[0][0], &sd.tm_info_c, &sh.full, tx * UW - 4, uy0, 0);
+    if (MV == 1) ring::tma_load_3d(&st->mv[0][0], &sd.tm_mv16, &sh.full, (tx * UW - MvBox<1>::OFF) * 2, uy0, 0);
+    if (MV == 2) ring::tma_load_3d(&st->mv[0][0], &sd.tm_mv32, &sh.full, (tx * UW - MvBox<2>::OFF) * 4, uy0, 0);
+  };
+  if (tid == 0) {
+    ring::mbar_init(&sh.full, 1);
+    ring::mbar_init_fence();
+  }
+  if (tid < 66) sh.tc[tid] = c_tc[tid];
+  if (tid < 64) sh.beta[tid] = c_beta[tid];
+  if (tid < 70) sh.chroma_scale[tid] = c_chroma_scale[tid];
+  for (int i = tid; i < SEARCH_WARPS_H * SEARCH_MAX * 3; i += SEARCH_THREADS) (&sh.acc[0][0][0])[i] = 0;
+  if (tid < SEARCH_WARPS_H * 3) (&sh.common[0][0])[tid] = 0;
+  __syncthreads();
+  if (tid == 0) issue(id);
+
+  // adds the CTA's sums of slot layer z to the result rows and clears them
+  auto flush = [&](int z) {
+    __syncthreads();
+    unsigned long long* o = out + (size_t)(first_slot + bc.slot[z]) * (SEARCH_MAX * 3);
+    for (int i = tid; i < K * 3; i += SEARCH_THREADS) {
+      unsigned long long s = 0;
+#pragma unroll
+      for (int w = 0; w < SEARCH_WARPS_H; w++) { s += (&sh.acc[w][0][0])[i] + sh.common[w][i % 3]; (&sh.acc[w][0][0])[i] = 0; }
+      if (s) atomicAdd(o + i, s);
+    }
+    __syncthreads();
+    if (tid < SEARCH_WARPS_H * 3) (&sh.common[0][0])[tid] = 0;   // read again behind at least one more barrier
+  };
+
+  const int max_y = (1 << g.bd_luma) - 1, max_c = (1 << g.bd_chroma) - 1, scale_y = 1 << (g.bd_luma - 8);
+  const int s_l = cands.shift_luma, s_c = cands.shift_chroma;
+  int cur = -1;
+  bool ctree = false;
+  uint32_t phase = 0;
+  for (; id < total; id += gridDim.x) {
+    const int z = id / per_pic, r = id - z * per_pic, ty = r / ntx, tx = r - ty * ntx;
+    const int next = id + (int)gridDim.x;
+    if (z != cur) {   // CTA-uniform
+      if (cur >= 0) flush(cur);
+      const SlotDev& sd = slots[first_slot + bc.slot[z]];
+      for (int i = tid; i < (int)(sizeof(ilf_deblock_params) / 4); i += SEARCH_THREADS) reinterpret_cast<uint32_t*>(&sh.prm)[i] = __ldg(reinterpret_cast<const uint32_t*>(sd.db_params) + i);
+      ctree = sd.info_c != nullptr;
+      cur = z;
+      __syncthreads();
+    }
+    const int y0 = ty * TH - 4, cy0 = ty * CTH - 2, x0 = tx * TW, cx0 = tx * CTW;
+    // this thread's horizontal-pass blocks of the original: the samples the deblocking kernel would store (y in [0, rows), x < width)
+    const int u = tid & 31, h = (tid >> 5) & 3;
+    const int pl = (tid >> 6) & 1, hc = (tid >> 5) & 1;
+    unsigned rows_y = 0, rows_c = 0;
+    uint2 org_y[8];
+    uint32_t org_c[8];
+    if (tid < 128) {
+      const SlotDev& sd = slots[first_slot + bc.slot[z]];
+      const int x = x0 + 4 * u;
+#pragma unroll
+      for (int i = 0; i < 8; i++) {
+        const int y = y0 + 8 * h + i;
+        const bool in = x < g.width && y >= 0 && y < rows;
+        rows_y |= (in ? 1u : 0u) << i;
+        org_y[i] = in ? ldg_u2(sd.org[0] + (size_t)y * g.pitch_y + x) : make_uint2(0, 0);
+      }
+      const int xc = cx0 + 2 * u;
+#pragma unroll
+      for (int i = 0; i < 8; i++) {
+        const int y = cy0 + 8 * hc + i;
+        const bool in = xc < cw && y >= 0 && y < crow;
+        rows_c |= (in ? 1u : 0u) << i;
+        org_c[i] = in ? __ldg(reinterpret_cast<const uint32_t*>(sd.org[1 + pl] + (size_t)y * g.pitch_c + xc)) : 0u;
+      }
+    }
+    Tile<MV> t;
+    t.st = st;
+    t.ctree = ctree;
+    ring::mbar_wait(&sh.full, phase);
+    phase ^= 1u;
+
+    // ---- offset-independent records of this thread's four segments (the task split of deblock_kernel) ----
+    const int thr = sh.prm.mv_threshold;
+    uint32_t rec_lv = 0, rec_cv = 0, rec_lh = 0, rec_ch = 0;
+    const int ev = tid < 128 ? (tid & 15) : 16, sgv = tid < 128 ? (tid >> 4) : tid - 128;    // luma vertical task (tid < 136)
+    const int plv = tid < 128 ? (tid >> 6) : ((tid - 128) >> 3), kv = tid < 128 ? ((tid >> 3) & 7) : 8, sgc = tid & 7;   // chroma vertical (tid < 144)
+    if (tid < 17 * 8) rec_lv = luma_edge_record<MV>(t, thr, sgv, 2 * ev, sgv, 2 * ev - 1, true);
+    if (tid < 2 * 9 * 8) rec_cv = chroma_edge_record(t.cinfo(sgc, 4 * kv), t.cinfo(sgc, 4 * kv - 1), sh, true, plv);
+    if (tid < 128) {
+      rec_lh = luma_edge_record<MV>(t, thr, 2 * h + 1, u, 2 * h, u, false);
+      rec_ch = chroma_edge_record(t.cinfo(4 * hc + 1, u), t.cinfo(4 * hc, u), sh, false, pl);
+    }
+    if (!__syncthreads_or((int)(rec_lv | rec_cv | rec_lh | rec_ch))) {
+      // nothing in the tile is filtered under any candidate: measure the staged samples once
+      if (tid < 128) {
+        uint2 raw[8];
+        uint32_t rc[8];
+#pragma unroll
+        for (int i = 0; i < 8; i++) {
+          raw[i] = *reinterpret_cast<const uint2*>(t.y(8 * h + i, 4 * u));
+          rc[i] = *reinterpret_cast<const uint32_t*>(t.ch(pl, 8 * hc + i, 2 * u));
+        }
+        const unsigned long long dy = warp_sum(dist_luma(raw, org_y, rows_y, s_l)), dc = warp_sum(dist_chroma(rc, org_c, rows_c, s_c));
+        if (lane == 0) { sh.common[warp][0] += dy; sh.common[warp][1 + pl] += dc; }
+      }
+      __syncthreads();   // the stage is free
+      if (tid == 0 && next < total) issue(next);
+      continue;
+    }
+
+    for (int k = 0; k < K; k++) {
+      SearchWork* const w = work + (k & 1);
+      {
+        const uint4* src = reinterpret_cast<const uint4*>(st);
+        uint4* dst = reinterpret_cast<uint4*>(w);
+        for (int i = tid; i < (int)(sizeof(SearchWork) / 16); i += SEARCH_THREADS) dst[i] = src[i];
+      }
+      __syncthreads();
+      // the records are in registers and the samples in the work buffer: the stage can take the next tile
+      if (k == K - 1 && tid == 0 && next < total) issue(next);
+      const int beta_off = cands.c[k].beta_offset_div2, tc_off = cands.c[k].tc_offset_div2;
+
+      // ---- vertical edges (deblock_kernel's luma and chroma tasks) ----
+      if (rec_lv) {
+        const EdgeParams ep = luma_edge_apply(rec_lv, sh, beta_off, tc_off, scale_y);
+        int16_t* pp = &w->y[4 * sgv][8 * ev - 4 + 8];
+        int16_t* pq = &w->y[4 * sgv][8 * ev + 8];
+        int L[4][8];
+#pragma unroll
+        for (int i = 0; i < 4; i++) {
+          const uint2 a = *reinterpret_cast<const uint2*>(pp + i * BW), b = *reinterpret_cast<const uint2*>(pq + i * BW);
+          unpack2(a.x, L[i][0], L[i][1]); unpack2(a.y, L[i][2], L[i][3]); unpack2(b.x, L[i][4], L[i][5]); unpack2(b.y, L[i][6], L[i][7]);
+        }
+        if (filter_luma_segment(L, ep, max_y)) {
+#pragma unroll
+          for (int i = 0; i < 4; i++) {
+            *reinterpret_cast<uint2*>(pp + i * BW) = make_uint2(pack2(L[i][0], L[i][1]), pack2(L[i][2], L[i][3]));
+            *reinterpret_cast<uint2*>(pq + i * BW) = make_uint2(pack2(L[i][4], L[i][5]), pack2(L[i][6], L[i][7]));
+          }
+        }
+      }
+      if (rec_cv) {
+        const int tc = chroma_edge_tc(rec_cv, sh, tc_off, g.bd_chroma);
+        int16_t* pp = &w->c[plv][2 * sgc][8 * kv - 2 + 8];
+        int16_t* pq = &w->c[plv][2 * sgc][8 * kv + 8];
+#pragma unroll
+        for (int i = 0; i < 2; i++) {
+          int p0 = pp[i * BCW + 1], q0 = pq[i * BCW];
+          filter_chroma_line(pp[i * BCW], p0, q0, pq[i * BCW + 1], tc, rec_cv & 2, rec_cv & 4, max_c);
+          pp[i * BCW + 1] = (int16_t)p0;
+          pq[i * BCW] = (int16_t)q0;
+        }
+      }
+      __syncthreads();
+
+      // ---- horizontal edges + distortion of the blocks the deblocking kernel would store ----
+      if (tid < 128) {
+        uint2 raw[8];
+#pragma unroll
+        for (int i = 0; i < 8; i++) raw[i] = *reinterpret_cast<const uint2*>(&w->y[8 * h + i][4 * u + 8]);
+        if (rec_lh) {
+          const EdgeParams ep = luma_edge_apply(rec_lh, sh, beta_off, tc_off, scale_y);
+          int L[4][8];
+#pragma unroll
+          for (int i = 0; i < 8; i++) { unpack2(raw[i].x, L[0][i], L[1][i]); unpack2(raw[i].y, L[2][i], L[3][i]); }
+          if (filter_luma_segment(L, ep, max_y)) {
+#pragma unroll
+            for (int i = 1; i < 7; i++) raw[i] = make_uint2(pack2(L[0][i], L[1][i]), pack2(L[2][i], L[3][i]));
+          }
+        }
+        uint32_t rc[8];
+#pragma unroll
+        for (int i = 0; i < 8; i++) rc[i] = *reinterpret_cast<const uint32_t*>(&w->c[pl][8 * hc + i][2 * u + 8]);
+        if (rec_ch) {
+          const int tc = chroma_edge_tc(rec_ch, sh, tc_off, g.bd_chroma);
+          int a[4], b[4];
+#pragma unroll
+          for (int i = 0; i < 4; i++) unpack2(rc[i], a[i], b[i]);
+          filter_chroma_line(a[0], a[1], a[2], a[3], tc, rec_ch & 2, rec_ch & 4, max_c);
+          filter_chroma_line(b[0], b[1], b[2], b[3], tc, rec_ch & 2, rec_ch & 4, max_c);
+          rc[1] = pack2(a[1], b[1]);
+          rc[2] = pack2(a[2], b[2]);
+        }
+        const unsigned long long dy = warp_sum(dist_luma(raw, org_y, rows_y, s_l)), dc = warp_sum(dist_chroma(rc, org_c, rows_c, s_c));
+        if (lane == 0) { sh.acc[warp][k][0] += dy; sh.acc[warp][k][1 + pl] += dc; }
+      }
+      // (no barrier: the next candidate copies into the other work buffer, and the one after it waits behind the next vertical pass)
+    }
+  }
+  flush(cur);
+}
+
+}  // namespace
+
+template <int MV>
+static void launch_deblock_search_mv(const Geom& g, const SlotDev* slots, int first_slot, int num_slots, const BatchCtl& ctl, const SearchCands& sc,
+                                     unsigned long long* out, cudaStream_t st) {
+  constexpr int smem = search_smem<MV>();
+  static bool attr_set[64] = {};
+  once_per_device(attr_set, [&] { cudaFuncSetAttribute(deblock_search_kernel<MV>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem); });
+  int dev = 0, sms = 0, per_sm = 0;
+  cudaGetDevice(&dev);
+  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+  cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, deblock_search_kernel<MV>, SEARCH_THREADS, smem);
+  const int ntx = (g.width + TW - 1) / TW, bands = (g.rows + 4 + TH - 1) / TH;
+  const long long total = (long long)ntx * bands * num_slots;
+  const dim3 grid((unsigned)std::min<long long>(total, (long long)std::max(1, sms * per_sm)));
+  deblock_search_kernel<MV><<<grid, SEARCH_THREADS, smem, st>>>(g, slots, first_slot, ctl, num_slots, sc, out);
+}
+
+// One launch per motion-vector representation present (ilf_api.cu); `out` = result rows of slot 0 of the context.
+void launch_deblock_search(const Geom& g, const SlotDev* slots, int first_slot, int num_slots, const BatchCtl& ctl, int mv_mode, const ilf_deblock_candidate* cands,
+                           int num_cands, int shift_luma, int shift_chroma, unsigned long long* out, cudaStream_t st) {
+  SearchCands sc = {};
+  for (int k = 0; k < num_cands; k++) sc.c[k] = cands[k];
+  sc.n = num_cands;
+  sc.shift_luma = shift_luma;
+  sc.shift_chroma = shift_chroma;
+  if (mv_mode == 0) launch_deblock_search_mv<0>(g, slots, first_slot, num_slots, ctl, sc, out, st);
+  else if (mv_mode == 1) launch_deblock_search_mv<1>(g, slots, first_slot, num_slots, ctl, sc, out, st);
+  else launch_deblock_search_mv<2>(g, slots, first_slot, num_slots, ctl, sc, out, st);
+}
+
 }  // namespace ilf

@@ -37,6 +37,7 @@ def lib_path():
 _LIB = None
 NUM_KERNELS = 6   # ILF_NUM_KERNELS
 ALF_STATS_WORDS = 25 * 105 + 36 + 36   # ILF_ALF_STATS_WORDS
+DEBLOCK_SEARCH_MAX = 64   # ILF_DEBLOCK_SEARCH_MAX
 
 
 def load_library():
@@ -89,6 +90,8 @@ def load_library():
     lib.ilf_alf_path.argtypes = [vp, i]
     lib.ilf_alf_stats.argtypes = [vp, i, i]
     lib.ilf_get_alf_stats.argtypes = [vp, i, vp]
+    lib.ilf_deblock_search.argtypes = [vp, i, i, vp, i, vp]
+    lib.ilf_get_deblock_search.argtypes = [vp, i, vp, i]
     lib.ilf_picture_hash.argtypes = [vp, i, i, C.POINTER(C.c_uint32 * 3)]
     lib.ilf_download_extended.argtypes = [vp, i, vp, pd, vp, pd, vp, pd, i]
     lib.ilf_launch_count.argtypes = [vp]
@@ -302,6 +305,26 @@ class InLoopFilter:
         out = np.zeros((n, ALF_STATS_WORDS), np.int64)
         self._ck(self._lib.ilf_get_alf_stats(self._h, slot, _ptr(out)))
         return out
+
+    # ---- encoder deblocking parameter search (EncGOP::applyDeblockingFilterParameterSelection) -----------
+    def deblock_search(self, candidates, shift=(0, 0), first_slot=0, num_slots=1):
+        """Score (beta_offset_div2, tc_offset_div2) pairs on the slots' uploaded pictures: per candidate and plane, the sum of
+        ((deblocked - original)^2 >> shift[luma / chroma]) with every slice's offsets replaced by the candidate's."""
+        c = np.asarray(candidates, dtype=np.int64).reshape(-1, 2)
+        if c.size and (c.min() < -128 or c.max() > 127):
+            raise IlfError("deblocking offsets must fit int8")
+        c = np.ascontiguousarray(c.astype(np.int8))
+        sh = np.ascontiguousarray(shift, dtype=np.int32)
+        assert sh.shape == (2,)
+        self._ck(self._lib.ilf_deblock_search(self._h, first_slot, num_slots, _ptr(c), len(c), _ptr(sh)))
+
+    def get_deblock_search(self, slot=0):
+        """uint64 [K, 3]: the sums of the slot's last deblock_search, per candidate and plane (Y, Cb, Cr)."""
+        out = np.zeros((DEBLOCK_SEARCH_MAX, 3), np.uint64)
+        r = self._lib.ilf_get_deblock_search(self._h, slot, _ptr(out), DEBLOCK_SEARCH_MAX)
+        if r < 0:
+            self._ck(r)
+        return out[:r].copy()
 
     def picture_hash(self, slot=0, kind="crc"):
         """calcCRC / calcChecksum of the slot's current picture on the device: [Y, Cb, Cr]."""
