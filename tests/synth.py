@@ -1,5 +1,6 @@
 """Synthetic side information and pictures for parity tests (seeded numpy; shapes follow include/ilf_b200.h)."""
 import numpy as np
+import pytest
 
 SAO_DT = np.dtype([("offset", "<i2", (3, 4)), ("type", "i1", (3,)), ("band_pos", "u1", (3,)), ("avail", "u1"), ("reserved", "u1")])
 assert SAO_DT.itemsize == 32
@@ -7,11 +8,18 @@ ALF_DT = np.dtype([("luma_coeff", "<i2", (25, 13)), ("chroma_coeff", "<i2", (7,)
 DB_DT = np.dtype([("cb_qp_offset", "<i4"), ("cr_qp_offset", "<i4"), ("mv_threshold", "<i4"), ("num_slices", "<i4"), ("slices", "i1", (64, 4))])
 
 
-def picture(rng, w, h, bd=10, kind="mix"):
-    """int16 planes with smooth areas, edges, noise and saturated patches (so clipping paths are hit)."""
-    mx = (1 << bd) - 1
+def keep_ids(rows, expand):
+    """pytest parameters of cases written before their test took more columns (e.g. one bit depth for both planes): expand(*row)
+    gives the test's columns, and each case keeps the id pytest gave the row as written."""
+    return [pytest.param(*expand(*r), id="-".join(map(str, r))) for r in rows]
 
-    def plane(ww, hh):
+
+def picture(rng, w, h, bd=10, kind="mix", bd_chroma=None):
+    """int16 planes with smooth areas, edges, noise and saturated patches (so clipping paths are hit); luma at `bd` bits,
+    chroma at `bd_chroma` (default: `bd`)."""
+
+    def plane(ww, hh, bd):
+        mx = (1 << bd) - 1
         y, x = np.mgrid[0:hh, 0:ww]
         base = mx / 2 + mx / 3 * np.sin(x / 9.0) * np.cos(y / 7.0)
         blk = np.kron(rng.integers(-mx // 16, mx // 16 + 1, ((hh + 7) // 8, (ww + 7) // 8)), np.ones((8, 8), np.int64))[:hh, :ww]
@@ -25,15 +33,19 @@ def picture(rng, w, h, bd=10, kind="mix"):
             p[yy:yy + 9, xx:xx + 13] = rng.choice([0, mx, mx // 2])
         return p.astype(np.int16)
 
-    return {"y": plane(w, h), "cb": plane(w // 2, h // 2), "cr": plane(w // 2, h // 2)}
+    bdc = bd if bd_chroma is None else bd_chroma
+    return {"y": plane(w, h, bd), "cb": plane(w // 2, h // 2, bdc), "cr": plane(w // 2, h // 2, bdc)}
 
 
-def sao_params(rng, ctus_w, ctus_h, bd=10, p_off=0.25, all_avail=False):
+def sao_params(rng, ctus_w, ctus_h, bd=10, p_off=0.25, all_avail=False, bd_chroma=None):
+    """Offsets of each component in the range of its own bit depth (luma `bd`, chroma `bd_chroma`, default `bd`)."""
     n = ctus_w * ctus_h
     a = np.zeros(n, SAO_DT)
-    maxo = min(127, 31 << max(0, bd - 10))
+    maxo_of = lambda b: min(127, 31 << max(0, b - 10))
+    maxos = (maxo_of(bd),) + 2 * (maxo_of(bd if bd_chroma is None else bd_chroma),)
     for i in range(n):
         for c in range(3):
+            maxo = maxos[c]
             t = -1 if rng.random() < p_off else int(rng.integers(0, 5))
             a["type"][i, c] = t
             a["band_pos"][i, c] = rng.integers(0, 32)
@@ -109,11 +121,13 @@ def deblock_info(rng, w, h, p_edge=0.5, p_intra=0.4, inter=False):
     return prm.tobytes(), info, mv16
 
 
-def deblock_info_stress(rng, w, h, ctu_log2=7, mv32=False):
+def deblock_info_stress(rng, w, h, ctu_log2=7, mv32=False, bd_luma=8, chroma_qp_offset=6):
     """Side information that real streams of the committed configurations rarely or never carry: several slices with their
     own beta / tc offsets (ctu_slice map), no-filter units (PCM / lossless), B-slice units with two reference ids and four
     motion-vector components, a separate chroma-tree layer, QPs over the whole range, optionally 32-bit motion vectors.
-    Returns a dict with the keys of the bench side information."""
+    The QPs of both layers come from [-6 (bd_luma - 8), 63] (negative at 10 and 12 bit, as the QP byte of the grid is signed),
+    the PPS chroma QP offsets from +-chroma_qp_offset (the syntax allows +-12).  The defaults keep the draws of the cases
+    written before these arguments existed.  Returns a dict with the keys of the bench side information."""
     uw, uh = w // 4, h // 4
     bw, bh = (uw + 1) // 2, (uh + 1) // 2
     up = lambda a: np.kron(a, np.ones((2, 2), a.dtype))[:uh, :uw]
@@ -122,7 +136,7 @@ def deblock_info_stress(rng, w, h, ctu_log2=7, mv32=False):
     def layer(p_intra):
         intra = up((rng.random((bh, bw)) < p_intra).astype(np.uint32))
         cbf = up((rng.random((bh, bw)) < 0.5).astype(np.uint32))
-        qp = up(rng.integers(0, 64, (bh, bw)).astype(np.uint32))
+        qp = up((rng.integers(-6 * (bd_luma - 8), 64, (bh, bw)) & 0xFF).astype(np.uint32))
         ev = up((rng.random((bh, bw)) < 0.6).astype(np.uint32)) * ((xs % 2 == 0) & (xs > 0))
         eh = up((rng.random((bh, bw)) < 0.6).astype(np.uint32)) * ((ys % 2 == 0) & (ys > 0))
         tv = up((rng.random((bh, bw)) < 0.7).astype(np.uint32))
@@ -141,7 +155,8 @@ def deblock_info_stress(rng, w, h, ctu_log2=7, mv32=False):
     ctu = 1 << ctu_log2
     cw, ch = (w + ctu - 1) // ctu, (h + ctu - 1) // ctu
     prm = np.zeros(1, DB_DT)
-    prm["cb_qp_offset"], prm["cr_qp_offset"], prm["mv_threshold"], prm["num_slices"] = rng.integers(-6, 7), rng.integers(-6, 7), 16 if mv32 else 4, 3
+    co = chroma_qp_offset
+    prm["cb_qp_offset"], prm["cr_qp_offset"], prm["mv_threshold"], prm["num_slices"] = rng.integers(-co, co + 1), rng.integers(-co, co + 1), 16 if mv32 else 4, 3
     prm["slices"][0, :3, 0] = rng.integers(-6, 7, 3)
     prm["slices"][0, :3, 1] = rng.integers(-6, 7, 3)
     d = {"db_params": prm.tobytes(), "db_info": info, "db_info_c": info_c, "ctu_slice": np.sort(rng.integers(0, 3, cw * ch)).astype(np.uint8)}

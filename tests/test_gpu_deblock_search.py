@@ -45,8 +45,10 @@ def oracle_search(O, pic, org, bd_l, bd_c, ctu_log2, params_bytes, info, info_c,
     return out
 
 
-def _org_of(rng, pic, bd):
-    return {k: np.clip(pic[k].astype(np.int32) + rng.integers(-12, 13, pic[k].shape), 0, (1 << bd) - 1).astype(np.int16) for k in K}
+def _org_of(rng, pic, bd, bd_chroma=None):
+    """The picture plus noise, each plane clipped to its own range (luma `bd`, chroma `bd_chroma`, default `bd`)."""
+    bds = dict(zip(K, (bd,) + 2 * (bd if bd_chroma is None else bd_chroma,)))
+    return {k: np.clip(pic[k].astype(np.int32) + rng.integers(-12, 13, pic[k].shape), 0, (1 << bds[k]) - 1).astype(np.int16) for k in K}
 
 
 def _mv(c):
@@ -110,22 +112,28 @@ def test_captures_equal_oracle(path, ilf_lib, oracle):
 
 
 # odd sizes (width / 2 not a multiple of 8, partial CTUs and tiles), every CTU size and bit depth, none / int16 / int32 motion, three
-# slices with their own base offsets (the candidate must override all of them) and the whole QP range
-@pytest.mark.parametrize("w,h,bd,ctu_log2,mv,seed", [(200, 136, 8, 5, "mv16", 1), (264, 72, 10, 6, "none", 2), (136, 264, 12, 7, "mv32", 3),
-                                                     (392, 72, 10, 6, "mv16", 4), (520, 392, 10, 7, "mv32", 5), (16, 16, 10, 5, "none", 6)])
-def test_synthetic_matrix_equals_oracle(w, h, bd, ctu_log2, mv, seed, ilf_lib, oracle):
+# slices with their own base offsets (the candidate must override all of them) and the whole QP range.  The cases at two bit depths
+# also draw the negative QPs of their luma depth and chroma QP offsets up to +-12 (the cases at one depth keep their draws).
+@pytest.mark.parametrize("w,h,bd_luma,bd_chroma,ctu_log2,mv,seed",
+                         synth.keep_ids([(200, 136, 8, 5, "mv16", 1), (264, 72, 10, 6, "none", 2), (136, 264, 12, 7, "mv32", 3),
+                                         (392, 72, 10, 6, "mv16", 4), (520, 392, 10, 7, "mv32", 5), (16, 16, 10, 5, "none", 6)],
+                                        lambda w, h, bd, c, mv, s: (w, h, bd, bd, c, mv, s)) +
+                         [(200, 136, 8, 12, 5, "mv16", 7), (264, 72, 12, 10, 6, "none", 8), (520, 392, 12, 10, 7, "mv32", 9)])
+def test_synthetic_matrix_equals_oracle(w, h, bd_luma, bd_chroma, ctu_log2, mv, seed, ilf_lib, oracle):
     rng = np.random.default_rng(seed)
-    pic = synth.picture(rng, w, h, bd, "mix")
-    org = _org_of(rng, pic, bd)
-    si = synth.deblock_info_stress(rng, w, h, ctu_log2, mv == "mv32")
+    pic = synth.picture(rng, w, h, bd_luma, "mix", bd_chroma=bd_chroma)
+    org = _org_of(rng, pic, bd_luma, bd_chroma)
+    wide = {} if bd_luma == bd_chroma else {"bd_luma": bd_luma, "chroma_qp_offset": 12}
+    si = synth.deblock_info_stress(rng, w, h, ctu_log2, mv == "mv32", **wide)
     mv16, mv32 = (si.get("db_mv16"), si.get("db_mv32")) if mv != "none" else (None, None)
     cands = [(0, 0), (3, -2), (-4, 5), (6, 6), (-128, 127), (127, -128), (20, -20), (-1, 1)]
-    want = oracle_search(oracle, pic, org, bd, bd, ctu_log2, si["db_params"], si["db_info"], si["db_info_c"], mv16, mv32, si["ctu_slice"], cands, [(0, 0), (2, 3)])
-    with ilf_lib.InLoopFilter(w, h, bd, bd, ctu_log2) as f:
+    shifts = [(0, 0), (2, 3), (0, 4), (4, 0)]
+    want = oracle_search(oracle, pic, org, bd_luma, bd_chroma, ctu_log2, si["db_params"], si["db_info"], si["db_info_c"], mv16, mv32, si["ctu_slice"], cands, shifts)
+    with ilf_lib.InLoopFilter(w, h, bd_luma, bd_chroma, ctu_log2) as f:
         f.upload(0, *(pic[k] for k in K))
         f.set_deblock_info(0, si["db_params"], si["db_info"], si["db_info_c"], mv16, mv32, si["ctu_slice"])
         f.set_original(0, org["y"], org["cb"], org["cr"], np.zeros(f.ctus_w * f.ctus_h, np.uint8))
-        for s in ((0, 0), (2, 3)):
+        for s in shifts:
             f.deblock_search(cands, s)
             assert np.array_equal(f.get_deblock_search(0), want[s]), f"shift {s}"
     if w * h > 16 * 16:

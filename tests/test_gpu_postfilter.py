@@ -11,14 +11,18 @@ pytestmark = pytest.mark.gpu
 K = ("y", "cb", "cr")
 
 
-@pytest.mark.parametrize("w,h,bd,seed", [(416, 240, 10, 1), (200, 136, 10, 2), (264, 72, 8, 3), (136, 264, 12, 4), (8, 8, 10, 5), (1920, 1080, 10, 6), (3840, 2160, 10, 7)])
-def test_picture_hash_matches_oracle(w, h, bd, seed, ilf_lib, oracle):
+# (8, 10): one byte per luma sample and two per chroma sample; (12, 8) the other way round
+@pytest.mark.parametrize("w,h,bd_luma,bd_chroma,seed",
+                         synth.keep_ids([(416, 240, 10, 1), (200, 136, 10, 2), (264, 72, 8, 3), (136, 264, 12, 4), (8, 8, 10, 5), (1920, 1080, 10, 6), (3840, 2160, 10, 7)],
+                                        lambda w, h, bd, s: (w, h, bd, bd, s)) +
+                         [(200, 136, 8, 10, 8), (264, 72, 12, 8, 9)])
+def test_picture_hash_matches_oracle(w, h, bd_luma, bd_chroma, seed, ilf_lib, oracle):
     rng = np.random.default_rng(seed)
-    pic = synth.picture(rng, w, h, bd, "noise")
-    with ilf_lib.InLoopFilter(w, h, bd, bd, 7) as f:
+    pic = synth.picture(rng, w, h, bd_luma, "noise", bd_chroma=bd_chroma)
+    with ilf_lib.InLoopFilter(w, h, bd_luma, bd_chroma, 7) as f:
         f.upload(0, *(pic[k] for k in K))
         for kind in ("crc", "checksum"):
-            assert f.picture_hash(0, kind) == oracle.picture_hash(pic, bd, bd, kind), kind
+            assert f.picture_hash(0, kind) == oracle.picture_hash(pic, bd_luma, bd_chroma, kind), kind
 
 
 def test_picture_hash_follows_the_filtered_picture(ilf_lib, oracle):

@@ -16,20 +16,26 @@ pytestmark = pytest.mark.gpu
 K = ("y", "cb", "cr")
 
 
-def _org_of(rng, pic, bd):
-    return {k: np.clip(pic[k].astype(np.int32) + rng.integers(-12, 13, pic[k].shape), 0, (1 << bd) - 1).astype(np.int16) for k in K}
+def _org_of(rng, pic, bd, bd_chroma=None):
+    """The picture plus noise, each plane clipped to its own range (luma `bd`, chroma `bd_chroma`, default `bd`)."""
+    bds = dict(zip(K, (bd,) + 2 * (bd if bd_chroma is None else bd_chroma,)))
+    return {k: np.clip(pic[k].astype(np.int32) + rng.integers(-12, 13, pic[k].shape), 0, (1 << bds[k]) - 1).astype(np.int16) for k in K}
 
 
-@pytest.mark.parametrize("w,h,bd,ctu_log2,seed", [(416, 240, 10, 7, 1), (200, 136, 10, 6, 2), (264, 72, 8, 5, 3), (136, 264, 12, 5, 4), (1920, 1080, 10, 7, 5)])
-def test_statistics_of_the_uploaded_picture(w, h, bd, ctu_log2, seed, ilf_lib, oracle):
-    """Random availability flags (multi-slice patterns), odd sizes with partial CTUs, 8/10/12 bit, noisy and smooth content."""
+@pytest.mark.parametrize("w,h,bd_luma,bd_chroma,ctu_log2,seed",
+                         synth.keep_ids([(416, 240, 10, 7, 1), (200, 136, 10, 6, 2), (264, 72, 8, 5, 3), (136, 264, 12, 5, 4), (1920, 1080, 10, 7, 5)],
+                                        lambda w, h, bd, c, s: (w, h, bd, bd, c, s)) +
+                         [(200, 136, 8, 10, 6, 6), (264, 72, 12, 10, 5, 7)])
+def test_statistics_of_the_uploaded_picture(w, h, bd_luma, bd_chroma, ctu_log2, seed, ilf_lib, oracle):
+    """Random availability flags (multi-slice patterns), odd sizes with partial CTUs, 8/10/12 bit (luma and chroma at the same or
+    at different depths: the band classes of each component follow its own depth), noisy and smooth content."""
     rng = np.random.default_rng(seed)
     ctu = 1 << ctu_log2
     n = ((w + ctu - 1) // ctu) * ((h + ctu - 1) // ctu)
-    with ilf_lib.InLoopFilter(w, h, bd, bd, ctu_log2) as f:
+    with ilf_lib.InLoopFilter(w, h, bd_luma, bd_chroma, ctu_log2) as f:
         for kind in ("noise", "smooth"):
-            pic = synth.picture(rng, w, h, bd, kind)
-            org = _org_of(rng, pic, bd)
+            pic = synth.picture(rng, w, h, bd_luma, kind, bd_chroma=bd_chroma)
+            org = _org_of(rng, pic, bd_luma, bd_chroma)
             cw = (w + ctu - 1) // ctu
             avail = rng.integers(0, 256, n).astype(np.uint8)
             for i in range(n):      # picture borders are never available
@@ -39,7 +45,7 @@ def test_statistics_of_the_uploaded_picture(w, h, bd, ctu_log2, seed, ilf_lib, o
             f.set_original(0, org["y"], org["cb"], org["cr"], avail)
             f.sao_stats(0, 1)
             got = f.get_sao_stats(0)
-            want = oracle.sao_stats(pic, org, bd, bd, ctu_log2, avail)
+            want = oracle.sao_stats(pic, org, bd_luma, bd_chroma, ctu_log2, avail)
             bad = np.argwhere(got != want)
             assert bad.size == 0, f"{kind}: first mismatch (ctu, comp, type, word) {bad[0]}: got {got[tuple(bad[0])]} want {want[tuple(bad[0])]}"
 
