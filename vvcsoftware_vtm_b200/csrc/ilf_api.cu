@@ -114,6 +114,7 @@ struct Slot {
   int result_buf[3] = {0, 0, 0};  // buffer holding the current picture, per plane
   bool sao_on[3] = {false, false, false};  // any CTU with SAO enabled, per component
   bool alf_on[3] = {false, false, false};
+  bool db_chroma = true;           // the chroma decisions' grid has an intra unit: deblocking may change the chroma planes
   bool alf_is7 = false;            // luma filter shape of the slot's ALF parameters
   // Transfer pipeline: H2D copies run on the context's upload stream, kernels on the compute stream, D2H copies on the
   // download stream; the three are ordered per slot with these events, so upload of picture n+1, filtering of picture n
@@ -879,6 +880,19 @@ void ilf_host_free(void* p) { if (p) cudaFreeHost(p); }
 int ilf_host_register(void* p, size_t bytes) { if (cudaHostRegister(p, bytes, cudaHostRegisterDefault) != cudaSuccess) { cudaGetLastError(); return ILF_ERR_CUDA; } return ILF_OK; }
 int ilf_host_unregister(void* p) { if (cudaHostUnregister(p) != cudaSuccess) { cudaGetLastError(); return ILF_ERR_CUDA; } return ILF_OK; }
 
+// Whether any of the n units of a dense grid is intra, in 64-bit words, a cache line at a time, stopping at the first hit.
+static bool any_intra(const uint32_t* grid, size_t n) {
+  constexpr uint64_t mask = ILF_BI_INTRA | (uint64_t)ILF_BI_INTRA << 32;
+  size_t i = 0;
+  for (; i + 16 <= n; i += 16) {
+    uint64_t w[8];
+    memcpy(w, grid + i, sizeof(w));
+    if ((w[0] | w[1] | w[2] | w[3] | w[4] | w[5] | w[6] | w[7]) & mask) return true;
+  }
+  for (; i < n; i++) if (grid[i] & ILF_BI_INTRA) return true;
+  return false;
+}
+
 // Grids cover the rows the context holds (units_h = held rows / 4); ctu_slice covers the full picture.
 int ilf_set_deblock_info(ilf_ctx* ctx, int slot, const ilf_deblock_params* params, const uint32_t* info, const uint32_t* info_chroma,
                          const int16_t* mv16, const int32_t* mv32, const uint8_t* ctu_slice) {
@@ -906,6 +920,9 @@ int ilf_set_deblock_info(ilf_ctx* ctx, int slot, const ilf_deblock_params* param
   s.dev.mv32 = mv32 ? (const int32_t*)s.mv : nullptr;
   s.dev.ctu_slice = ctu_slice ? s.ctu_slice : nullptr;
   s.dev.db_params = s.db_params;
+  // A chroma edge is filtered only when a side is intra (bS == 2, LoopFilter.cpp:769): without an intra unit in the layer the
+  // chroma decisions read, deblocking leaves both chroma planes as uploaded, and run_stage skips them.
+  s.db_chroma = any_intra(info_chroma ? info_chroma : info, (size_t)ctx->g.units_w * ctx->g.units_h);
   s.has_db = true;
   CU(ctx, cudaEventRecord(s.ev_side[0], ctx->s_up));
   return push_desc(ctx, slot);
@@ -1051,7 +1068,7 @@ static int run_stage(ilf_ctx* ctx, int first, int n, int stage, cudaStream_t str
       unsigned v = 0;
       const bool mine = !lane_of || lane_of[c0 + i - first] == lane;
       for (int p = 0; p < 3; p++) {
-        on[i][p] = mine && (stage == 0 ? true : (stage == 1 ? s.sao_on[p] : s.alf_on[p]));
+        on[i][p] = mine && (stage == 0 ? (p == 0 || s.db_chroma) : (stage == 1 ? s.sao_on[p] : s.alf_on[p]));
         v |= (unsigned)s.result_buf[p] << (2 * p);
         if (!on[i][p]) { v |= 1u << (6 + p); continue; }   // (a slot of another lane is not launched at all: compact() below)
         s.result_buf[p] = s.result_buf[p] == 1 ? 2 : 1;
@@ -1166,7 +1183,7 @@ int ilf_run(ilf_ctx* ctx, int first_slot, int num_slots, unsigned stages) {
         int c = 0;
         for (int p = 0; p < 3; p++) {
           const int w = p == 0 ? 4 : 1;
-          if (stages & ILF_STAGE_DEBLOCK) c += w;
+          if ((stages & ILF_STAGE_DEBLOCK) && (p == 0 || s.db_chroma)) c += w;
           if ((stages & ILF_STAGE_SAO) && s.sao_on[p]) c += w;
           if ((stages & ILF_STAGE_ALF) && s.alf_on[p]) c += 2 * w;
         }

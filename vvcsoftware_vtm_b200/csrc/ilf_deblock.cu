@@ -37,6 +37,8 @@
 // luma horizontal (4 edge rows x 32 = 128), chroma horizontal (2 x 2 x 32 = 128) -- so edge flag, bS, QP, tc and beta are
 // derived once per segment and segments without an edge cost a few instructions.  The fifth warp has vertical tasks only: its
 // first thread draws the next tile from the queue while the other four run the horizontal pass.
+// A chroma plane with the skip bit in its picture's control word (ilf_set_deblock_info found no intra unit: chroma is filtered
+// for bS == 2 only, so the plane would come out unchanged) is not loaded, filtered or stored; it stays in the upload buffer.
 #include <algorithm>
 #include <cstdlib>
 
@@ -275,22 +277,26 @@ __global__ void __launch_bounds__(NTHREADS, ILF_DB_MIN_CTAS) deblock_kernel(Geom
   auto pack_id = [&](int id) { if (id >= total) return -1; const int tx = id % ntx, r = id / ntx; return tx | (r % bands) << 8 | (r / bands) << 20; };
   auto decode = [&](int id, int& z, int& ty, int& tx) { tx = id & 255; ty = (id >> 8) & 4095; z = id >> 20; };
   // The boxes of a tile are issued by the first lanes of the CTA's warps, one part each, so that their descriptor fetches
-  // overlap: part 0 arms the barrier and loads luma, 1 both chroma planes, 2 the unit grids, 3 motion.
+  // overlap: part 0 arms the barrier and loads luma, 1 both chroma planes, 2 the unit grids, 3 motion.  A skipped chroma plane
+  // (a picture without an intra unit: no chroma edge is filtered) is neither loaded nor stored.  The tile may belong to another
+  // picture than sh.cur_slot, so its control word is read from bc.
   auto issue_part = [&](int id, int si, int part) {  // tile id into stage si
     int z, ty, tx;
     decode(id, z, ty, tx);
     const SlotDev& sd = slots[first_slot + bc.slot[z]];
-    const int src_b = ctl_src(bc.v[z], 0);
+    const unsigned c = bc.v[z];
+    const int src_b = ctl_src(c, 0);
     const int y0 = ty * TH - 4, cy0 = ty * CTH - 2, uy0 = ty * UH - 1;  // band origin (local rows)
     const bool has_ctree = (part == 0 || part == 2) ? (z == sh.cur_slot ? sh.ctree != 0 : sd.info_c != nullptr) : false;
     Stage<MV>* st = reinterpret_cast<Stage<MV>*>(smem + si * STRIDE);
     uint64_t* bar = &full[si];
     if (part == 0) {
-      ring::mbar_expect_tx(bar, (uint32_t)stage_tx_bytes<MV>(has_ctree));
+      const int skipped = (int)ctl_skip(c, 1) + (int)ctl_skip(c, 2);
+      ring::mbar_expect_tx(bar, (uint32_t)(stage_tx_bytes<MV>(has_ctree) - skipped * (CTH * BCW * 2)));
       ring::tma_load_3d(&st->y[0][0], &sd.tm_db[0], bar, tx * TW - 8, y0, src_b);
     } else if (part == 1) {
-      ring::tma_load_3d(&st->c[0][0][0], &sd.tm_db[1], bar, tx * CTW - 8, cy0, src_b);
-      ring::tma_load_3d(&st->c[1][0][0], &sd.tm_db[2], bar, tx * CTW - 8, cy0, src_b);
+      if (!ctl_skip(c, 1)) ring::tma_load_3d(&st->c[0][0][0], &sd.tm_db[1], bar, tx * CTW - 8, cy0, src_b);
+      if (!ctl_skip(c, 2)) ring::tma_load_3d(&st->c[1][0][0], &sd.tm_db[2], bar, tx * CTW - 8, cy0, src_b);
     } else if (part == 2) {
       ring::tma_load_3d(&st->info[0][0], &sd.tm_info, bar, tx * UW - 4, uy0, 0);
       if (has_ctree) ring::tma_load_3d(&st->info_c[0][0], &sd.tm_info_c, bar, tx * UW - 4, uy0, 0);
@@ -332,7 +338,7 @@ __global__ void __launch_bounds__(NTHREADS, ILF_DB_MIN_CTAS) deblock_kernel(Geom
       if (tid == 0) {
         sh.ctu_slice = __ldg(&sd.db_params->num_slices) == 1 ? nullptr : sd.ctu_slice;  // one slice: no per-CTU lookup
         const unsigned c = bc.v[z];
-        const int db = ctl_dst(c, 0);  // deblocking starts from the uploaded picture: all planes in one buffer
+        const int db = ctl_dst(c, 0);  // deblocking starts from the uploaded picture: all planes in one buffer (skipped planes are not written)
         sh.ctl = c; sh.dst[0] = sd.buf[db][0]; sh.dst[1] = sd.buf[db][1]; sh.dst[2] = sd.buf[db][2];
         sh.ctree = sd.info_c != nullptr;
         sh.cur_slot = z;
@@ -375,9 +381,10 @@ __global__ void __launch_bounds__(NTHREADS, ILF_DB_MIN_CTAS) deblock_kernel(Geom
         }
       }
       // ---- vertical edges, chroma: task = one unit = 2 lines x 4 samples.  2 planes x 9 edge columns x 8 unit rows (tasks 128 .. 143: edge 8) ----
-      if (tid >= VC0 && tid < VC0 + 2 * 9 * 8) {
-        const int task = tid - VC0;
-        const int pl = task < 128 ? (task >> 6) : ((task - 128) >> 3), k = task < 128 ? ((task >> 3) & 7) : 8, sg = task & 7;
+      const int task = tid - VC0;
+      const int pl = task < 128 ? (task >> 6) : ((task - 128) >> 3);
+      if (tid >= VC0 && task < 2 * 9 * 8 && !ctl_skip(sh.ctl, 1 + pl)) {
+        const int k = task < 128 ? ((task >> 3) & 7) : 8, sg = task & 7;
         bool no_p, no_q;
         const int tc = chroma_tc(t.cinfo(sg, 4 * k), t.cinfo(sg, 4 * k - 1), g, sh, true, pl, 2 * (cx0 + 8 * k), 2 * (cy0 + 2 * sg), no_p, no_q);
         if (tc >= 0) {
@@ -436,7 +443,7 @@ __global__ void __launch_bounds__(NTHREADS, ILF_DB_MIN_CTAS) deblock_kernel(Geom
     }
     // ---- horizontal edges, chroma: task = 2 columns x 8 rows (the edge lies between rows 1 and 2), filtered and stored.
     //      2 planes x 2 row groups x 32 unit columns ----
-    if (tid >= HC0 && tid < HC0 + 128) {
+    if (tid >= HC0 && tid < HC0 + 128 && !ctl_skip(sh.ctl, 1 + ((tid - HC0) >> 6))) {
       const int ht = tid - HC0;
       const int pl = ht >> 6, h = (ht >> 5) & 1, u = ht & 31;
       const int16_t* sp = t.ch(pl, 8 * h, 2 * u);
