@@ -236,7 +236,7 @@ int ilf_alf_classify(ilf_ctx* ctx, int slot, uint8_t* out);
  * CURRENT state of the slots' pictures (after ilf_deblock: the deblocked picture, which is what the encoder measures);
  * ilf_get_sao_stats copies a slot's result to the host: out[num_ctus][3][5][64] int64, per CTU, component and SAO type
  * diff[32] followed by count[32] -- the memory layout of SAOStatData (EncSampleAdaptiveOffset.h:53-57).
- * Not available on band contexts.
+ * ilf_set_original refuses band contexts; a band context takes its original with ilf_set_original_band (band section below).
  * ------------------------------------------------------------------------------------------- */
 #define ILF_SAO_STATS_WORDS (5 * 64)
 int ilf_set_original(ilf_ctx* ctx, int slot, const int16_t* y, ptrdiff_t stride_y, const int16_t* cb, ptrdiff_t stride_cb, const int16_t* cr,
@@ -253,7 +253,7 @@ int ilf_get_sao_stats(ilf_ctx* ctx, int slot, int64_t* out);
  *   luma  [25 classes][105]   7x7 shape: E[k][l] for k <= l row-major (91), y[k] (13), pixAcc (1)
  *   Cb    [36], Cr [36]       5x5 shape: E (28), y (7), pixAcc
  * The luma statistics of the 5x5 shape (m_filterShapes[CHANNEL_TYPE_LUMA][0]) are rows / columns {2, 5, 6, 7, 10, 11, 12} of the 7x7
- * record: under every transposition the 5x5 taps are those taps of the 7x7 diamond.  Not available on band contexts.
+ * record: under every transposition the 5x5 taps are those taps of the 7x7 diamond.  On a band context: after ilf_set_original_band.
  * ------------------------------------------------------------------------------------------- */
 #define ILF_ALF_STATS_WORDS (25 * 105 + 36 + 36)
 int ilf_alf_stats(ilf_ctx* ctx, int first_slot, int num_slots);
@@ -275,7 +275,7 @@ int ilf_get_alf_stats(ilf_ctx* ctx, int slot, int64_t* out);
  * ilf_download / ilf_run after a search give what they gave before it.
  * Errors: ILF_ERR_ARG for a bad slot range, num_cands outside 1..ILF_DEBLOCK_SEARCH_MAX, NULL pointers or a shift outside 0..31;
  * ILF_ERR_STATE for a slot without an upload, without deblocking side information or without ilf_set_original since its upload,
- * and on band contexts.  Ordering: the search waits for the slots' uploads and side information, runs on the context's stream and
+ * and on a band context without ilf_set_original_band since its upload.  Ordering: the search waits for the slots' uploads and side information, runs on the context's stream and
  * is waited for by the slots' next uploads.  ilf_get_deblock_search synchronises and returns the K of the slot's last search
  * (ILF_ERR_STATE before any search, ILF_ERR_ARG when max_cands < K).
  * ------------------------------------------------------------------------------------------- */
@@ -297,7 +297,7 @@ int ilf_get_deblock_search(ilf_ctx* ctx, int slot, uint64_t* out /* [K][3] */, i
  *   ilf_download_extended  ilf_download into planes that have `margin` luma (margin / 2 chroma) samples of room on every side (a
  *                          PelStorage of Picture::create, Picture.cpp:791-…), and the margins filled by replication as
  *                          Picture::extendPicBorder does (Picture.cpp:996-1040) -- the caller marks the picture as extended.
- * Not available on band contexts.
+ * Both refuse band contexts: their twins are ilf_picture_hash_band + ilf_hash_combine and ilf_download_band_extended (band section).
  * ------------------------------------------------------------------------------------------- */
 #define ILF_HASH_CRC 1
 #define ILF_HASH_CHECKSUM 2
@@ -362,6 +362,33 @@ void* ilf_stream(ilf_ctx* ctx); /* cudaStream_t of the context */
  *   ilf_download_band   the band's own rows of the filtered picture
  * Side information of a band context: unit grids cover the rows the context HOLDS (ilf_get_band: first_row,
  * num_rows); ctu_slice, SAO parameters and ALF flags cover the full picture.
+ *
+ * Consumers of the filtered picture on a band context (the band twins of the post-filter and encoder entry points above):
+ *   ilf_picture_hash_band  CRC and checksum of the band's OWN rows of the slot's current picture, as a part that ilf_hash_combine
+ *                          folds with the other bands' parts into ilf_picture_hash of the whole picture.  crc[p] is what the rows
+ *                          contribute to the CRC register from a ZERO register, sum[p] the checksum partial sum (row masks in picture
+ *                          coordinates).  The part carries the picture geometry, so parts can travel between processes as bytes.
+ *                          Waits for the slot's upload and last run, like ilf_picture_hash, and returns after a synchronise.
+ *   ilf_hash_combine       host only, no context: out[Y, Cb, Cr] of ILF_HASH_CRC / ILF_HASH_CHECKSUM from parts in any order.
+ *                          ILF_ERR_ARG unless the parts tile [0, height) exactly (no gap, no overlap), share geometry and bit depths,
+ *                          num_parts >= 1, kind is valid and no pointer is NULL.
+ *   ilf_download_band_extended  ilf_download_band with Picture::extendPicBorder's margins (see ilf_download_extended): the pointers
+ *                          address the band's first own row inside the caller's FULL-picture planes, which have `margin` luma
+ *                          (margin / 2 chroma) samples of room on every side.  Writes the own rows and their left / right margins,
+ *                          the top margin rows (and corners) only when the band owns picture row 0, the bottom ones only when it
+ *                          owns the last row; no other row.  Once every band has run into the same planes they equal
+ *                          ilf_download_extended of the whole picture.  margin must be even and >= 0.
+ *   ilf_set_original_band  the source picture of the band's OWN rows (host planes as ilf_upload_band) and ctu_avail of the FULL
+ *                          picture (as ilf_set_original).  After it (since the slot's upload) ilf_sao_stats, ilf_alf_stats,
+ *                          ilf_deblock_search and their ilf_get_* accept the band slot:
+ *                            statistics records are those of the band's own CTUs, num_ctu_rows x ctus_w records in raster order
+ *                            (in band order they concatenate to the whole picture's records); ilf_alf_classify returns the held
+ *                            unit rows, whose own rows equal the whole picture's; the search sums cover the own rows (summed over
+ *                            the bands they are the whole picture's sums).
+ *                          The kernels read the halo rows of the slot's current picture, so the halo must have been exchanged since
+ *                          the upload (ilf_band_exchange), as for ilf_run.
+ * ilf_picture_hash_band, ilf_download_band_extended and ilf_set_original_band return ILF_ERR_STATE on a whole-picture context
+ * and before the slot's upload.
  * ------------------------------------------------------------------------------------------- */
 typedef struct {
   int32_t first_ctu_row; /* first CTU row owned by this band */
@@ -382,6 +409,19 @@ int ilf_band_export(ilf_ctx* ctx, int slot, ilf_band_handle* out);
 int ilf_band_connect(ilf_ctx* ctx, int slot, int side, const ilf_band_handle* neighbour);
 int ilf_band_exchange(ilf_ctx* ctx, int slot);
 int ilf_band_exchange_batch(ilf_ctx* ctx, int first_slot, int num_slots); /* the same for several slots with one launch */
+
+typedef struct {
+  int32_t width, height, bd_luma, bd_chroma; /* full picture, copied from the context                                   */
+  int32_t first_row, num_rows;               /* luma picture rows covered: the band's own rows                          */
+  uint32_t crc[3];                           /* per plane: CRC register contribution of these rows from a ZERO register */
+  uint32_t sum[3];                           /* per plane: checksum partial sum (mod 2^32), masks in picture coordinates */
+} ilf_hash_part;
+int ilf_picture_hash_band(ilf_ctx* ctx, int slot, ilf_hash_part* out);
+int ilf_hash_combine(const ilf_hash_part* parts, int num_parts, int kind, uint32_t out[3]);
+int ilf_download_band_extended(ilf_ctx* ctx, int slot, int16_t* y, ptrdiff_t stride_y, int16_t* cb, ptrdiff_t stride_cb, int16_t* cr,
+                               ptrdiff_t stride_cr, int margin);
+int ilf_set_original_band(ilf_ctx* ctx, int slot, const int16_t* y, ptrdiff_t stride_y, const int16_t* cb, ptrdiff_t stride_cb, const int16_t* cr,
+                          ptrdiff_t stride_cr, const uint8_t* ctu_avail /* [ctus_h*ctus_w], full picture */);
 
 #ifdef __cplusplus
 }

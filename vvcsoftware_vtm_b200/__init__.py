@@ -4,5 +4,5 @@ The product is the C-ABI CUDA library ``libilf_b200.so`` (include/ilf_b200.h, cs
 keeps the reference's LoopFilter / SampleAdaptiveOffset / AdaptiveLoopFilter class interfaces (shim/).
 This Python package is a thin ctypes binding of the C ABI used by the tests and bench.py.
 """
-from .ilf import BAND_ABOVE, BAND_BELOW, IlfError, InLoopFilter, lib_path, load_library, pinned_planes  # noqa: F401
+from .ilf import BAND_ABOVE, BAND_BELOW, IlfError, IlfHashPart, InLoopFilter, hash_combine, lib_path, load_library, pinned_planes  # noqa: F401
 from . import bands  # noqa: F401

@@ -16,6 +16,8 @@
 // as a low and a high word: 64-bit shared atomics are CAS loops on sm_100a, 32-bit ones are native), (3) after a barrier the
 // non-zero accumulators go to L2 with one 64-bit reduction each.  A CTA sends a few hundred reductions instead of 105 per block
 // (26 880), which is what bounded the first version of this kernel (14 ms for the luma planes of 17 4K pictures).
+// A band context measures its own rows: tiles start at its first own row, border clamps and CTU records use picture coordinates,
+// plane rows are addressed from the first held row.  The strip reaches 3 rows (chroma 2) beyond the own rows, inside the halo.
 #include <algorithm>
 #include "ilf_common.cuh"
 
@@ -54,9 +56,10 @@ __global__ void __launch_bounds__(NT, 3) alf_stats_kernel(Geom g, const SlotDev*
   const unsigned ctl = bc.v[blockIdx.z];
   const int sh = plane ? 1 : 0;
   const int w = g.width >> sh, h = g.height >> sh, pitch = plane ? g.pitch_c : g.pitch_y;
+  const int r0 = g.row0 >> sh, yend = (g.out_row0 + g.out_rows) >> sh;   // first held row, end of the own rows (picture rows)
   const int16_t* __restrict__ rec = sd.buf[ctl_src(ctl, plane)][plane];
   const int16_t* __restrict__ org = sd.org[plane];
-  const int x0 = blockIdx.x * ST_W, y0 = blockIdx.y * ST_H;
+  const int x0 = blockIdx.x * ST_W, y0 = (g.out_row0 >> sh) + blockIdx.y * ST_H;
   const int ctu_log2 = g.ctu_log2 - sh;
   // CTUs under this tile: sets_x across, sets_y down (1 x 1 for the 128-sample CTUs of the reference's configurations)
   const int sets_x = max(1, ST_W >> ctu_log2), sets_y = max(1, ST_H >> ctu_log2);
@@ -70,7 +73,7 @@ __global__ void __launch_bounds__(NT, 3) alf_stats_kernel(Geom g, const SlotDev*
     if (i < TR * CH) {
       const int ty = i / CH, cx = i - ty * CH;
       const int y = min(max(y0 + ty - HALF, 0), h - 1), xs = x0 - 8 + 8 * cx;
-      const int16_t* row = rec + (size_t)y * pitch;
+      const int16_t* row = rec + (size_t)(y - r0) * pitch;
       uint4 v;
       if (xs >= 0 && xs + 8 <= w) v = __ldg(reinterpret_cast<const uint4*>(row + xs));
       else {
@@ -89,15 +92,15 @@ __global__ void __launch_bounds__(NT, 3) alf_stats_kernel(Geom g, const SlotDev*
   for (int it = 0; it < (ST_H * (ST_W / 8)) / NT; it++) {
     const int i = threadIdx.x + it * NT;
     const int ty = i / (ST_W / 8), cx = i - ty * (ST_W / 8);
-    if (y0 + ty < h && x0 + 8 * cx < w)   // rows are padded to 64 samples: a chunk that starts inside the picture is readable
-      *reinterpret_cast<uint4*>(sorg + ty * ST_W + 8 * cx) = __ldg(reinterpret_cast<const uint4*>(org + (size_t)(y0 + ty) * pitch + x0 + 8 * cx));
+    if (y0 + ty < yend && x0 + 8 * cx < w)   // rows are padded to 64 samples: a chunk that starts inside the picture is readable
+      *reinterpret_cast<uint4*>(sorg + ty * ST_W + 8 * cx) = __ldg(reinterpret_cast<const uint4*>(org + (size_t)(y0 + ty - r0) * pitch + x0 + 8 * cx));
   }
   __syncthreads();
   const int bj = threadIdx.x % (ST_W / 4), bi = threadIdx.x / (ST_W / 4);
   const int bx = x0 + 4 * bj, by = y0 + 4 * bi;
-  const bool valid = bx < w && by < h;
+  const bool valid = bx < w && by < yend;
   int cls = 0;
-  if (CLASSES && valid) cls = sd.alf_class[(size_t)(by >> 2) * g.units_w + (bx >> 2)];
+  if (CLASSES && valid) cls = sd.alf_class[(size_t)((by - r0) >> 2) * g.units_w + (bx >> 2)];
   const int t = cls >> 5;
   // the block's transposed frame: sample (u, v) sits at P0 + u ex + v ey; transposeIdx 0: ex = (1, 0), ey = (0, 1); 1: (0, 1), (1, 0);
   // 2: (-1, 0), (0, 1) from the block's right edge; 3: (0, -1), (1, 0) from its bottom edge (EncAdaptiveLoopFilter.cpp:1463-1510)
@@ -169,7 +172,8 @@ __global__ void __launch_bounds__(NT, 3) alf_stats_kernel(Geom g, const SlotDev*
     if (!(l | hgh)) continue;
     const int k = e / WORDS, i = e - k * WORDS;
     const int st = CLASSES ? k / 25 : k, c = CLASSES ? k - st * 25 : 0;
-    const int cx = (x0 >> ctu_log2) + st % sets_x, cy = (y0 >> ctu_log2) + st / sets_x;
+    // record row among the own CTU rows: the own rows start on a CTU row, so it follows from the tile row alone
+    const int cx = (x0 >> ctu_log2) + st % sets_x, cy = (int)((blockIdx.y * ST_H) >> ctu_log2) + st / sets_x;
     long long* out = sd.alf_stats + (size_t)(cy * g.ctus_w + cx) * ILF_ALF_STATS_WORDS + (plane == 0 ? (size_t)c * WORDS : (size_t)(25 * 105 + (plane - 1) * 36)) + i;
     atomicAdd(reinterpret_cast<unsigned long long*>(out), ((unsigned long long)hgh << 32) | l);
   }
@@ -182,8 +186,8 @@ void launch_alf_stats(const Geom& g, const SlotDev* slots, int first_slot, int n
   auto sets = [&](int sh) { const int l = g.ctu_log2 - sh; return std::max(1, ST_W >> l) * std::max(1, ST_H >> l); };
   const int smem_y = sets(0) * 25 * Shape<3>::WORDS * 8, smem_c = sets(1) * Shape<2>::WORDS * 8;
   if (smem_y > 36 * 1024) cudaFuncSetAttribute(alf_stats_kernel<3, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_y);   // CTUs below 128: several records per tile
-  alf_stats_kernel<3, true><<<dim3((g.width + ST_W - 1) / ST_W, (g.height + ST_H - 1) / ST_H, num_slots), NT, smem_y, st>>>(g, slots, first_slot, ctl, 0);
-  const dim3 gc((g.width / 2 + ST_W - 1) / ST_W, (g.height / 2 + ST_H - 1) / ST_H, num_slots);
+  alf_stats_kernel<3, true><<<dim3((g.width + ST_W - 1) / ST_W, (g.out_rows + ST_H - 1) / ST_H, num_slots), NT, smem_y, st>>>(g, slots, first_slot, ctl, 0);
+  const dim3 gc((g.width / 2 + ST_W - 1) / ST_W, (g.out_rows / 2 + ST_H - 1) / ST_H, num_slots);
   alf_stats_kernel<2, false><<<gc, NT, smem_c, st>>>(g, slots, first_slot, ctl, 1);
   alf_stats_kernel<2, false><<<gc, NT, smem_c, st>>>(g, slots, first_slot, ctl, 2);
 }

@@ -793,18 +793,24 @@ static int order_after_run(ilf_ctx* ctx, Slot& s, cudaStream_t st) {
   return ILF_OK;
 }
 
+// The slot's current planes for a hash, with the compute stream ordered after the slot's upload and last run.
+static int hash_planes(ilf_ctx* ctx, Slot& s, const int16_t* planes[3]) {
+  CU(ctx, cudaSetDevice(ctx->cfg.device));
+  if (!ctx->hash_scratch) CU(ctx, cudaMalloc(&ctx->hash_scratch, (6 * 16384 + 8) * sizeof(uint32_t)));
+  if (s.h2d_pending) CU(ctx, cudaStreamWaitEvent(ctx->stream, s.ev_up, 0));   // a picture no stage has touched yet
+  if (int rc = order_after_run(ctx, s, ctx->stream)) return rc;
+  for (int p = 0; p < 3; p++) planes[p] = plane_ptr(ctx, s, s.result_buf[p], p);
+  return ILF_OK;
+}
+
 int ilf_picture_hash(ilf_ctx* ctx, int slot, int kind, uint32_t out[3]) {
   if (int rc = check_slot(ctx, slot)) return rc;
   if (!out || (kind != ILF_HASH_CRC && kind != ILF_HASH_CHECKSUM)) return fail(ctx, ILF_ERR_ARG, "bad hash kind or null output");
   if (ctx->is_band) return fail(ctx, ILF_ERR_STATE, "a band context holds a part of the picture only");
   Slot& s = ctx->slots[slot];
   if (!s.uploaded) return fail(ctx, ILF_ERR_STATE, "slot %d: hash before upload", slot);
-  CU(ctx, cudaSetDevice(ctx->cfg.device));
-  if (!ctx->hash_scratch) CU(ctx, cudaMalloc(&ctx->hash_scratch, (6 * 16384 + 8) * sizeof(uint32_t)));
-  if (s.h2d_pending) CU(ctx, cudaStreamWaitEvent(ctx->stream, s.ev_up, 0));   // a picture no stage has touched yet
-  if (int rc = order_after_run(ctx, s, ctx->stream)) return rc;
   const int16_t* planes[3];
-  for (int p = 0; p < 3; p++) planes[p] = plane_ptr(ctx, s, s.result_buf[p], p);
+  if (int rc = hash_planes(ctx, s, planes)) return rc;
   uint32_t crc[3], sum[3];
   CU(ctx, picture_hash(ctx->g, planes, ctx->hash_scratch, ctx->stream, crc, sum));
   ctx->launches += 2;
@@ -812,22 +818,39 @@ int ilf_picture_hash(ilf_ctx* ctx, int slot, int kind, uint32_t out[3]) {
   return ILF_OK;
 }
 
+// The band's own rows as a part of the picture's hash (ilf_hash_combine in ilf_hash.cu folds the parts).
+int ilf_picture_hash_band(ilf_ctx* ctx, int slot, ilf_hash_part* out) {
+  if (int rc = check_slot(ctx, slot)) return rc;
+  if (!out) return fail(ctx, ILF_ERR_ARG, "null output");
+  if (!ctx->is_band) return fail(ctx, ILF_ERR_STATE, "not a band context (ilf_picture_hash hashes the whole picture)");
+  Slot& s = ctx->slots[slot];
+  if (!s.uploaded) return fail(ctx, ILF_ERR_STATE, "slot %d: hash before upload", slot);
+  const int16_t* planes[3];
+  if (int rc = hash_planes(ctx, s, planes)) return rc;
+  const Geom& g = ctx->g;
+  ilf_hash_part part;
+  memset(&part, 0, sizeof(part));
+  part.width = g.width; part.height = g.height; part.bd_luma = g.bd_luma; part.bd_chroma = g.bd_chroma;
+  part.first_row = g.out_row0; part.num_rows = g.out_rows;
+  CU(ctx, hash_rows(g, planes, ctx->hash_scratch, ctx->stream, g.out_row0 - g.row0, g.out_rows, g.out_row0, part.crc, part.sum));
+  ctx->launches += 2;
+  *out = part;
+  return ILF_OK;
+}
+
 // Reference border extension on the way down (Picture::extendPicBorder, Picture.cpp:996-1040): the planes are downloaded into buffers
 // that have `margin` luma (margin / 2 chroma) samples of room on every side, and the margins are filled by replication -- rows by
 // the copy threads, so the decoder's own extendPicBorder pass over the picture is not needed any more.
-int ilf_download_extended(ilf_ctx* ctx, int slot, int16_t* y, ptrdiff_t sy, int16_t* cb, ptrdiff_t scb, int16_t* cr, ptrdiff_t scr, int margin) {
-  if (margin < 0 || (margin & 1)) return fail(ctx, ILF_ERR_ARG, "margin must be even and >= 0");
-  if (ctx && ctx->is_band) return fail(ctx, ILF_ERR_STATE, "not available on band contexts");
-  if (int rc = ilf_download(ctx, slot, y, sy, cb, scb, cr, scr)) return rc;
+// Fills the left / right margins of the n luma rows (n / 2 chroma rows) the plane pointers start at, and the margin rows above the
+// first row (with the corners) when `top`, those below the last row when `bottom`.
+static void extend_margins(ilf_ctx* ctx, int16_t* const planes[3], const ptrdiff_t strides[3], int margin, int n, bool top, bool bottom) {
   const Geom& g = ctx->g;
-  int16_t* planes[3] = {y, cb, cr};
-  const ptrdiff_t strides[3] = {sy, scb, scr};
   // left / right margins of every row, in row chunks on the copy threads; then the top / bottom rows (which include the corners)
   struct Job { int plane, row0, rows; };
   Job jobs[COPY_CHUNKS_MAX];
   int nj = 0;
   for (int p = 0; p < 3; p++) {
-    const int h = p ? g.height / 2 : g.height, pieces = std::max(1, std::min(p ? 2 : 8, h / 64));
+    const int h = p ? n / 2 : n, pieces = std::max(1, std::min(p ? 2 : 8, h / 64));
     for (int i = 0; i < pieces; i++) jobs[nj++] = {p, (int)((long long)h * i / pieces), (int)((long long)h * (i + 1) / pieces) - (int)((long long)h * i / pieces)};
   }
   auto sides = [&](int i) {
@@ -842,14 +865,35 @@ int ilf_download_extended(ilf_ctx* ctx, int slot, int16_t* y, ptrdiff_t sy, int1
   if (ctx->copy_pool.threads() > 1) { ctx->copy_pool.start(nj, sides); ctx->copy_pool.wait(); }
   else for (int i = 0; i < nj; i++) sides(i);
   for (int p = 0; p < 3; p++) {
-    const int w = p ? g.width / 2 : g.width, h = p ? g.height / 2 : g.height, m = p ? margin / 2 : margin;
-    int16_t* top = planes[p] - m;
-    int16_t* bot = planes[p] + (ptrdiff_t)(h - 1) * strides[p] - m;
+    const int w = p ? g.width / 2 : g.width, h = p ? n / 2 : n, m = p ? margin / 2 : margin;
+    int16_t* first = planes[p] - m;
+    int16_t* last = planes[p] + (ptrdiff_t)(h - 1) * strides[p] - m;
     for (int r = 1; r <= m; r++) {
-      memcpy(top - (ptrdiff_t)r * strides[p], top, sizeof(int16_t) * (size_t)(w + 2 * m));
-      memcpy(bot + (ptrdiff_t)r * strides[p], bot, sizeof(int16_t) * (size_t)(w + 2 * m));
+      if (top) memcpy(first - (ptrdiff_t)r * strides[p], first, sizeof(int16_t) * (size_t)(w + 2 * m));
+      if (bottom) memcpy(last + (ptrdiff_t)r * strides[p], last, sizeof(int16_t) * (size_t)(w + 2 * m));
     }
   }
+}
+
+int ilf_download_extended(ilf_ctx* ctx, int slot, int16_t* y, ptrdiff_t sy, int16_t* cb, ptrdiff_t scb, int16_t* cr, ptrdiff_t scr, int margin) {
+  if (margin < 0 || (margin & 1)) return fail(ctx, ILF_ERR_ARG, "margin must be even and >= 0");
+  if (ctx && ctx->is_band) return fail(ctx, ILF_ERR_STATE, "not available on band contexts");
+  if (int rc = ilf_download(ctx, slot, y, sy, cb, scb, cr, scr)) return rc;
+  int16_t* const planes[3] = {y, cb, cr};
+  const ptrdiff_t strides[3] = {sy, scb, scr};
+  extend_margins(ctx, planes, strides, margin, ctx->g.height, true, true);
+  return ILF_OK;
+}
+
+// The band's own rows and their margins; the rows above / below the picture only from the band that owns its first / last row.
+int ilf_download_band_extended(ilf_ctx* ctx, int slot, int16_t* y, ptrdiff_t sy, int16_t* cb, ptrdiff_t scb, int16_t* cr, ptrdiff_t scr, int margin) {
+  if (margin < 0 || (margin & 1)) return fail(ctx, ILF_ERR_ARG, "margin must be even and >= 0");
+  if (ctx && !ctx->is_band) return fail(ctx, ILF_ERR_STATE, "not a band context (ilf_download_extended downloads the whole picture)");
+  if (int rc = ilf_download_band(ctx, slot, y, sy, cb, scb, cr, scr)) return rc;
+  const Geom& g = ctx->g;
+  int16_t* const planes[3] = {y, cb, cr};
+  const ptrdiff_t strides[3] = {sy, scb, scr};
+  extend_margins(ctx, planes, strides, margin, g.out_rows, g.out_row0 == 0, g.out_row0 + g.out_rows == g.height);
   return ILF_OK;
 }
 
@@ -1250,9 +1294,10 @@ int ilf_alf_classify(ilf_ctx* ctx, int slot, uint8_t* out) {
 // ---------------------------------------------------------------------------------------------------------------
 // Encoder SAO statistics (include/ilf_b200.h; EncSampleAdaptiveOffset::getStatistics)
 // ---------------------------------------------------------------------------------------------------------------
-int ilf_set_original(ilf_ctx* ctx, int slot, const int16_t* y, ptrdiff_t sy, const int16_t* cb, ptrdiff_t scb, const int16_t* cr, ptrdiff_t scr, const uint8_t* ctu_avail) {
-  if (int rc = check_slot(ctx, slot)) return rc;
-  if (ctx->is_band) return fail(ctx, ILF_ERR_STATE, "SAO statistics are not available on band contexts");
+// Copies the source picture's LOCAL luma rows [first, first + n) of the held region (chroma rows halved) and the full picture's
+// ctu_avail.  The original lives in the held-row layout of the slot's buffers, so the kernels address it as they address the picture.
+static int set_original_rows(ilf_ctx* ctx, int slot, const int16_t* y, ptrdiff_t sy, const int16_t* cb, ptrdiff_t scb, const int16_t* cr, ptrdiff_t scr,
+                             const uint8_t* ctu_avail, int first, int n) {
   if (!y || !cb || !cr || !ctu_avail) return fail(ctx, ILF_ERR_ARG, "null pointer");
   Slot& s = ctx->slots[slot];
   const Geom& g = ctx->g;
@@ -1269,9 +1314,10 @@ int ilf_set_original(ilf_ctx* ctx, int slot, const int16_t* y, ptrdiff_t sy, con
   const int16_t* srcs[3] = {y, cb, cr};
   const ptrdiff_t strides[3] = {sy, scb, scr};
   for (int p = 0; p < 3; p++) {
-    const int w = p ? g.width / 2 : g.width, h = p ? g.height / 2 : g.height, pitch = p ? g.pitch_c : g.pitch_y;
+    const int sh = p ? 1 : 0, w = g.width >> sh, h = n >> sh, pitch = p ? g.pitch_c : g.pitch_y;
     // pageable sources are staged by the runtime (the call returns when the source may be reused); page-locked ones are asynchronous
-    CU(ctx, cudaMemcpy2DAsync(const_cast<int16_t*>(s.dev.org[p]), (size_t)pitch * 2, srcs[p], (size_t)strides[p] * 2, (size_t)w * 2, h, cudaMemcpyHostToDevice, ctx->s_up));
+    CU(ctx, cudaMemcpy2DAsync(const_cast<int16_t*>(s.dev.org[p]) + (size_t)(first >> sh) * pitch, (size_t)pitch * 2, srcs[p], (size_t)strides[p] * 2, (size_t)w * 2, h,
+                              cudaMemcpyHostToDevice, ctx->s_up));
   }
   CU(ctx, cudaMemcpyAsync(s.stats_avail, ctu_avail, ctx->num_ctus, cudaMemcpyHostToDevice, ctx->s_up));
   if (!is_pinned(ctu_avail)) CU(ctx, cudaStreamSynchronize(ctx->s_up));  // the caller may reuse ctu_avail
@@ -1280,6 +1326,27 @@ int ilf_set_original(ilf_ctx* ctx, int slot, const int16_t* y, ptrdiff_t sy, con
   return push_desc(ctx, slot);
 }
 
+int ilf_set_original(ilf_ctx* ctx, int slot, const int16_t* y, ptrdiff_t sy, const int16_t* cb, ptrdiff_t scb, const int16_t* cr, ptrdiff_t scr, const uint8_t* ctu_avail) {
+  if (int rc = check_slot(ctx, slot)) return rc;
+  if (ctx->is_band) return fail(ctx, ILF_ERR_STATE, "SAO statistics are not available on band contexts");
+  return set_original_rows(ctx, slot, y, sy, cb, scb, cr, scr, ctu_avail, 0, ctx->g.height);
+}
+
+// Host planes cover the band's OWN rows, as for ilf_upload_band; the statistics and the search read the original at own samples only.
+int ilf_set_original_band(ilf_ctx* ctx, int slot, const int16_t* y, ptrdiff_t sy, const int16_t* cb, ptrdiff_t scb, const int16_t* cr, ptrdiff_t scr,
+                          const uint8_t* ctu_avail) {
+  if (int rc = check_slot(ctx, slot)) return rc;
+  if (!ctx->is_band) return fail(ctx, ILF_ERR_STATE, "not a band context (ilf_set_original takes the whole picture)");
+  if (!ctx->slots[slot].uploaded) return fail(ctx, ILF_ERR_STATE, "slot %d: ilf_set_original_band before the slot's upload", slot);
+  return set_original_rows(ctx, slot, y, sy, cb, scb, cr, scr, ctu_avail, ctx->g.out_row0 - ctx->g.row0, ctx->g.out_rows);
+}
+
+// CTUs whose statistics records a slot produces: the picture's, or a band's own (num_ctu_rows x ctus_w).
+static int own_ctus(const ilf_ctx* ctx) { return ctx->is_band ? ctx->band.num_ctu_rows * ctx->g.ctus_w : ctx->num_ctus; }
+
+// A band slot is measured only against an original of its own rows given since its upload (ilf_set_original_band).
+static bool band_org_missing(const ilf_ctx* ctx, const Slot& s) { return ctx->is_band && !s.org_since_upload; }
+
 int ilf_sao_stats(ilf_ctx* ctx, int first_slot, int num_slots) {
   if (!ctx) return ILF_ERR_ARG;
   if (first_slot < 0 || num_slots < 1 || first_slot + num_slots > (int)ctx->slots.size()) return fail(ctx, ILF_ERR_ARG, "slot range [%d,+%d) out of range", first_slot, num_slots);
@@ -1287,7 +1354,7 @@ int ilf_sao_stats(ilf_ctx* ctx, int first_slot, int num_slots) {
   const Geom& g = ctx->g;
   for (int i = first_slot; i < first_slot + num_slots; i++) {
     Slot& s = ctx->slots[i];
-    if (!s.uploaded || !s.has_org) return fail(ctx, ILF_ERR_STATE, "slot %d: statistics need ilf_upload and ilf_set_original", i);
+    if (!s.uploaded || !s.has_org || band_org_missing(ctx, s)) return fail(ctx, ILF_ERR_STATE, "slot %d: statistics need ilf_upload and ilf_set_original", i);
     if (s.h2d_pending) { CU(ctx, cudaStreamWaitEvent(ctx->stream, s.ev_up, 0)); s.h2d_pending = false; }
     if (int rc = order_after_run(ctx, s, ctx->stream)) return rc;
   }
@@ -1299,8 +1366,8 @@ int ilf_sao_stats(ilf_ctx* ctx, int first_slot, int num_slots) {
       ctl.v[i] = (uint16_t)(s.result_buf[0] | (s.result_buf[1] << 2) | (s.result_buf[2] << 4));
       ctl.slot[i] = (uint8_t)i;
     }
-    // algorithmic bytes: the deblocked and the original picture are read once (2 B x 1.5 samples x 2 pictures per luma pixel)
-    if (int rc = timed_begin(ctx, ILF_KERNEL_SAO_STATS, 6.0 * g.width * g.height * cn)) return rc;
+    // algorithmic bytes: the deblocked and the original picture (own rows) are read once (2 B x 1.5 samples x 2 pictures per luma pixel)
+    if (int rc = timed_begin(ctx, ILF_KERNEL_SAO_STATS, 6.0 * g.width * g.out_rows * cn)) return rc;
     launch_sao_stats(g, ctx->slots_dev, c0, cn, ctl, ctx->stream);
     if (int rc = timed_end(ctx)) return rc;
     ctx->launches++;
@@ -1318,7 +1385,7 @@ int ilf_get_sao_stats(ilf_ctx* ctx, int slot, int64_t* out) {
   Slot& s = ctx->slots[slot];
   if (!s.stats) return fail(ctx, ILF_ERR_STATE, "slot %d: no statistics (ilf_set_original / ilf_sao_stats first)", slot);
   CU(ctx, cudaSetDevice(ctx->cfg.device));
-  CU(ctx, cudaMemcpyAsync(out, s.stats, (size_t)ctx->num_ctus * 3 * ILF_SAO_STATS_WORDS * sizeof(long long), cudaMemcpyDeviceToHost, ctx->stream));
+  CU(ctx, cudaMemcpyAsync(out, s.stats, (size_t)own_ctus(ctx) * 3 * ILF_SAO_STATS_WORDS * sizeof(long long), cudaMemcpyDeviceToHost, ctx->stream));
   CU(ctx, cudaStreamSynchronize(ctx->stream));
   return ILF_OK;
 }
@@ -1327,10 +1394,11 @@ int ilf_get_sao_stats(ilf_ctx* ctx, int slot, int64_t* out) {
 int ilf_alf_stats(ilf_ctx* ctx, int first_slot, int num_slots) {
   if (!ctx) return ILF_ERR_ARG;
   if (first_slot < 0 || num_slots < 1 || first_slot + num_slots > (int)ctx->slots.size()) return fail(ctx, ILF_ERR_ARG, "slot range [%d,+%d) out of range", first_slot, num_slots);
-  if (ctx->is_band) return fail(ctx, ILF_ERR_STATE, "not available on band contexts");
+  for (int i = first_slot; i < first_slot + num_slots; i++)
+    if (band_org_missing(ctx, ctx->slots[i])) return fail(ctx, ILF_ERR_STATE, "not available on band contexts");
   CU(ctx, cudaSetDevice(ctx->cfg.device));
   const Geom& g = ctx->g;
-  const size_t bytes = (size_t)ctx->num_ctus * ILF_ALF_STATS_WORDS * sizeof(long long);
+  const size_t bytes = (size_t)own_ctus(ctx) * ILF_ALF_STATS_WORDS * sizeof(long long);
   for (int i = first_slot; i < first_slot + num_slots; i++) {
     Slot& s = ctx->slots[i];
     if (!s.uploaded || !s.has_org) return fail(ctx, ILF_ERR_STATE, "slot %d: statistics need ilf_upload and ilf_set_original", i);
@@ -1351,8 +1419,8 @@ int ilf_alf_stats(ilf_ctx* ctx, int first_slot, int num_slots) {
       ctl.v[i] = (uint16_t)(s.result_buf[0] | (s.result_buf[1] << 2) | (s.result_buf[2] << 4));
       ctl.slot[i] = (uint8_t)i;
     }
-    // algorithmic bytes: the reconstructed and the original picture are read once (2 B x 1.5 samples x 2 pictures per luma pixel)
-    if (int rc = timed_begin(ctx, ILF_KERNEL_ALF_STATS, 6.0 * g.width * g.height * cn)) return rc;
+    // algorithmic bytes: the reconstructed and the original picture (own rows) are read once (2 B x 1.5 samples x 2 pictures per luma pixel)
+    if (int rc = timed_begin(ctx, ILF_KERNEL_ALF_STATS, 6.0 * g.width * g.out_rows * cn)) return rc;
     launch_alf_classify(g, ctx->slots_dev, c0, cn, ctl, ctx->stream);
     launch_alf_stats(g, ctx->slots_dev, c0, cn, ctl, ctx->stream);
     if (int rc = timed_end(ctx)) return rc;
@@ -1371,7 +1439,7 @@ int ilf_get_alf_stats(ilf_ctx* ctx, int slot, int64_t* out) {
   Slot& s = ctx->slots[slot];
   if (!s.alf_stats) return fail(ctx, ILF_ERR_STATE, "slot %d: no statistics (ilf_set_original / ilf_alf_stats first)", slot);
   CU(ctx, cudaSetDevice(ctx->cfg.device));
-  CU(ctx, cudaMemcpyAsync(out, s.alf_stats, (size_t)ctx->num_ctus * ILF_ALF_STATS_WORDS * sizeof(long long), cudaMemcpyDeviceToHost, ctx->stream));
+  CU(ctx, cudaMemcpyAsync(out, s.alf_stats, (size_t)own_ctus(ctx) * ILF_ALF_STATS_WORDS * sizeof(long long), cudaMemcpyDeviceToHost, ctx->stream));
   CU(ctx, cudaStreamSynchronize(ctx->stream));
   return ILF_OK;
 }
@@ -1385,7 +1453,8 @@ int ilf_deblock_search(ilf_ctx* ctx, int first_slot, int num_slots, const ilf_de
   if (!cands || !shift) return fail(ctx, ILF_ERR_ARG, "null pointer");
   if (num_cands < 1 || num_cands > ILF_DEBLOCK_SEARCH_MAX) return fail(ctx, ILF_ERR_ARG, "num_cands %d outside 1..%d", num_cands, ILF_DEBLOCK_SEARCH_MAX);
   if (shift[0] < 0 || shift[0] > 31 || shift[1] < 0 || shift[1] > 31) return fail(ctx, ILF_ERR_ARG, "shift (%d, %d) outside 0..31", shift[0], shift[1]);
-  if (ctx->is_band) return fail(ctx, ILF_ERR_STATE, "not available on band contexts");
+  for (int i = first_slot; i < first_slot + num_slots; i++)
+    if (band_org_missing(ctx, ctx->slots[i])) return fail(ctx, ILF_ERR_STATE, "not available on band contexts");
   for (int i = first_slot; i < first_slot + num_slots; i++) {
     const Slot& s = ctx->slots[i];
     if (!s.uploaded || !s.has_db || !s.org_since_upload)

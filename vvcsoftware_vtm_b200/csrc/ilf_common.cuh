@@ -165,6 +165,9 @@ void launch_sao(const Geom& g, const SlotDev* slots, int first_slot, int num_slo
 void launch_alf(const Geom& g, const SlotDev* slots, int first_slot, int num_slots, const BatchCtl& ctl, int planes /* bit 0 luma, bit 1 chroma */, cudaStream_t st);
 void launch_sao_stats(const Geom& g, const SlotDev* slots, int first_slot, int num_slots, const BatchCtl& ctl, cudaStream_t st);
 cudaError_t picture_hash(const Geom& g, const int16_t* const planes[3], uint32_t* scratch, cudaStream_t st, uint32_t out_crc[3], uint32_t out_sum[3]);
+// The same kernels over luma rows [first, first + n) of the held planes (chroma halved), y0 = their first picture row: the CRC register
+// contribution from a zero register and the checksum partial sum (ilf_picture_hash_band).  Synchronises `st`.
+cudaError_t hash_rows(const Geom& g, const int16_t* const planes[3], uint32_t* scratch, cudaStream_t st, int first, int n, int y0, uint32_t reg[3], uint32_t sum[3]);
 void launch_alf_stats(const Geom& g, const SlotDev* slots, int first_slot, int num_slots, const BatchCtl& ctl, cudaStream_t st);
 void launch_alf_classify(const Geom& g, const SlotDev* slots, int first_slot, int num_slots, const BatchCtl& ctl, cudaStream_t st);
 

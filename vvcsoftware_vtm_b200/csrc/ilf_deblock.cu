@@ -658,7 +658,8 @@ __global__ void __launch_bounds__(SEARCH_THREADS, SEARCH_MIN_CTAS) deblock_searc
   SearchWork* const work = reinterpret_cast<SearchWork*>(smem + STRIDE);
   SearchShared& sh = *reinterpret_cast<SearchShared*>(smem + STRIDE + 2 * sizeof(SearchWork));
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const int rows = g.rows, crow = g.rows >> 1, cw = g.width >> 1;
+  const int cw = g.width >> 1;
+  const int own0 = g.out_row0 - g.row0, own1 = own0 + g.out_rows;   // held rows whose samples count: all of a whole picture, a band's own
   const int ntx = (g.width + TW - 1) / TW, bands = (g.rows + 4 + TH - 1) / TH;
   const int per_pic = ntx * bands, total = per_pic * num_slots;
   const int K = cands.n;
@@ -723,7 +724,8 @@ __global__ void __launch_bounds__(SEARCH_THREADS, SEARCH_MIN_CTAS) deblock_searc
       __syncthreads();
     }
     const int y0 = ty * TH - 4, cy0 = ty * CTH - 2, x0 = tx * TW, cx0 = tx * CTW;
-    // this thread's horizontal-pass blocks of the original: the samples the deblocking kernel would store (y in [0, rows), x < width)
+    // this thread's horizontal-pass blocks of the original: the samples the deblocking kernel would store (x < width) in the rows
+    // the context owns (a band context deblocks its halo rows too, but they are another band's samples)
     const int u = tid & 31, h = (tid >> 5) & 3;
     const int pl = (tid >> 6) & 1, hc = (tid >> 5) & 1;
     unsigned rows_y = 0, rows_c = 0;
@@ -735,7 +737,7 @@ __global__ void __launch_bounds__(SEARCH_THREADS, SEARCH_MIN_CTAS) deblock_searc
 #pragma unroll
       for (int i = 0; i < 8; i++) {
         const int y = y0 + 8 * h + i;
-        const bool in = x < g.width && y >= 0 && y < rows;
+        const bool in = x < g.width && y >= own0 && y < own1;
         rows_y |= (in ? 1u : 0u) << i;
         org_y[i] = in ? ldg_u2(sd.org[0] + (size_t)y * g.pitch_y + x) : make_uint2(0, 0);
       }
@@ -743,7 +745,7 @@ __global__ void __launch_bounds__(SEARCH_THREADS, SEARCH_MIN_CTAS) deblock_searc
 #pragma unroll
       for (int i = 0; i < 8; i++) {
         const int y = cy0 + 8 * hc + i;
-        const bool in = xc < cw && y >= 0 && y < crow;
+        const bool in = xc < cw && y >= (own0 >> 1) && y < (own1 >> 1);
         rows_c |= (in ? 1u : 0u) << i;
         org_c[i] = in ? __ldg(reinterpret_cast<const uint32_t*>(sd.org[1 + pl] + (size_t)y * g.pitch_c + xc)) : 0u;
       }

@@ -11,6 +11,13 @@
 // A = M^(bits per row), and a tree over the rows (front-padded with empty rows to a power of two, level l combining with
 // A^(2^l)) gives R(picture) from a zero register.  The host finishes: the 0xffff start value and the 16 appended zero bits are
 // two more matrix products.  Checksum (compChecksum): a plain sum of masked bytes, reduced next to the CRC.
+//
+// The kernels hash a window of rows: the whole picture, or the own rows of a band context (the row origin of the window keeps the
+// checksum's row mask in picture coordinates).  Parts of consecutive rows combine on the host (ilf_hash_combine): a part of n rows
+// advances the register by A^n, so folding s = A^n s + R(part) over the parts in row order gives R(picture).
+#include <algorithm>
+#include <vector>
+
 #include "ilf_common.cuh"
 
 namespace ilf {
@@ -28,7 +35,8 @@ __device__ __forceinline__ uint32_t mat_apply(const uint16_t* col, uint32_t s) {
 
 struct HashArgs {
   const int16_t* plane[3];
-  int pitch[3], width[3], height[3], bd[3], padded[3];  // padded = rows rounded up to a power of two
+  int pitch[3], width[3], height[3], bd[3], padded[3];  // height = rows of the window; padded = rows rounded up to a power of two
+  int y0[3];                                             // picture row of the window's first row (checksum mask)
   uint32_t* rows;                                        // [3][16384] {crc | checksum hi?} -> two arrays
   uint32_t* sums;
   uint16_t pow[3][14][16];                               // per plane: columns of A^(2^l), A = one row's worth of register steps
@@ -45,7 +53,8 @@ __global__ void __launch_bounds__(32) hash_rows_kernel(HashArgs a) {
   const bool two = a.bd[p] > 8;
   const uint4* row = reinterpret_cast<const uint4*>(a.plane[p] + (size_t)r * a.pitch[p]);
   uint32_t s = 0, sum = 0;
-  const uint32_t my = (r & 0xff) ^ (r >> 8);
+  const int y = a.y0[p] + r;
+  const uint32_t my = (y & 0xff) ^ (y >> 8);
   auto sample = [&](uint32_t smp, int x) {
     const uint32_t mask = (my ^ (x & 0xff) ^ (x >> 8)) & 0xff;
     s = crc_byte(tab, s, smp & 0xff);
@@ -113,26 +122,27 @@ Mat mat_pow_bits(unsigned long long nbits) {  // M^nbits
 
 }  // namespace
 
-// planes[p]: device pointers of the picture's current planes.  out_crc / out_sum: the values compCRC / compChecksum put into the digest.
-cudaError_t picture_hash(const Geom& g, const int16_t* const planes[3], uint32_t* scratch /* 2 * 3 * 16384 + 8 words */, cudaStream_t st, uint32_t out_crc[3], uint32_t out_sum[3]) {
+// planes[p]: device pointers of the held planes.  reg / sum: R(rows) from a zero register and the checksum partial sum of luma rows
+// [first, first + n) of the held planes (chroma rows halved); y0 = picture row of `first`.
+cudaError_t hash_rows(const Geom& g, const int16_t* const planes[3], uint32_t* scratch /* 2 * 3 * 16384 + 8 words */, cudaStream_t st, int first, int n, int y0,
+                      uint32_t reg[3], uint32_t sum[3]) {
   static bool tab_set[64] = {};
   int dev = 0;
   cudaGetDevice(&dev);
   HashArgs a;
-  unsigned long long row_bits[3], total_bits[3];
   for (int p = 0; p < 3; p++) {
-    a.plane[p] = planes[p];
+    const int sh = p ? 1 : 0;
     a.pitch[p] = p ? g.pitch_c : g.pitch_y;
-    a.width[p] = p ? g.width / 2 : g.width;
-    a.height[p] = p ? g.height / 2 : g.height;
+    a.plane[p] = planes[p] + (size_t)(first >> sh) * a.pitch[p];
+    a.width[p] = g.width >> sh;
+    a.height[p] = n >> sh;
+    a.y0[p] = y0 >> sh;
     a.bd[p] = p ? g.bd_chroma : g.bd_luma;
-    int n = 1;
-    while (n < a.height[p]) n <<= 1;
-    a.padded[p] = n;
-    row_bits[p] = (unsigned long long)a.width[p] * (a.bd[p] > 8 ? 16 : 8);
-    total_bits[p] = row_bits[p] * a.height[p];
-    Mat m = mat_pow_bits(row_bits[p]);
-    for (int l = 0; l < 14; l++) { for (int i = 0; i < 16; i++) a.pow[p][l][i] = m.col[i]; m = mul(m, m); }
+    int m = 1;
+    while (m < a.height[p]) m <<= 1;
+    a.padded[p] = m;
+    Mat mp = mat_pow_bits((unsigned long long)a.width[p] * (a.bd[p] > 8 ? 16 : 8));
+    for (int l = 0; l < 14; l++) { for (int i = 0; i < 16; i++) a.pow[p][l][i] = mp.col[i]; mp = mul(mp, mp); }
   }
   a.rows = scratch;
   a.sums = scratch + 3 * 16384;
@@ -152,12 +162,63 @@ cudaError_t picture_hash(const Geom& g, const int16_t* const planes[3], uint32_t
   e = cudaStreamSynchronize(st);
   if (e != cudaSuccess) return e;
   for (int p = 0; p < 3; p++) {
-    // register after the whole picture from 0xffff, then the 16 appended zero bits
-    const uint16_t s = (uint16_t)(apply(mat_pow_bits(total_bits[p]), 0xffff) ^ (uint16_t)h[2 * p]);
-    out_crc[p] = apply(mat_pow_bits(16), s);
-    out_sum[p] = h[2 * p + 1];
+    reg[p] = h[2 * p];
+    sum[p] = h[2 * p + 1];
   }
   return cudaGetLastError();
 }
 
+// The register compCRC leaves after `bits` message bits from 0xffff whose contribution from a zero register is `reg`, followed by
+// the 16 appended zero bits.
+static uint32_t crc_finish(uint16_t reg, unsigned long long bits) {
+  const uint16_t s = (uint16_t)(apply(mat_pow_bits(bits), 0xffff) ^ reg);
+  return apply(mat_pow_bits(16), s);
+}
+
+cudaError_t picture_hash(const Geom& g, const int16_t* const planes[3], uint32_t* scratch, cudaStream_t st, uint32_t out_crc[3], uint32_t out_sum[3]) {
+  uint32_t reg[3];
+  cudaError_t e = hash_rows(g, planes, scratch, st, 0, g.height, 0, reg, out_sum);
+  if (e != cudaSuccess) return e;
+  for (int p = 0; p < 3; p++) {
+    const unsigned long long row_bits = (unsigned long long)(g.width >> (p ? 1 : 0)) * ((p ? g.bd_chroma : g.bd_luma) > 8 ? 16 : 8);
+    out_crc[p] = crc_finish((uint16_t)reg[p], row_bits * (unsigned long long)(g.height >> (p ? 1 : 0)));
+  }
+  return cudaSuccess;
+}
+
 }  // namespace ilf
+
+// Host only: parts may come from other processes, so everything is checked before it is used.
+extern "C" int ilf_hash_combine(const ilf_hash_part* parts, int num_parts, int kind, uint32_t out[3]) {
+  using namespace ilf;
+  if (!parts || !out || num_parts < 1 || (kind != ILF_HASH_CRC && kind != ILF_HASH_CHECKSUM)) return ILF_ERR_ARG;
+  const ilf_hash_part& p0 = parts[0];
+  if (p0.width <= 0 || p0.height <= 0 || ((p0.width | p0.height) & 1) || p0.bd_luma < 8 || p0.bd_luma > 12 || p0.bd_chroma < 8 || p0.bd_chroma > 12) return ILF_ERR_ARG;
+  std::vector<const ilf_hash_part*> order(num_parts);
+  for (int i = 0; i < num_parts; i++) {
+    const ilf_hash_part& q = parts[i];
+    if (q.width != p0.width || q.height != p0.height || q.bd_luma != p0.bd_luma || q.bd_chroma != p0.bd_chroma) return ILF_ERR_ARG;
+    if (q.first_row < 0 || q.num_rows < 1 || (long long)q.first_row + q.num_rows > p0.height) return ILF_ERR_ARG;
+    if ((q.first_row | q.num_rows) & 1) return ILF_ERR_ARG;   // even rows: chroma rows are exactly half
+    order[i] = &q;
+  }
+  std::sort(order.begin(), order.end(), [](const ilf_hash_part* a, const ilf_hash_part* b) { return a->first_row < b->first_row; });
+  long long next = 0;   // the parts tile [0, height): no gap, no overlap (each part lies inside the picture, so no overflow)
+  for (const ilf_hash_part* q : order) {
+    if (q->first_row != next) return ILF_ERR_ARG;
+    next += q->num_rows;
+  }
+  if (next != p0.height) return ILF_ERR_ARG;
+  for (int p = 0; p < 3; p++) {
+    const int sh = p ? 1 : 0;
+    const unsigned long long row_bits = (unsigned long long)(p0.width >> sh) * ((p ? p0.bd_chroma : p0.bd_luma) > 8 ? 16 : 8);
+    uint16_t s = 0;
+    uint32_t sum = 0;
+    for (const ilf_hash_part* q : order) {
+      s = (uint16_t)(apply(mat_pow_bits(row_bits * (unsigned long long)(q->num_rows >> sh)), s) ^ (uint16_t)q->crc[p]);
+      sum += q->sum[p];
+    }
+    out[p] = kind == ILF_HASH_CRC ? crc_finish(s, row_bits * (unsigned long long)(p0.height >> sh)) : sum;
+  }
+  return ILF_OK;
+}

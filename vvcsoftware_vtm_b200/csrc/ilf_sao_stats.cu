@@ -15,6 +15,8 @@
 // conflict-free.  At the end every warp reduces its words (REDUX), one shared-memory atomic per class and warp builds the
 // CTA totals, and the CTA writes the 5 x 64 int64 words of SAOStatData.
 // Bound: HBM reads of two pictures (6 B per luma pixel); the output is 7.7 KB per CTU.
+// A band context measures its own CTUs (record = blockIdx.x): decisions in picture coordinates, plane rows addressed from the first
+// held row.  Its rows reach one deblocked row beyond the own rows, inside the 16-row halo.
 #include "ilf_common.cuh"
 
 namespace ilf {
@@ -36,7 +38,7 @@ __global__ void __launch_bounds__(NT, 1024 / NT) sao_stats_kernel(Geom g, const 
   pdl_launch_dependents();
   const SlotDev& sd = slots[first_slot + bc.slot[blockIdx.z]];
   const unsigned ctl = bc.v[blockIdx.z];
-  const int comp = blockIdx.y, ctu = blockIdx.x, tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+  const int comp = blockIdx.y, ctu = blockIdx.x + (g.out_row0 >> g.ctu_log2) * g.ctus_w, tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const int cx = ctu % g.ctus_w, cy = ctu / g.ctus_w;
   const int sh = comp ? 1 : 0, csz = 1 << g.ctu_log2;
   const int lx0 = cx << g.ctu_log2, ly0 = cy << g.ctu_log2;
@@ -76,7 +78,8 @@ __global__ void __launch_bounds__(NT, 1024 / NT) sao_stats_kernel(Geom g, const 
     int* bo = acc + EO_WORDS + lane;    // + band * 32
     // 32-bit sample indices (a plane has < 2^31 samples)
     const int oL = gxl - gx, oR = gxr - gx;
-    int iu = max(y0 + ya - 1, 0) * pitch + gx, ic = (y0 + ya) * pitch + gx;
+    const int col = gx - (g.row0 >> sh) * pitch;   // sample index of picture row 0 in this column (held rows start at row0)
+    int iu = max(y0 + ya - 1, 0) * pitch + col, ic = (y0 + ya) * pitch + col;
     int ul = src[iu + oL], u = src[iu], ur = src[iu + oR];
     int l = src[ic + oL], c = src[ic], r = src[ic + oR];
     const int e0 = 2 * 32 * 4, e1 = e0 + 160 * 4, e2 = e0 + 320 * 4, e3 = e0 + 480 * 4;  // byte offsets of class 0 of every EO type
@@ -90,9 +93,9 @@ __global__ void __launch_bounds__(NT, 1024 / NT) sao_stats_kernel(Geom g, const 
 #pragma unroll
       for (int k = 0; k < G; k++) {
         const int gy = y0 + yg + k;
-        const int id = min(gy + 1, ph - 1) * pitch + gx;
+        const int id = min(gy + 1, ph - 1) * pitch + col;
         D[k][0] = src[id + oL]; D[k][1] = src[id]; D[k][2] = src[id + oR];
-        O[k] = org[min(gy, ph - 1) * pitch + gx];
+        O[k] = org[min(gy, ph - 1) * pitch + col];
       }
 #pragma unroll
       for (int k = 0; k < G; k++) {
@@ -141,7 +144,7 @@ __global__ void __launch_bounds__(NT, 1024 / NT) sao_stats_kernel(Geom g, const 
   }
   __syncthreads();
   // SAOStatData layout: [type][diff[32], count[32]] int64
-  long long* out = sd.stats + ((size_t)ctu * 3 + comp) * (5 * 64);
+  long long* out = sd.stats + ((size_t)blockIdx.x * 3 + comp) * (5 * 64);
   for (int i = tid; i < 5 * 64; i += NT) out[i] = (&tot[0][0])[i];
 }
 
@@ -150,7 +153,8 @@ __global__ void __launch_bounds__(NT, 1024 / NT) sao_stats_kernel(Geom g, const 
 void launch_sao_stats(const Geom& g, const SlotDev* slots, int first_slot, int num_slots, const BatchCtl& ctl, cudaStream_t st) {
   static bool attr_set[64] = {};
   once_per_device(attr_set, [&] { cudaFuncSetAttribute(sao_stats_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES); });
-  launch_pdl(sao_stats_kernel, dim3(g.ctus_w * g.ctus_h, 3, num_slots), dim3(NT), SMEM_BYTES, st, g, slots, first_slot, ctl);
+  const int ctu_rows = ((g.out_row0 + g.out_rows - 1) >> g.ctu_log2) - (g.out_row0 >> g.ctu_log2) + 1;   // own CTU rows
+  launch_pdl(sao_stats_kernel, dim3(g.ctus_w * ctu_rows, 3, num_slots), dim3(NT), SMEM_BYTES, st, g, slots, first_slot, ctl);
 }
 
 }  // namespace ilf

@@ -30,6 +30,12 @@ class IlfBand(C.Structure):
     _fields_ = [("first_ctu_row", C.c_int32), ("num_ctu_rows", C.c_int32)]
 
 
+class IlfHashPart(C.Structure):
+    """ilf_hash_part: a band's share of the decoded-picture hash (InLoopFilter.picture_hash_band, hash_combine)."""
+    _fields_ = [(n, C.c_int32) for n in ("width", "height", "bd_luma", "bd_chroma", "first_row", "num_rows")] + \
+               [("crc", C.c_uint32 * 3), ("sum", C.c_uint32 * 3)]
+
+
 def lib_path():
     return os.environ.get("ILF_B200_LIB") or os.path.join(_HERE, "libilf_b200.so")
 
@@ -94,6 +100,10 @@ def load_library():
     lib.ilf_get_deblock_search.argtypes = [vp, i, vp, i]
     lib.ilf_picture_hash.argtypes = [vp, i, i, C.POINTER(C.c_uint32 * 3)]
     lib.ilf_download_extended.argtypes = [vp, i, vp, pd, vp, pd, vp, pd, i]
+    lib.ilf_picture_hash_band.argtypes = [vp, i, C.POINTER(IlfHashPart)]
+    lib.ilf_hash_combine.argtypes = [C.POINTER(IlfHashPart), i, i, C.POINTER(C.c_uint32 * 3)]
+    lib.ilf_download_band_extended.argtypes = [vp, i, vp, pd, vp, pd, vp, pd, i]
+    lib.ilf_set_original_band.argtypes = [vp, i, vp, pd, vp, pd, vp, pd, vp]
     lib.ilf_launch_count.argtypes = [vp]
     lib.ilf_launch_count.restype = C.c_longlong
     lib.ilf_run_lanes.argtypes = [vp]
@@ -114,6 +124,26 @@ def _ptr(a):
 
 def _arr(a, dt):
     return None if a is None else np.ascontiguousarray(a, dtype=dt)
+
+
+def hash_combine(parts, kind="crc"):
+    """ilf_hash_combine: [Y, Cb, Cr] of the whole picture from the parts of all its bands (picture_hash_band), in any order.  A part
+    is the bytes picture_hash_band returned (or an IlfHashPart), so parts can come from other processes."""
+    kinds = {"crc": 1, "checksum": 2}
+    if kind not in kinds:
+        raise IlfError(f"unknown hash kind {kind!r}: 'crc' or 'checksum'")
+    lib = load_library()
+    arr = (IlfHashPart * max(1, len(parts)))()
+    for j, p in enumerate(parts):
+        b = bytes(p)
+        if len(b) != C.sizeof(IlfHashPart):
+            raise IlfError(f"a hash part is {C.sizeof(IlfHashPart)} bytes, got {len(b)}")
+        C.memmove(C.byref(arr, j * C.sizeof(IlfHashPart)), b, len(b))
+    out = (C.c_uint32 * 3)()
+    rc = lib.ilf_hash_combine(arr, len(parts), kinds[kind], C.byref(out))
+    if rc != 0:
+        raise IlfError(f"ilf_hash_combine failed ({rc}): the parts do not tile one picture")
+    return [int(v) for v in out]
 
 
 def pinned_planes(width, height):
@@ -152,6 +182,7 @@ class InLoopFilter:
         self.width, self.height = width, height
         ctu = 1 << ctu_log2
         self.ctus_w, self.ctus_h = (width + ctu - 1) // ctu, (height + ctu - 1) // ctu
+        self.own_ctus = self.ctus_w * ((self.own_row0 + self.own_rows + ctu - 1) // ctu - self.own_row0 // ctu)   # statistics records
 
     def close(self):
         if getattr(self, "_h", None) and self._h.value:
@@ -214,6 +245,37 @@ class InLoopFilter:
         self._ck(self._lib.ilf_download_band(self._h, slot, _ptr(y), y.shape[1], _ptr(cb), cb.shape[1], _ptr(cr), cr.shape[1]))
         return {"y": y, "cb": cb, "cr": cr}
 
+    def download_band_extended(self, slot, margin, out=None):
+        """The band's own rows, with Picture::extendPicBorder's margins, into full-picture planes of size (h + 2 m, w + 2 m),
+        m = margin (luma) or margin / 2: only the own rows, their left / right margins and, for the first / last band, the margin
+        rows above / below the picture are written.  `out`: such a dict to fill (every band into the same one), else new planes
+        filled with -1."""
+        if out is None:
+            out = {k: np.full(((self.height >> sh) + 2 * (margin >> sh), (self.width >> sh) + 2 * (margin >> sh)), -1, np.int16)
+                   for k, sh in (("y", 0), ("cb", 1), ("cr", 1))}
+        ptrs = []
+        for k, sh in (("y", 0), ("cb", 1), ("cr", 1)):
+            m, a = margin >> sh, out[k]
+            assert a.dtype == np.int16 and a.flags.c_contiguous and a.shape == ((self.height >> sh) + 2 * m, (self.width >> sh) + 2 * m)
+            ptrs += [C.c_void_p(a.ctypes.data + 2 * ((m + (self.own_row0 >> sh)) * a.shape[1] + m)), a.shape[1]]
+        self._ck(self._lib.ilf_download_band_extended(self._h, slot, *ptrs, margin))
+        return out
+
+    def picture_hash_band(self, slot=0):
+        """The band's part of the decoded-picture hash (CRC and checksum of its own rows) as bytes of an ilf_hash_part: picklable,
+        for hash_combine in whichever process gathers the bands."""
+        part = IlfHashPart()
+        self._ck(self._lib.ilf_picture_hash_band(self._h, slot, C.byref(part)))
+        return bytes(part)
+
+    def set_original_band(self, slot, y, cb, cr, ctu_avail):
+        """Source picture of the band's OWN rows (own_rows x width) and the ILF_AVAIL_* flags of every CTU of the picture."""
+        y, cb, cr = (_arr(a, np.int16) for a in (y, cb, cr))
+        assert y.shape == (self.own_rows, self.width) and cb.shape == cr.shape == (self.own_rows // 2, self.width // 2)
+        av = _arr(ctu_avail, np.uint8)
+        assert av.size == self.ctus_w * self.ctus_h
+        self._ck(self._lib.ilf_set_original_band(self._h, slot, _ptr(y), y.shape[1], _ptr(cb), cb.shape[1], _ptr(cr), cr.shape[1], _ptr(av)))
+
     def band_export(self, slot=0):
         """Opaque handle (bytes) of the slot's planes for the neighbouring band contexts, in this or another process."""
         buf = C.create_string_buffer(BAND_HANDLE_BYTES)
@@ -261,9 +323,11 @@ class InLoopFilter:
         self._ck(self._lib.ilf_alf(self._h, slot))
 
     def alf_classify(self, slot=0):
+        """classIdx | transposeIdx << 5 per 4x4 luma block of the rows the context produces (a band context: its own rows)."""
         out = np.empty((self.rows // 4, self.width // 4), np.uint8)
         self._ck(self._lib.ilf_alf_classify(self._h, slot, _ptr(out)))
-        return out
+        u0 = (self.own_row0 - self.row0) // 4
+        return out[u0:u0 + self.own_rows // 4].copy()
 
     # ---- encoder SAO statistics (EncSampleAdaptiveOffset::getStatistics) ---------------------------------
     def set_original(self, slot, y, cb, cr, ctu_avail):
@@ -276,10 +340,8 @@ class InLoopFilter:
         self._ck(self._lib.ilf_sao_stats(self._h, first_slot, num_slots))
 
     def get_sao_stats(self, slot=0):
-        """int64 [num_ctus, 3, 5, 64]: per CTU, component and SAO type diff[32] then count[32] (SAOStatData)."""
-        ctu = 1 << self.cfg.ctu_log2
-        n = ((self.width + ctu - 1) // ctu) * ((self.height + ctu - 1) // ctu)
-        out = np.empty((n, 3, 5, 64), np.int64)
+        """int64 [num_ctus, 3, 5, 64]: per CTU, component and SAO type diff[32] then count[32] (SAOStatData); a band context: its own CTUs."""
+        out = np.empty((self.own_ctus, 3, 5, 64), np.int64)
         self._ck(self._lib.ilf_get_sao_stats(self._h, slot, _ptr(out)))
         return out
 
@@ -300,9 +362,8 @@ class InLoopFilter:
         self._ck(self._lib.ilf_alf_stats(self._h, first_slot, num_slots))
 
     def get_alf_stats(self, slot=0):
-        ctu = 1 << self.cfg.ctu_log2
-        n = ((self.width + ctu - 1) // ctu) * ((self.height + ctu - 1) // ctu)
-        out = np.zeros((n, ALF_STATS_WORDS), np.int64)
+        """int64 [num_ctus, ALF_STATS_WORDS]; a band context: its own CTUs."""
+        out = np.zeros((self.own_ctus, ALF_STATS_WORDS), np.int64)
         self._ck(self._lib.ilf_get_alf_stats(self._h, slot, _ptr(out)))
         return out
 
