@@ -314,8 +314,8 @@ int ilf_download_extended(ilf_ctx* ctx, int slot, int16_t* y, ptrdiff_t stride_y
  * ------------------------------------------------------------------------------------------- */
 #define ILF_KERNEL_DEBLOCK 0
 #define ILF_KERNEL_SAO 1
-#define ILF_KERNEL_ALF_LUMA 2   /* the whole ALF stage: luma and chroma bands are CTAs of ONE launch (luma only when ILF_ALF_SPLIT=1) */
-#define ILF_KERNEL_ALF_CHROMA 3 /* the separate chroma launch of ILF_ALF_SPLIT=1 (measurement aid); otherwise unused */
+#define ILF_KERNEL_ALF_LUMA 2   /* the whole ALF stage: luma and chroma bands are CTAs of ONE launch */
+#define ILF_KERNEL_ALF_CHROMA 3 /* reserved: always zero */
 #define ILF_KERNEL_SAO_STATS 4  /* ilf_sao_stats */
 #define ILF_KERNEL_ALF_STATS 5  /* ilf_alf_stats: classification + the three statistics launches */
 #define ILF_NUM_KERNELS 6

@@ -97,14 +97,12 @@ def test_batched_slots(ilf_lib):
         assert 1 <= f.launch_count() <= 4    # planes whose stage is off in every picture of the batch are not launched
 
 
-@pytest.mark.parametrize("policy", [0, 1])
-def test_chain_dealt_to_lanes(policy, ilf_lib, monkeypatch):
+def test_chain_dealt_to_lanes(ilf_lib, monkeypatch):
     """A chain over a batch at or above the lane threshold is dealt to several compute streams (ilf_run, ILF_RUN_LANES): every
     slot still gets the reference result, also when the grouping changes between runs (a slot moves to another lane), when a
     single-stage run on the compute stream follows, and for the picture hash taken on the compute stream afterwards."""
     monkeypatch.setenv("ILF_RUN_LANES", "3")
     monkeypatch.setenv("ILF_RUN_LANE_MIN", "4")
-    monkeypatch.setenv("ILF_RUN_LANE_POLICY", str(policy))
     caps = [G.load_golden(p) for p in G.golden_files() if "ra_416x240" in p]
     n = 7
     with _ctx(ilf_lib, caps[0], num_slots=n) as f:

@@ -551,15 +551,13 @@ __device__ __forceinline__ void alf_chroma_cta(unsigned char* smem, const Geom& 
 
 // One launch for the whole ALF stage: grid rows [0, bands_y) are luma bands, [bands_y, bands_y + 2 bands_c) chroma bands.
 // The instruction-bound luma CTAs and the memory-bound chroma CTAs share the SMs instead of running back to back.
-// PLANES: 1 = luma only, 2 = chroma only (split launches, ILF_ALF_SPLIT=1), 3 = both.
-template <int PLANES>
 __global__ void __launch_bounds__(NT, L_CTAS) alf_kernel(Geom g, const SlotDev* __restrict__ slots, int first_slot, BatchCtl bc, int bands_y, int bands_c, int nseg_y, int nseg_c) {
   extern __shared__ __align__(128) unsigned char smem[];
   pdl_launch_dependents();
   const SlotDev& sd = slots[first_slot + bc.slot[blockIdx.z]];
   const unsigned ctl = bc.v[blockIdx.z];
-  if (PLANES == 1 || (PLANES == 3 && (int)blockIdx.y < bands_y)) alf_luma_cta<false>(smem, g, sd, ctl, nseg_y);
-  else alf_chroma_cta(smem, g, sd, ctl, (int)blockIdx.y - (PLANES == 3 ? bands_y : 0), bands_c, nseg_c);
+  if ((int)blockIdx.y < bands_y) alf_luma_cta<false>(smem, g, sd, ctl, nseg_y);
+  else alf_chroma_cta(smem, g, sd, ctl, (int)blockIdx.y - bands_y, bands_c, nseg_c);
 }
 __global__ void __launch_bounds__(NT, L_CTAS) alf_classify_kernel(Geom g, const SlotDev* __restrict__ slots, int first_slot, BatchCtl bc, int nseg) {
   extern __shared__ __align__(128) unsigned char smem[];
@@ -576,23 +574,17 @@ static int alf_nseg(int bands_total, int ntx, bool luma) {
   return nseg < 1 ? 1 : (nseg > ntx ? ntx : nseg);
 }
 
-// planes: bit 0 = luma, bit 1 = chroma (the slots' control words say which planes of which slot really run)
-void launch_alf(const Geom& g, const SlotDev* slots, int first_slot, int num_slots, const BatchCtl& ctl, int planes, cudaStream_t st) {
+// The slots' control words say which planes of which slot really run.
+void launch_alf(const Geom& g, const SlotDev* slots, int first_slot, int num_slots, const BatchCtl& ctl, cudaStream_t st) {
   static bool attr_set[64] = {};
   static const int pad = env_int("ILF_ALF_SMEM_PAD");
-  const int smem_l = L_SMEM_BYTES + pad, smem_c = C_SMEM_BYTES + pad, smem_lc = smem_l > smem_c ? smem_l : smem_c;
-  once_per_device(attr_set, [&] {
-    cudaFuncSetAttribute(alf_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_l);
-    cudaFuncSetAttribute(alf_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_c);
-    cudaFuncSetAttribute(alf_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_lc);
-  });
+  const int smem = (L_SMEM_BYTES > C_SMEM_BYTES ? L_SMEM_BYTES : C_SMEM_BYTES) + pad;
+  once_per_device(attr_set, [&] { cudaFuncSetAttribute(alf_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem); });
   const int bands_y = (g.rows + BR - 1) / BR, bands_c = (g.rows / 2 + BR - 1) / BR;
   const int nseg_y = alf_nseg(bands_y * num_slots, (g.width + TW - 1) / TW, true);
   const int nseg_c = alf_nseg(2 * bands_c * num_slots, (g.width / 2 + TW - 1) / TW, false);
-  if (planes == 1) launch_pdl(alf_kernel<1>, dim3(nseg_y, bands_y, num_slots), dim3(NT), smem_l, st, g, slots, first_slot, ctl, bands_y, bands_c, nseg_y, nseg_c);
-  else if (planes == 2) launch_pdl(alf_kernel<2>, dim3(nseg_c, 2 * bands_c, num_slots), dim3(NT), smem_c, st, g, slots, first_slot, ctl, bands_y, bands_c, nseg_y, nseg_c);
-  else launch_pdl(alf_kernel<3>, dim3(nseg_y > nseg_c ? nseg_y : nseg_c, bands_y + 2 * bands_c, num_slots), dim3(NT), smem_lc, st, g,
-                  slots, first_slot, ctl, bands_y, bands_c, nseg_y, nseg_c);
+  launch_pdl(alf_kernel, dim3(nseg_y > nseg_c ? nseg_y : nseg_c, bands_y + 2 * bands_c, num_slots), dim3(NT), smem, st, g, slots, first_slot, ctl, bands_y,
+             bands_c, nseg_y, nseg_c);
 }
 
 void launch_alf_classify(const Geom& g, const SlotDev* slots, int first_slot, int num_slots, const BatchCtl& ctl, cudaStream_t st) {

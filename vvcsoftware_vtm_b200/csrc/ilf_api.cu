@@ -116,17 +116,12 @@ struct Slot {
   bool alf_on[3] = {false, false, false};
   bool db_chroma = true;           // the chroma decisions' grid has an intra unit: deblocking may change the chroma planes
   bool alf_is7 = false;            // luma filter shape of the slot's ALF parameters
-  // Transfer pipeline: H2D copies run on the context's upload stream, kernels on the compute stream, D2H copies on the
-  // download stream; the three are ordered per slot with these events, so upload of picture n+1, filtering of picture n
-  // and download of picture n-1 overlap when the caller cycles through several slots.
-  cudaEvent_t ev_up = nullptr;     // all H2D copies of the slot (planes + side information) issued so far are done
-  cudaEvent_t ev_run = nullptr;    // all kernels issued so far on the slot are done (an event of the context's run ring, shared by the slots of a run)
-  cudaStream_t run_stream = nullptr;  // stream ev_run was recorded on: the compute stream or one of its lanes (nullptr: no kernel yet)
-  cudaEvent_t ev_down = nullptr;   // the last D2H copy of the slot is done
-  cudaEvent_t ev_side[3] = {nullptr, nullptr, nullptr};  // the pinned side-information region of stage k is free again
+  // ordering of the slot's copies and kernels (see "Per-slot ordering" above join())
+  cudaEvent_t ev_up = nullptr, ev_run = nullptr, ev_down = nullptr;
+  cudaStream_t run_stream = nullptr;
+  cudaEvent_t ev_side[3] = {nullptr, nullptr, nullptr};
   size_t side_off[4] = {0, 0, 0, 0};                       // regions of pinned_side per stage
-  bool h2d_pending = false;        // H2D work was issued since the last kernel launch on this slot
-  bool d2h_pending = false;        // a D2H copy was issued since the last kernel launch on this slot
+  bool h2d_pending = false, d2h_pending = false;
   // band mode: planes of the neighbouring bands' matching slot (above, below)
   struct Neighbour { const int16_t* planes = nullptr; void* ipc_base = nullptr; int device = -1, row0 = 0, rows = 0, pitch_y = 0, pitch_c = 0; size_t plane_y = 0, plane_c = 0; } nb[2];
 };
@@ -147,7 +142,6 @@ struct ilf_ctx {
   cudaStream_t lane[MAX_LANES] = {};
   int num_lanes = 1;
   int lane_min_slots = 8;          // batches smaller than this run on the compute stream alone
-  int lane_policy = 1;             // how ilf_run deals slots to lanes (see there)
   std::vector<Slot> slots;
   SlotDev* slots_dev = nullptr;
   size_t plane_y = 0, plane_c = 0, buf_elems = 0;  // elements per plane / per 3-plane buffer
@@ -158,8 +152,7 @@ struct ilf_ctx {
   struct TimedLaunch { int kernel; cudaEvent_t a, b; };
   std::vector<TimedLaunch> timed;
   std::vector<cudaEvent_t> free_events;
-  // one event per ilf_run (and lane) marks the end of its kernels for every slot of the run; a ring PER STREAM (0: the compute
-  // stream, 1 + i: lane i) is enough because waiting on an event that was re-recorded on the same stream only waits longer
+  // run events (fence()): a ring per stream, 0: the compute stream, 1 + i: lane i
   static constexpr int RUN_RING = 64;
   cudaEvent_t run_ring[1 + MAX_LANES][RUN_RING] = {};
   unsigned run_pos[1 + MAX_LANES] = {};
@@ -199,6 +192,108 @@ int check_slot(ilf_ctx* ctx, int slot) {
   return ILF_OK;
 }
 
+int check_range(ilf_ctx* ctx, int first, int n) {
+  if (!ctx) return ILF_ERR_ARG;
+  if (first < 0 || n < 1 || first + n > (int)ctx->slots.size()) return fail(ctx, ILF_ERR_ARG, "slot range [%d,+%d) out of range", first, n);
+  return ILF_OK;
+}
+
+// Per-slot ordering.  H2D copies run on the upload stream, kernels on the compute stream or one of its lanes, D2H copies on the
+// download stream, so the upload of picture n+1, the filtering of picture n and the download of picture n-1 overlap when the caller
+// cycles through several slots.  These events of the slot order the three:
+//   ev_up        every H2D copy issued so far for the slot (planes, side information, original, descriptor, halo rows) is done;
+//                h2d_pending: such a copy was issued since a compute stream last waited for ev_up.
+//   ev_side[k]   the pinned staging region of side-information stage k is free again (the host waits for it before refilling).
+//   ev_run       every kernel issued so far on the slot is done: an event of the context's run ring, shared by the slots of one
+//                run, recorded on run_stream (the compute stream or a lane; nullptr: no kernel yet).  Copies that overwrite what a
+//                kernel reads (uploads, side information, originals, halo rows) and downloads wait for it.
+//   ev_down      the last D2H copy of the slot is done (uploads wait for it); d2h_pending: a download was issued since ilf_run last
+//                waited for ev_down.
+// A batched entry point validates every slot before it issues anything, then joins each slot to the stream it launches on,
+// launches, and fences.
+
+// Orders `st` after the slot's pending upload and, when its last kernels ran on another stream, after them.  Clearing h2d_pending
+// is safe because every later kernel of the slot is then ordered after the upload: on `st` by stream order, on another stream
+// through the run event that fence() records on `st` after the launches.  The hash and the ALF classification record no run event;
+// they synchronise `st` before they return, so the upload is complete.  overwrites_buffers (ilf_run only): the launches write work
+// buffers that a download may still read.
+int join(ilf_ctx* ctx, Slot& s, cudaStream_t st, bool overwrites_buffers) {
+  if (s.h2d_pending) { CU(ctx, cudaStreamWaitEvent(st, s.ev_up, 0)); s.h2d_pending = false; }
+  if (overwrites_buffers && s.d2h_pending) { CU(ctx, cudaStreamWaitEvent(st, s.ev_down, 0)); s.d2h_pending = false; }
+  if (s.run_stream && s.run_stream != st) CU(ctx, cudaStreamWaitEvent(st, s.ev_run, 0));
+  return ILF_OK;
+}
+
+// One event of ring `ring` recorded on `st` becomes ev_run of the slots [first, first + n) (of those with lane_of[i - first] == lane,
+// when lane_of is given).  A ring per stream is enough: waiting on an event that was re-recorded on the same stream only waits longer.
+int fence(ilf_ctx* ctx, int first, int n, cudaStream_t st, int ring, const uint8_t* lane_of = nullptr, int lane = 0) {
+  cudaEvent_t done = ctx->next_run_event(ring);
+  CU(ctx, cudaEventRecord(done, st));
+  for (int i = 0; i < n; i++)
+    if (!lane_of || lane_of[i] == lane) { ctx->slots[first + i].ev_run = done; ctx->slots[first + i].run_stream = st; }
+  return ILF_OK;
+}
+
+// Control word of a slot's current picture: plane p from buffer result_buf[p] (BatchCtl).
+unsigned buf_word(const Slot& s) { return s.result_buf[0] | s.result_buf[1] << 2 | s.result_buf[2] << 4; }
+
+// Compact launch list of the chunk of slots [c0, c0 + cn): grid layer m works on slot c0 + ctl.slot[m] under control word ctl.v[m].
+// word(i) gives the control word of slot c0 + i, or < 0 to leave it out; mv_mode >= 0 keeps the slots of that motion-vector
+// representation only (none / int16 / int32 are different deblocking kernels).
+template <typename Word>
+int compact(const ilf_ctx* ctx, int c0, int cn, int mv_mode, BatchCtl& ctl, Word word) {
+  int m = 0;
+  for (int i = 0; i < cn; i++) {
+    const int v = word(i);
+    if (v < 0 || (mv_mode >= 0 && ctx->slots[c0 + i].mv_mode != mv_mode)) continue;
+    ctl.v[m] = (uint16_t)v;
+    ctl.slot[m++] = (uint8_t)i;
+  }
+  return m;
+}
+
+int timed_collect(ilf_ctx* ctx) {
+  if (ctx->timed.empty()) return ILF_OK;
+  CU(ctx, cudaStreamSynchronize(ctx->stream));
+  for (auto& t : ctx->timed) {
+    float ms = 0;
+    CU(ctx, cudaEventElapsedTime(&ms, t.a, t.b));
+    ctx->kernel_ms[t.kernel] += ms;
+    ctx->kernel_launches[t.kernel]++;
+    ctx->free_events.push_back(t.a);
+    ctx->free_events.push_back(t.b);
+  }
+  ctx->timed.clear();
+  return ILF_OK;
+}
+
+// Opens the event pair around a launch while timing is on (ilf_set_timing / ilf_kernel_times); at most 4096 pairs stay pending.
+int timed_begin(ilf_ctx* ctx, int kernel, double algo_bytes) {
+  if (ctx->timed.size() >= 4096) if (int rc = timed_collect(ctx)) return rc;
+  ctx->kernel_bytes[kernel] += algo_bytes;
+  cudaEvent_t ev[2];
+  for (int i = 0; i < 2; i++) {
+    if (!ctx->free_events.empty()) { ev[i] = ctx->free_events.back(); ctx->free_events.pop_back(); }
+    else CU(ctx, cudaEventCreate(&ev[i]));
+  }
+  ctx->timed.push_back({kernel, ev[0], ev[1]});
+  CU(ctx, cudaEventRecord(ev[0], ctx->stream));
+  return ILF_OK;
+}
+
+// Issues `count` kernels through enqueue() and counts them.  kernel >= 0: while timing is on, an event pair on the compute stream
+// brackets them and `bytes` are accounted to that kernel.
+template <typename Enqueue>
+int launch(ilf_ctx* ctx, int kernel, double bytes, int count, Enqueue enqueue) {
+  const bool timed = ctx->timing && kernel >= 0;
+  if (timed) if (int rc = timed_begin(ctx, kernel, bytes)) return rc;
+  enqueue();
+  if (timed) CU(ctx, cudaEventRecord(ctx->timed.back().b, ctx->stream));
+  ctx->launches += count;
+  CU(ctx, cudaGetLastError());
+  return ILF_OK;
+}
+
 // cuTensorMapEncodeTiled through the runtime's driver entry point lookup: the library does not link libcuda, so it still
 // loads (and exports its symbols) on a machine without a driver.
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*, const cuuint32_t*,
@@ -225,6 +320,13 @@ int16_t* plane_ptr(const ilf_ctx* ctx, const Slot& s, int buf, int plane) {
   if (plane >= 1) p += ctx->plane_y;
   if (plane == 2) p += ctx->plane_c;
   return p;
+}
+
+// Plane p's part of LOCAL luma rows [first, first + n): width, rows and first row in the plane's samples (chroma halved), pitch.
+struct PlaneRows { int w, h, r0, pitch; };
+PlaneRows plane_rows(const Geom& g, int p, int first, int n) {
+  const int sh = p ? 1 : 0;
+  return {g.width >> sh, n >> sh, first >> sh, p ? g.pitch_c : g.pitch_y};
 }
 
 int make_map3(ilf_ctx* ctx, CUtensorMap* out, CUtensorMapDataType dt, void* base, int w, int h, int nz, size_t pitch_bytes, size_t layer_bytes, int bw, int bh) {
@@ -261,16 +363,33 @@ bool is_pinned(const void* p) {
   return at.type == cudaMemoryTypeHost;
 }
 
-// Side information goes host -> pinned staging region of its stage -> device, asynchronously on the upload stream.
-int stage_side(ilf_ctx* ctx, Slot& s, void* dst, const void* src, size_t bytes, size_t& cursor, size_t limit) {
-  if (bytes >= 4096 && is_pinned(src)) {  // page-locked source: copy straight from the caller's array
-    CU(ctx, cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, ctx->s_up));
-    return ILF_OK;
+// A side-information setter stages its arrays between side_begin and side_end: host -> pinned staging region k of the slot ->
+// device, asynchronously on the upload stream.
+int side_begin(ilf_ctx* ctx, Slot& s, int k, size_t& cursor) {
+  CU(ctx, cudaSetDevice(ctx->cfg.device));
+  CU(ctx, cudaEventSynchronize(s.ev_side[k]));  // the previous copy out of this staging region is done
+  CU(ctx, cudaStreamWaitEvent(ctx->s_up, s.ev_run, 0));  // kernels of the slot's previous picture may still read the device arrays
+  cursor = s.side_off[k];
+  return ILF_OK;
+}
+
+int side_end(ilf_ctx* ctx, int slot, int k) {
+  CU(ctx, cudaEventRecord(ctx->slots[slot].ev_side[k], ctx->s_up));
+  return push_desc(ctx, slot);
+}
+
+// `rows` rows of `row` bytes, dense in the caller's array, `dpitch` bytes apart on the device (0: dense there too).
+int stage_side(ilf_ctx* ctx, Slot& s, int k, void* dst, const void* src, size_t row, size_t& cursor, size_t rows = 1, size_t dpitch = 0) {
+  const size_t bytes = row * rows;
+  const void* from = src;
+  if (!(bytes >= 4096 && is_pinned(src))) {  // a page-locked source is copied straight from the caller's array
+    if (cursor + bytes > s.side_off[k + 1]) return fail(ctx, ILF_ERR_STATE, "side-information staging overflow");
+    memcpy(s.pinned_side + cursor, src, bytes);
+    from = s.pinned_side + cursor;
+    cursor += (bytes + 255) & ~size_t(255);
   }
-  if (cursor + bytes > limit) return fail(ctx, ILF_ERR_STATE, "side-information staging overflow");
-  memcpy(s.pinned_side + cursor, src, bytes);
-  CU(ctx, cudaMemcpyAsync(dst, s.pinned_side + cursor, bytes, cudaMemcpyHostToDevice, ctx->s_up));
-  cursor += (bytes + 255) & ~size_t(255);
+  if (!dpitch || dpitch == row) CU(ctx, cudaMemcpyAsync(dst, from, bytes, cudaMemcpyHostToDevice, ctx->s_up));
+  else CU(ctx, cudaMemcpy2DAsync(dst, dpitch, from, row, row, rows, cudaMemcpyHostToDevice, ctx->s_up));
   return ILF_OK;
 }
 
@@ -283,20 +402,11 @@ struct BandHandle {  // what ilf_band_export writes into ilf_band_handle::opaque
 static_assert(sizeof(BandHandle) <= sizeof(ilf_band_handle), "ilf_band_handle too small");
 constexpr uint32_t BAND_MAGIC = 0x424C4649u;
 
-// Unit grids live on the device with a row pitch of units_pitch elements (multiple of 4); the caller's arrays are dense.
-int stage_grid(ilf_ctx* ctx, Slot& s, void* dst, const void* src, size_t elem_bytes, size_t& cursor, size_t limit) {
+// Unit grids (deblocking side information, region 0) live on the device with a row pitch of units_pitch elements (multiple of 4);
+// the caller's arrays are dense.
+int stage_grid(ilf_ctx* ctx, Slot& s, void* dst, const void* src, size_t elem_bytes, size_t& cursor) {
   const Geom& g = ctx->g;
-  const size_t row = (size_t)g.units_w * elem_bytes, bytes = row * g.units_h;
-  if (g.units_pitch == g.units_w) return stage_side(ctx, s, dst, src, bytes, cursor, limit);
-  const void* from = src;
-  if (!(bytes >= 4096 && is_pinned(src))) {
-    if (cursor + bytes > limit) return fail(ctx, ILF_ERR_STATE, "side-information staging overflow");
-    memcpy(s.pinned_side + cursor, src, bytes);
-    from = s.pinned_side + cursor;
-    cursor += (bytes + 255) & ~size_t(255);
-  }
-  CU(ctx, cudaMemcpy2DAsync(dst, (size_t)g.units_pitch * elem_bytes, from, row, row, g.units_h, cudaMemcpyHostToDevice, ctx->s_up));
-  return ILF_OK;
+  return stage_side(ctx, s, 0, dst, src, g.units_w * elem_bytes, cursor, g.units_h, g.units_pitch * elem_bytes);
 }
 
 int create_impl(ilf_ctx** out, const ilf_config* cfg, const ilf_band* band) {
@@ -361,7 +471,6 @@ int create_impl(ilf_ctx** out, const ilf_config* cfg, const ilf_band* band) {
   CU(ctx, cudaStreamCreateWithFlags(&ctx->s_down, cudaStreamNonBlocking));
   ctx->num_lanes = std::max(1, std::min((int)ilf_ctx::MAX_LANES, env_int("ILF_RUN_LANES", 2)));
   ctx->lane_min_slots = std::max(2, env_int("ILF_RUN_LANE_MIN", 8));
-  ctx->lane_policy = env_int("ILF_RUN_LANE_POLICY", 1);
   if (ctx->num_lanes > 1)
     for (int i = 0; i < ctx->num_lanes; i++) CU(ctx, cudaStreamCreateWithFlags(&ctx->lane[i], cudaStreamNonBlocking));
   for (auto& ring : ctx->run_ring)
@@ -412,14 +521,14 @@ int create_impl(ilf_ctx** out, const ilf_config* cfg, const ilf_band* band) {
       if (int rc = make_map3(ctx, &s.dev.tm_mv32, CU_TENSOR_MAP_DATA_TYPE_UINT32, s.mv, g.units_w * 4, g.units_h, 1, (size_t)g.units_pitch * 16, units * 16, DB_BOX_MV32_WORDS, 8)) return rc;
     }
     for (int p = 0; p < 3; p++) {
-      const int pw = p ? cfg->width / 2 : cfg->width, ph = p ? g.rows / 2 : g.rows, pitch = p ? g.pitch_c : g.pitch_y;
-      if (int rc = make_map3(ctx, &s.dev.tm_db[p], CU_TENSOR_MAP_DATA_TYPE_UINT16, plane_ptr(ctx, s, 0, p), pw, ph, 3, (size_t)pitch * 2, ctx->buf_elems * 2, p ? DB_BOX_CW : DB_BOX_W,
+      const PlaneRows pr = plane_rows(g, p, 0, g.rows);
+      if (int rc = make_map3(ctx, &s.dev.tm_db[p], CU_TENSOR_MAP_DATA_TYPE_UINT16, plane_ptr(ctx, s, 0, p), pr.w, pr.h, 3, (size_t)pr.pitch * 2, ctx->buf_elems * 2, p ? DB_BOX_CW : DB_BOX_W,
                              p ? DB_BAND_ROWS / 2 : DB_BAND_ROWS))
         return rc;
-      if (int rc = make_map3(ctx, &s.dev.tm_sao[p], CU_TENSOR_MAP_DATA_TYPE_UINT16, plane_ptr(ctx, s, 0, p), pw, ph, 3, (size_t)pitch * 2, ctx->buf_elems * 2, SAO_TILE,
+      if (int rc = make_map3(ctx, &s.dev.tm_sao[p], CU_TENSOR_MAP_DATA_TYPE_UINT16, plane_ptr(ctx, s, 0, p), pr.w, pr.h, 3, (size_t)pr.pitch * 2, ctx->buf_elems * 2, SAO_TILE,
                              SAO_BAND_ROWS + 2))
         return rc;
-      if (int rc = make_map3(ctx, &s.dev.tm_alf[p], CU_TENSOR_MAP_DATA_TYPE_UINT16, plane_ptr(ctx, s, 0, p), pw, ph, 3, (size_t)pitch * 2, ctx->buf_elems * 2, ALF_TILE + 16,
+      if (int rc = make_map3(ctx, &s.dev.tm_alf[p], CU_TENSOR_MAP_DATA_TYPE_UINT16, plane_ptr(ctx, s, 0, p), pr.w, pr.h, 3, (size_t)pr.pitch * 2, ctx->buf_elems * 2, ALF_TILE + 16,
                              ALF_BAND_ROWS + 2 * (p ? ALF_HALO_C : ALF_HALO_Y)))
         return rc;
     }
@@ -459,7 +568,8 @@ int ilf_create_band(ilf_ctx** out, const ilf_config* cfg, const ilf_band* band) 
 int ilf_destroy(ilf_ctx* ctx) {
   if (!ctx) return ILF_OK;
   cudaSetDevice(ctx->cfg.device);
-  for (cudaStream_t st : {ctx->s_up, ctx->stream, ctx->s_down, ctx->lane[0], ctx->lane[1], ctx->lane[2], ctx->lane[3]}) if (st) cudaStreamSynchronize(st);
+  const auto streams = {ctx->s_up, ctx->stream, ctx->s_down, ctx->lane[0], ctx->lane[1], ctx->lane[2], ctx->lane[3]};
+  for (cudaStream_t st : streams) if (st) cudaStreamSynchronize(st);
   for (Slot& s : ctx->slots) {
     for (auto& nb : s.nb) if (nb.ipc_base) cudaIpcCloseMemHandle(nb.ipc_base);
     cudaFree(s.planes); cudaFree(s.info); cudaFree(s.info_c); cudaFree(s.mv); cudaFree(s.ctu_slice); cudaFree(s.db_params);
@@ -479,7 +589,7 @@ int ilf_destroy(ilf_ctx* ctx) {
   cudaFree(ctx->search_out);
   for (auto& t : ctx->timed) { cudaEventDestroy(t.a); cudaEventDestroy(t.b); }
   for (cudaEvent_t e : ctx->free_events) cudaEventDestroy(e);
-  for (cudaStream_t st : {ctx->s_up, ctx->stream, ctx->s_down, ctx->lane[0], ctx->lane[1], ctx->lane[2], ctx->lane[3]}) if (st) cudaStreamDestroy(st);
+  for (cudaStream_t st : streams) if (st) cudaStreamDestroy(st);
   delete ctx;
   return ILF_OK;
 }
@@ -506,13 +616,13 @@ static int make_chunks(const Geom& g, int first, int n, CopyChunk* out) {
   int k = 0;
   size_t off = 0;
   for (int p = 0; p < 3; p++) {
-    const int w = p ? g.width / 2 : g.width, h = p ? n / 2 : n, r0 = p ? first / 2 : first;
-    const int pieces = std::max(1, std::min(p ? 2 : 8, h / 64));
+    const PlaneRows pr = plane_rows(g, p, first, n);
+    const int pieces = std::max(1, std::min(p ? 2 : 8, pr.h / 64));
     for (int i = 0; i < pieces; i++) {
-      const int a = (int)((long long)h * i / pieces), b = (int)((long long)h * (i + 1) / pieces);
-      out[k++] = {p, r0 + a, b - a, off + (size_t)a * w};
+      const int a = (int)((long long)pr.h * i / pieces), b = (int)((long long)pr.h * (i + 1) / pieces);
+      out[k++] = {p, pr.r0 + a, b - a, off + (size_t)a * pr.w};
     }
-    off += (size_t)w * h;
+    off += (size_t)pr.w * pr.h;
   }
   return k;
 }
@@ -529,30 +639,26 @@ static int upload_rows(ilf_ctx* ctx, int slot, const int16_t* y, ptrdiff_t sy, c
   CU(ctx, cudaStreamWaitEvent(ctx->s_up, s.ev_down, 0));
   const int16_t* srcs[3] = {y, cb, cr};
   const ptrdiff_t strides[3] = {sy, scb, scr};
-  const bool direct = is_pinned(y) && is_pinned(cb) && is_pinned(cr);
-  if (!direct) {
-    if (!s.pinned) CU(ctx, cudaMallocHost(&s.pinned, ctx->buf_elems * sizeof(int16_t)));
-    CU(ctx, cudaEventSynchronize(s.ev_up));    // staging buffer: the previous staged upload has been consumed
-  }
-  if (direct) {
+  if (is_pinned(y) && is_pinned(cb) && is_pinned(cr)) {
     for (int p = 0; p < 3; p++) {
-      const int w = p ? g.width / 2 : g.width, h = p ? n / 2 : n, r0 = p ? first / 2 : first, pitch = p ? g.pitch_c : g.pitch_y;
-      CU(ctx, cudaMemcpy2DAsync(plane_ptr(ctx, s, 0, p) + (size_t)r0 * pitch, (size_t)pitch * 2, srcs[p], (size_t)strides[p] * 2, (size_t)w * 2, h, cudaMemcpyHostToDevice, ctx->s_up));
+      const PlaneRows pr = plane_rows(g, p, first, n);
+      CU(ctx, cudaMemcpy2DAsync(plane_ptr(ctx, s, 0, p) + (size_t)pr.r0 * pr.pitch, (size_t)pr.pitch * 2, srcs[p], (size_t)strides[p] * 2, (size_t)pr.w * 2, pr.h, cudaMemcpyHostToDevice, ctx->s_up));
     }
   } else {
+    if (!s.pinned) CU(ctx, cudaMallocHost(&s.pinned, ctx->buf_elems * sizeof(int16_t)));
+    CU(ctx, cudaEventSynchronize(s.ev_up));    // staging buffer: the previous staged upload has been consumed
     // helper threads fill the staging buffer chunk by chunk; this thread hands every finished chunk to the DMA engine, in order
     CopyChunk ch[COPY_CHUNKS_MAX];
     const int nch = make_chunks(g, first, n, ch);
-    const int first_l = first;
     std::atomic<int> ready[COPY_CHUNKS_MAX];
     for (int i = 0; i < nch; i++) ready[i].store(0, std::memory_order_relaxed);
     int16_t* stage = s.pinned;
     auto copy = [&, stage](int i) {
       const CopyChunk& c = ch[i];
-      const int w = c.plane ? g.width / 2 : g.width, base = c.plane ? first_l / 2 : first_l;
-      const int16_t* src = srcs[c.plane] + (ptrdiff_t)(c.row0 - base) * strides[c.plane];
+      const PlaneRows pr = plane_rows(g, c.plane, first, n);
+      const int16_t* src = srcs[c.plane] + (ptrdiff_t)(c.row0 - pr.r0) * strides[c.plane];
       int16_t* d = stage + c.stage_off;
-      for (int r = 0; r < c.rows; r++) memcpy(d + (size_t)r * w, src + (ptrdiff_t)r * strides[c.plane], (size_t)w * 2);
+      for (int r = 0; r < c.rows; r++) memcpy(d + (size_t)r * pr.w, src + (ptrdiff_t)r * strides[c.plane], (size_t)pr.w * 2);
       ready[i].store(1, std::memory_order_release);
     };
     const bool par = ctx->copy_pool.threads() > 1 && nch > 1;
@@ -562,9 +668,9 @@ static int upload_rows(ilf_ctx* ctx, int slot, const int16_t* y, ptrdiff_t sy, c
       if (par) while (!ready[i].load(std::memory_order_acquire)) std::this_thread::yield();
       else copy(i);
       const CopyChunk& c = ch[i];
-      const int w = c.plane ? g.width / 2 : g.width, pitch = c.plane ? g.pitch_c : g.pitch_y;
-      const cudaError_t e = cudaMemcpy2DAsync(plane_ptr(ctx, s, 0, c.plane) + (size_t)c.row0 * pitch, (size_t)pitch * 2, stage + c.stage_off, (size_t)w * 2, (size_t)w * 2, c.rows,
-                                              cudaMemcpyHostToDevice, ctx->s_up);
+      const PlaneRows pr = plane_rows(g, c.plane, first, n);
+      const cudaError_t e = cudaMemcpy2DAsync(plane_ptr(ctx, s, 0, c.plane) + (size_t)c.row0 * pr.pitch, (size_t)pr.pitch * 2, stage + c.stage_off, (size_t)pr.w * 2, (size_t)pr.w * 2,
+                                              c.rows, cudaMemcpyHostToDevice, ctx->s_up);
       if (e != cudaSuccess && err == cudaSuccess) err = e;
     }
     if (par) ctx->copy_pool.wait();
@@ -605,11 +711,10 @@ static int download_rows(ilf_ctx* ctx, int slot, int16_t* y, ptrdiff_t sy, int16
   CU(ctx, cudaStreamWaitEvent(ctx->s_down, s.ev_up, 0));  // a picture that no stage touched is read from the upload buffer
   int16_t* dsts[3] = {y, cb, cr};
   const ptrdiff_t strides[3] = {sy, scb, scr};
-  const bool direct = is_pinned(y) && is_pinned(cb) && is_pinned(cr);
-  if (direct) {
+  if (is_pinned(y) && is_pinned(cb) && is_pinned(cr)) {
     for (int p = 0; p < 3; p++) {
-      const int w = p ? g.width / 2 : g.width, h = p ? n / 2 : n, r0 = p ? first / 2 : first, pitch = p ? g.pitch_c : g.pitch_y;
-      CU(ctx, cudaMemcpy2DAsync(dsts[p], (size_t)strides[p] * 2, plane_ptr(ctx, s, s.result_buf[p], p) + (size_t)r0 * pitch, (size_t)pitch * 2, (size_t)w * 2, h, cudaMemcpyDeviceToHost, ctx->s_down));
+      const PlaneRows pr = plane_rows(g, p, first, n);
+      CU(ctx, cudaMemcpy2DAsync(dsts[p], (size_t)strides[p] * 2, plane_ptr(ctx, s, s.result_buf[p], p) + (size_t)pr.r0 * pr.pitch, (size_t)pr.pitch * 2, (size_t)pr.w * 2, pr.h, cudaMemcpyDeviceToHost, ctx->s_down));
     }
     CU(ctx, cudaEventRecord(s.ev_down, ctx->s_down));
     s.d2h_pending = true;
@@ -623,10 +728,10 @@ static int download_rows(ilf_ctx* ctx, int slot, int16_t* y, ptrdiff_t sy, int16
   int16_t* stage = s.pinned_down;
   for (int i = 0; i < nch; i++) {
     const CopyChunk& c = ch[i];
-    const int w = c.plane ? g.width / 2 : g.width, pitch = c.plane ? g.pitch_c : g.pitch_y;
+    const PlaneRows pr = plane_rows(g, c.plane, first, n);
     if (!ctx->chunk_ev[i]) CU(ctx, cudaEventCreateWithFlags(&ctx->chunk_ev[i], cudaEventDisableTiming));
-    CU(ctx, cudaMemcpy2DAsync(stage + c.stage_off, (size_t)w * 2, plane_ptr(ctx, s, s.result_buf[c.plane], c.plane) + (size_t)c.row0 * pitch, (size_t)pitch * 2, (size_t)w * 2, c.rows,
-                              cudaMemcpyDeviceToHost, ctx->s_down));
+    CU(ctx, cudaMemcpy2DAsync(stage + c.stage_off, (size_t)pr.w * 2, plane_ptr(ctx, s, s.result_buf[c.plane], c.plane) + (size_t)c.row0 * pr.pitch, (size_t)pr.pitch * 2,
+                              (size_t)pr.w * 2, c.rows, cudaMemcpyDeviceToHost, ctx->s_down));
     CU(ctx, cudaEventRecord(ctx->chunk_ev[i], ctx->s_down));
   }
   CU(ctx, cudaEventRecord(s.ev_down, ctx->s_down));
@@ -636,10 +741,10 @@ static int download_rows(ilf_ctx* ctx, int slot, int16_t* y, ptrdiff_t sy, int16
     const CopyChunk& c = ch[i];
     cudaSetDevice(device);
     if (cudaEventSynchronize(ctx->chunk_ev[i]) != cudaSuccess) { failed.store(1); return; }
-    const int w = c.plane ? g.width / 2 : g.width, base = c.plane ? first / 2 : first;
-    int16_t* d = dsts[c.plane] + (ptrdiff_t)(c.row0 - base) * strides[c.plane];
+    const PlaneRows pr = plane_rows(g, c.plane, first, n);
+    int16_t* d = dsts[c.plane] + (ptrdiff_t)(c.row0 - pr.r0) * strides[c.plane];
     const int16_t* src = stage + c.stage_off;
-    for (int r = 0; r < c.rows; r++) memcpy(d + (ptrdiff_t)r * strides[c.plane], src + (size_t)r * w, (size_t)w * 2);
+    for (int r = 0; r < c.rows; r++) memcpy(d + (ptrdiff_t)r * strides[c.plane], src + (size_t)r * pr.w, (size_t)pr.w * 2);
   };
   if (ctx->copy_pool.threads() > 1 && nch > 1) { ctx->copy_pool.start(nch, copy); ctx->copy_pool.wait(); }
   else for (int i = 0; i < nch; i++) copy(i);
@@ -734,41 +839,42 @@ __global__ void __launch_bounds__(256) band_halo_kernel(HaloBatch hb) {
 }  // namespace
 
 int ilf_band_exchange_batch(ilf_ctx* ctx, int first_slot, int num_slots) {
-  if (!ctx) return ILF_ERR_ARG;
-  if (first_slot < 0 || num_slots < 1 || first_slot + num_slots > (int)ctx->slots.size()) return fail(ctx, ILF_ERR_ARG, "slot range [%d,+%d) out of range", first_slot, num_slots);
+  if (int rc = check_range(ctx, first_slot, num_slots)) return rc;
   if (!ctx->is_band) return fail(ctx, ILF_ERR_STATE, "not a band context");
   const Geom& g = ctx->g;
+  // picture rows [h0, h1) of the halo above (side 0) and below (side 1); empty at a picture border
+  const int h0[2] = {g.row0, g.out_row0 + g.out_rows}, h1[2] = {g.out_row0, g.row0 + g.rows};
+  for (int slot = first_slot; slot < first_slot + num_slots; slot++)
+    for (int side = 0; side < 2; side++) {
+      const Slot::Neighbour& nb = ctx->slots[slot].nb[side];
+      if (h1[side] <= h0[side]) continue;
+      if (!nb.planes) return fail(ctx, ILF_ERR_STATE, "slot %d: no neighbour connected %s the band", slot, side == ILF_BAND_ABOVE ? "above" : "below");
+      if (h0[side] < nb.row0 || h1[side] > nb.row0 + nb.rows) return fail(ctx, ILF_ERR_ARG, "neighbour band does not hold picture rows [%d,%d)", h0[side], h1[side]);
+    }
   CU(ctx, cudaSetDevice(ctx->cfg.device));
   HaloBatch hb;
   int n = 0;
   auto flush = [&]() -> int {
-    if (!n) return ILF_OK;
-    band_halo_kernel<<<dim3(8, n), 256, 0, ctx->s_up>>>(hb);
-    CU(ctx, cudaGetLastError());
-    ctx->launches++;
+    const int rc = n ? launch(ctx, -1, 0, 1, [&] { band_halo_kernel<<<dim3(8, n), 256, 0, ctx->s_up>>>(hb); }) : ILF_OK;
     n = 0;
-    return ILF_OK;
+    return rc;
   };
   for (int slot = first_slot; slot < first_slot + num_slots; slot++) {
     Slot& s = ctx->slots[slot];
     CU(ctx, cudaStreamWaitEvent(ctx->s_up, s.ev_run, 0));  // kernels of the slot's previous run may still read the halo rows
     for (int side = 0; side < 2; side++) {
-      // picture rows of the halo on this side
-      const int h0 = side == ILF_BAND_ABOVE ? g.row0 : g.out_row0 + g.out_rows;
-      const int h1 = side == ILF_BAND_ABOVE ? g.out_row0 : g.row0 + g.rows;
-      if (h1 <= h0) continue;  // picture border
+      if (h1[side] <= h0[side]) continue;
       const Slot::Neighbour& nb = s.nb[side];
-      if (!nb.planes) return fail(ctx, ILF_ERR_STATE, "slot %d: no neighbour connected %s the band", slot, side == ILF_BAND_ABOVE ? "above" : "below");
-      if (h0 < nb.row0 || h1 > nb.row0 + nb.rows) return fail(ctx, ILF_ERR_ARG, "neighbour band does not hold picture rows [%d,%d)", h0, h1);
       for (int p = 0; p < 3; p++) {
-        const int sh = p ? 1 : 0, w = g.width >> sh, pitch = p ? g.pitch_c : g.pitch_y, npitch = p ? nb.pitch_c : nb.pitch_y;
+        const PlaneRows pr = plane_rows(g, p, h0[side] - g.row0, h1[side] - h0[side]);
+        const int npitch = p ? nb.pitch_c : nb.pitch_y;
         if (n == HALO_MAX) if (int rc = flush()) return rc;
         HaloCopy& c = hb.c[n++];
-        c.src = nb.planes + (p >= 1 ? nb.plane_y : 0) + (p == 2 ? nb.plane_c : 0) + (size_t)((h0 - nb.row0) >> sh) * npitch;  // neighbour's input buffer (buffer 0)
-        c.dst = plane_ptr(ctx, s, 0, p) + (size_t)((h0 - g.row0) >> sh) * pitch;
-        c.src_pitch = npitch; c.dst_pitch = pitch;
-        c.words = (w * 2) / 8;   // widths are multiples of 8 luma / 4 chroma samples
-        c.rows = (h1 - h0) >> sh;
+        c.src = nb.planes + (p >= 1 ? nb.plane_y : 0) + (p == 2 ? nb.plane_c : 0) + (size_t)((h0[side] - nb.row0) >> (p ? 1 : 0)) * npitch;  // neighbour's input buffer (buffer 0)
+        c.dst = plane_ptr(ctx, s, 0, p) + (size_t)pr.r0 * pr.pitch;
+        c.src_pitch = npitch; c.dst_pitch = pr.pitch;
+        c.words = (pr.w * 2) / 8;   // widths are multiples of 8 luma / 4 chroma samples
+        c.rows = pr.h;
       }
     }
   }
@@ -787,18 +893,11 @@ int ilf_band_exchange(ilf_ctx* ctx, int slot) {
 }
 
 // Decoded-picture hash of the slot's current picture, computed where the picture is (ilf_hash.cu).
-// Orders stream `st` after the kernels issued so far on the slot when they ran on another stream (a lane, or the compute stream).
-static int order_after_run(ilf_ctx* ctx, Slot& s, cudaStream_t st) {
-  if (s.run_stream && s.run_stream != st) CU(ctx, cudaStreamWaitEvent(st, s.ev_run, 0));
-  return ILF_OK;
-}
-
-// The slot's current planes for a hash, with the compute stream ordered after the slot's upload and last run.
+// The slot's current planes for a hash, with the compute stream joined to the slot.
 static int hash_planes(ilf_ctx* ctx, Slot& s, const int16_t* planes[3]) {
   CU(ctx, cudaSetDevice(ctx->cfg.device));
   if (!ctx->hash_scratch) CU(ctx, cudaMalloc(&ctx->hash_scratch, (6 * 16384 + 8) * sizeof(uint32_t)));
-  if (s.h2d_pending) CU(ctx, cudaStreamWaitEvent(ctx->stream, s.ev_up, 0));   // a picture no stage has touched yet
-  if (int rc = order_after_run(ctx, s, ctx->stream)) return rc;
+  if (int rc = join(ctx, s, ctx->stream, false)) return rc;
   for (int p = 0; p < 3; p++) planes[p] = plane_ptr(ctx, s, s.result_buf[p], p);
   return ILF_OK;
 }
@@ -812,8 +911,9 @@ int ilf_picture_hash(ilf_ctx* ctx, int slot, int kind, uint32_t out[3]) {
   const int16_t* planes[3];
   if (int rc = hash_planes(ctx, s, planes)) return rc;
   uint32_t crc[3], sum[3];
-  CU(ctx, picture_hash(ctx->g, planes, ctx->hash_scratch, ctx->stream, crc, sum));
-  ctx->launches += 2;
+  cudaError_t e = cudaSuccess;
+  if (int rc = launch(ctx, -1, 0, 2, [&] { e = picture_hash(ctx->g, planes, ctx->hash_scratch, ctx->stream, crc, sum); })) return rc;
+  CU(ctx, e);
   for (int p = 0; p < 3; p++) out[p] = kind == ILF_HASH_CRC ? crc[p] : sum[p];
   return ILF_OK;
 }
@@ -832,8 +932,9 @@ int ilf_picture_hash_band(ilf_ctx* ctx, int slot, ilf_hash_part* out) {
   memset(&part, 0, sizeof(part));
   part.width = g.width; part.height = g.height; part.bd_luma = g.bd_luma; part.bd_chroma = g.bd_chroma;
   part.first_row = g.out_row0; part.num_rows = g.out_rows;
-  CU(ctx, hash_rows(g, planes, ctx->hash_scratch, ctx->stream, g.out_row0 - g.row0, g.out_rows, g.out_row0, part.crc, part.sum));
-  ctx->launches += 2;
+  cudaError_t e = cudaSuccess;
+  if (int rc = launch(ctx, -1, 0, 2, [&] { e = hash_rows(g, planes, ctx->hash_scratch, ctx->stream, g.out_row0 - g.row0, g.out_rows, g.out_row0, part.crc, part.sum); })) return rc;
+  CU(ctx, e);
   *out = part;
   return ILF_OK;
 }
@@ -845,29 +946,26 @@ int ilf_picture_hash_band(ilf_ctx* ctx, int slot, ilf_hash_part* out) {
 // first row (with the corners) when `top`, those below the last row when `bottom`.
 static void extend_margins(ilf_ctx* ctx, int16_t* const planes[3], const ptrdiff_t strides[3], int margin, int n, bool top, bool bottom) {
   const Geom& g = ctx->g;
-  // left / right margins of every row, in row chunks on the copy threads; then the top / bottom rows (which include the corners)
-  struct Job { int plane, row0, rows; };
-  Job jobs[COPY_CHUNKS_MAX];
-  int nj = 0;
-  for (int p = 0; p < 3; p++) {
-    const int h = p ? n / 2 : n, pieces = std::max(1, std::min(p ? 2 : 8, h / 64));
-    for (int i = 0; i < pieces; i++) jobs[nj++] = {p, (int)((long long)h * i / pieces), (int)((long long)h * (i + 1) / pieces) - (int)((long long)h * i / pieces)};
-  }
+  // left / right margins of every row, in the row chunks of a staged transfer on the copy threads; then the top / bottom rows
+  // (which include the corners)
+  CopyChunk ch[COPY_CHUNKS_MAX];
+  const int nch = make_chunks(g, 0, n, ch);
   auto sides = [&](int i) {
-    const Job& j = jobs[i];
-    const int w = j.plane ? g.width / 2 : g.width, m = j.plane ? margin / 2 : margin;
-    for (int r = j.row0; r < j.row0 + j.rows; r++) {
-      int16_t* row = planes[j.plane] + (ptrdiff_t)r * strides[j.plane];
+    const CopyChunk& c = ch[i];
+    const int w = plane_rows(g, c.plane, 0, n).w, m = c.plane ? margin / 2 : margin;
+    for (int r = c.row0; r < c.row0 + c.rows; r++) {
+      int16_t* row = planes[c.plane] + (ptrdiff_t)r * strides[c.plane];
       const int16_t a = row[0], b = row[w - 1];
       for (int x = 0; x < m; x++) { row[-m + x] = a; row[w + x] = b; }
     }
   };
-  if (ctx->copy_pool.threads() > 1) { ctx->copy_pool.start(nj, sides); ctx->copy_pool.wait(); }
-  else for (int i = 0; i < nj; i++) sides(i);
+  if (ctx->copy_pool.threads() > 1) { ctx->copy_pool.start(nch, sides); ctx->copy_pool.wait(); }
+  else for (int i = 0; i < nch; i++) sides(i);
   for (int p = 0; p < 3; p++) {
-    const int w = p ? g.width / 2 : g.width, h = p ? n / 2 : n, m = p ? margin / 2 : margin;
+    const PlaneRows pr = plane_rows(g, p, 0, n);
+    const int w = pr.w, m = p ? margin / 2 : margin;
     int16_t* first = planes[p] - m;
-    int16_t* last = planes[p] + (ptrdiff_t)(h - 1) * strides[p] - m;
+    int16_t* last = planes[p] + (ptrdiff_t)(pr.h - 1) * strides[p] - m;
     for (int r = 1; r <= m; r++) {
       if (top) memcpy(first - (ptrdiff_t)r * strides[p], first, sizeof(int16_t) * (size_t)(w + 2 * m));
       if (bottom) memcpy(last + (ptrdiff_t)r * strides[p], last, sizeof(int16_t) * (size_t)(w + 2 * m));
@@ -945,19 +1043,16 @@ int ilf_set_deblock_info(ilf_ctx* ctx, int slot, const ilf_deblock_params* param
   if (mv16 && mv32) return fail(ctx, ILF_ERR_ARG, "give mv16 or mv32, not both");
   if (params->num_slices < 1 || params->num_slices > ILF_MAX_SLICES) return fail(ctx, ILF_ERR_ARG, "num_slices %d out of range", params->num_slices);
   Slot& s = ctx->slots[slot];
-  CU(ctx, cudaSetDevice(ctx->cfg.device));
-  CU(ctx, cudaEventSynchronize(s.ev_side[0]));  // the previous copy out of this staging region is done
-  CU(ctx, cudaStreamWaitEvent(ctx->s_up, s.ev_run, 0));  // kernels of the slot's previous picture may still read the device arrays
-  size_t cur = s.side_off[0];
-  const size_t lim = s.side_off[1];
-  if (int rc = stage_side(ctx, s, s.db_params, params, sizeof(*params), cur, lim)) return rc;
-  if (int rc = stage_grid(ctx, s, s.info, info, 4, cur, lim)) return rc;
+  size_t cur;
+  if (int rc = side_begin(ctx, s, 0, cur)) return rc;
+  if (int rc = stage_side(ctx, s, 0, s.db_params, params, sizeof(*params), cur)) return rc;
+  if (int rc = stage_grid(ctx, s, s.info, info, 4, cur)) return rc;
   s.has_ctree = info_chroma != nullptr;
-  if (info_chroma) if (int rc = stage_grid(ctx, s, s.info_c, info_chroma, 4, cur, lim)) return rc;
+  if (info_chroma) if (int rc = stage_grid(ctx, s, s.info_c, info_chroma, 4, cur)) return rc;
   s.mv_mode = mv16 ? 1 : (mv32 ? 2 : 0);
-  if (mv16) if (int rc = stage_grid(ctx, s, s.mv, mv16, 8, cur, lim)) return rc;
-  if (mv32) if (int rc = stage_grid(ctx, s, s.mv, mv32, 16, cur, lim)) return rc;
-  if (ctu_slice) if (int rc = stage_side(ctx, s, s.ctu_slice, ctu_slice, ctx->num_ctus, cur, lim)) return rc;
+  if (mv16) if (int rc = stage_grid(ctx, s, s.mv, mv16, 8, cur)) return rc;
+  if (mv32) if (int rc = stage_grid(ctx, s, s.mv, mv32, 16, cur)) return rc;
+  if (ctu_slice) if (int rc = stage_side(ctx, s, 0, s.ctu_slice, ctu_slice, ctx->num_ctus, cur)) return rc;
   s.dev.info = s.info;
   s.dev.info_c = info_chroma ? s.info_c : nullptr;
   s.dev.mv16 = mv16 ? (const int16_t*)s.mv : nullptr;
@@ -968,8 +1063,7 @@ int ilf_set_deblock_info(ilf_ctx* ctx, int slot, const ilf_deblock_params* param
   // chroma decisions read, deblocking leaves both chroma planes as uploaded, and run_stage skips them.
   s.db_chroma = any_intra(info_chroma ? info_chroma : info, (size_t)ctx->g.units_w * ctx->g.units_h);
   s.has_db = true;
-  CU(ctx, cudaEventRecord(s.ev_side[0], ctx->s_up));
-  return push_desc(ctx, slot);
+  return side_end(ctx, slot, 0);
 }
 
 int ilf_set_sao_params(ilf_ctx* ctx, int slot, const ilf_sao_ctu* ctus) {
@@ -989,15 +1083,12 @@ int ilf_set_sao_params(ilf_ctx* ctx, int slot, const ilf_sao_ctu* ctus) {
         if (ctus[i].offset[c][k] < -128 || ctus[i].offset[c][k] > 127)
           return fail(ctx, ILF_ERR_UNSUPPORTED, "CTU %d comp %d: SAO offset %d outside [-128,127]", i, c, ctus[i].offset[c][k]);
     }
-  CU(ctx, cudaSetDevice(ctx->cfg.device));
-  CU(ctx, cudaEventSynchronize(s.ev_side[1]));
-  CU(ctx, cudaStreamWaitEvent(ctx->s_up, s.ev_run, 0));
-  size_t cur = s.side_off[1];
-  if (int rc = stage_side(ctx, s, s.sao, ctus, sizeof(ilf_sao_ctu) * ctx->num_ctus, cur, s.side_off[2])) return rc;
+  size_t cur;
+  if (int rc = side_begin(ctx, s, 1, cur)) return rc;
+  if (int rc = stage_side(ctx, s, 1, s.sao, ctus, sizeof(ilf_sao_ctu) * ctx->num_ctus, cur)) return rc;
   s.dev.sao = s.sao;
   s.has_sao = true;
-  CU(ctx, cudaEventRecord(s.ev_side[1], ctx->s_up));
-  return push_desc(ctx, slot);
+  return side_end(ctx, slot, 1);
 }
 
 int ilf_set_alf_params(ilf_ctx* ctx, int slot, const ilf_alf_params* params, const uint8_t* ctu_enable) {
@@ -1008,13 +1099,10 @@ int ilf_set_alf_params(ilf_ctx* ctx, int slot, const ilf_alf_params* params, con
     s.alf_on[c] = false;
     for (int i = 0; i < ctx->num_ctus; i++) s.alf_on[c] |= ctu_enable[(size_t)c * ctx->num_ctus + i] != 0;
   }
-  CU(ctx, cudaSetDevice(ctx->cfg.device));
-  CU(ctx, cudaEventSynchronize(s.ev_side[2]));
-  CU(ctx, cudaStreamWaitEvent(ctx->s_up, s.ev_run, 0));
-  size_t cur = s.side_off[2];
-  const size_t lim = s.side_off[3];
-  if (int rc = stage_side(ctx, s, s.alf, params, sizeof(*params), cur, lim)) return rc;
-  if (int rc = stage_side(ctx, s, s.alf_ctu_enable, ctu_enable, 3 * (size_t)ctx->num_ctus, cur, lim)) return rc;
+  size_t cur;
+  if (int rc = side_begin(ctx, s, 2, cur)) return rc;
+  if (int rc = stage_side(ctx, s, 2, s.alf, params, sizeof(*params), cur)) return rc;
+  if (int rc = stage_side(ctx, s, 2, s.alf_ctu_enable, ctu_enable, 3 * (size_t)ctx->num_ctus, cur)) return rc;
   {
     // Coefficient order after transposition (filterBlk, AdaptiveLoopFilter.cpp:541-575), expanded once per picture so
     // that a 4x4 block fetches its 13 (7) coefficients with four 16-byte loads.
@@ -1027,173 +1115,85 @@ int ilf_set_alf_params(ilf_ctx* ctx, int slot, const ilf_alf_params* params, con
       for (int tr = 0; tr < 4; tr++)
         for (int k = 0; k < 16; k++)
           tab[cl][tr][k] = is7 ? (k < 13 ? params->luma_coeff[cl][perm7[tr][k]] : 0) : (k < 7 ? params->luma_coeff[cl][perm5[tr][k]] : 0);
-    if (int rc = stage_side(ctx, s, s.alf_coef, tab, sizeof(tab), cur, lim)) return rc;
+    if (int rc = stage_side(ctx, s, 2, s.alf_coef, tab, sizeof(tab), cur)) return rc;
     // The same filters in the dot-product layout (ilf_alf_tab.cuh); a picture whose outer coefficients do not fit int8 keeps
-    // the general path.  ILF_ALF_GENERAL=1 forces the general path (measurement / parity aid).
-    static const bool force_general = getenv("ILF_ALF_GENERAL") && atoi(getenv("ILF_ALF_GENERAL")) != 0;
+    // the general path.
     uint32_t dp[ALF_DP_WORDS];
-    bool luma_ok = !force_general, luma_nhi = false;
+    bool luma_ok = true, luma_nhi = false;
     for (int cl = 0; cl < 25 && luma_ok; cl++)
       for (int tr = 0; tr < 4; tr++) {
         uint32_t* e = dp + (cl * 4 + tr) * alftab::LUMA_WORDS;
         luma_ok &= is7 ? alftab::build_entry<3, 3>(tab[cl][tr], e, alftab::LUMA_WORDS, &luma_nhi) : alftab::build_entry<3, 2>(tab[cl][tr], e, alftab::LUMA_WORDS, &luma_nhi);
       }
     // the chroma filter (meaningful only when chroma ALF is on: a slice without it leaves the array unset)
-    static const bool chroma_general = getenv("ILF_ALF_CHROMA_GENERAL") && atoi(getenv("ILF_ALF_CHROMA_GENERAL")) != 0;
     bool chroma_nhi = false;
     int fc[7];
     for (int k = 0; k < 7; k++) fc[k] = params->chroma_coeff[k];
-    const bool chroma_ok = !force_general && !chroma_general && alftab::build_entry<2, 2>(fc, dp + 25 * 4 * alftab::LUMA_WORDS, alftab::CHROMA_WORDS, &chroma_nhi);
+    const bool chroma_ok = alftab::build_entry<2, 2>(fc, dp + 25 * 4 * alftab::LUMA_WORDS, alftab::CHROMA_WORDS, &chroma_nhi);
     s.dev.alf_mode = (luma_ok ? 1 : 0) | (chroma_ok ? 2 : 0) | (luma_ok && !luma_nhi ? 4 : 0) | (chroma_ok && !chroma_nhi ? 8 : 0);
     s.alf_is7 = is7;
-    if (int rc = stage_side(ctx, s, s.alf_coef_dp, dp, sizeof(dp), cur, lim)) return rc;
+    if (int rc = stage_side(ctx, s, 2, s.alf_coef_dp, dp, sizeof(dp), cur)) return rc;
   }
-  CU(ctx, cudaEventRecord(s.ev_side[2], ctx->s_up));
   s.dev.alf_coef = s.alf_coef;
   s.dev.alf_coef_dp = s.alf_coef_dp;
   s.dev.alf = s.alf;
   s.dev.alf_ctu_enable = s.alf_ctu_enable;
   s.has_alf = true;
-  return push_desc(ctx, slot);
+  return side_end(ctx, slot, 2);
 }
 
-// Event pair around one kernel launch while timing is on (ilf_set_timing / ilf_kernel_times).
-static int timed_begin(ilf_ctx* ctx, int kernel, double algo_bytes) {
-  if (!ctx->timing) return ILF_OK;
-  ctx->kernel_bytes[kernel] += algo_bytes;
-  cudaEvent_t ev[2];
-  for (int i = 0; i < 2; i++) {
-    if (!ctx->free_events.empty()) { ev[i] = ctx->free_events.back(); ctx->free_events.pop_back(); }
-    else CU(ctx, cudaEventCreate(&ev[i]));
-  }
-  ctx->timed.push_back({kernel, ev[0], ev[1]});
-  CU(ctx, cudaEventRecord(ev[0], ctx->stream));
-  return ILF_OK;
-}
-static int timed_end(ilf_ctx* ctx) {
-  if (!ctx->timing) return ILF_OK;
-  CU(ctx, cudaEventRecord(ctx->timed.back().b, ctx->stream));
-  return ILF_OK;
-}
-static int timed_collect(ilf_ctx* ctx) {
-  if (ctx->timed.empty()) return ILF_OK;
-  CU(ctx, cudaStreamSynchronize(ctx->stream));
-  for (auto& t : ctx->timed) {
-    float ms = 0;
-    CU(ctx, cudaEventElapsedTime(&ms, t.a, t.b));
-    ctx->kernel_ms[t.kernel] += ms;
-    ctx->kernel_launches[t.kernel]++;
-    ctx->free_events.push_back(t.a);
-    ctx->free_events.push_back(t.b);
-  }
-  ctx->timed.clear();
-  return ILF_OK;
-}
-
-// One stage over a batch of slots.  Buffer rotation per plane: the stage reads the plane's current buffer and writes
-// the other work buffer (1 or 2), never buffer 0, so the uploaded input survives and ilf_run can be repeated.  Planes
-// for which the stage is off in the whole picture are skipped and keep their buffer.
-// lane_of / lane: when given, only the slots i of [first, first + n) with lane_of[i - first] == lane take part.
-static int stream_index(const ilf_ctx* ctx, cudaStream_t st) {
-  for (int i = 0; i < ilf_ctx::MAX_LANES; i++) if (ctx->lane[i] && ctx->lane[i] == st) return 1 + i;
-  return 0;
-}
-
-static int run_stage(ilf_ctx* ctx, int first, int n, int stage, cudaStream_t stream, const uint8_t* lane_of = nullptr, int lane = 0) {
+// One stage over a batch of slots on stream `st` (ring: its run ring, which also picks its deblocking tile queue).  Buffer rotation
+// per plane: the stage reads the plane's current buffer and writes the other work buffer (1 or 2), never buffer 0, so the uploaded
+// input survives and ilf_run can be repeated.  Planes for which the stage is off in the whole picture are skipped and keep their
+// buffer.  Only the slots i of [first, first + n) with lane_of[i - first] == lane take part.
+static int run_stage(ilf_ctx* ctx, int first, int n, int stage, cudaStream_t st, int ring, const uint8_t* lane_of, int lane) {
   const Geom& g = ctx->g;
   const double plane_bytes[3] = {2.0 * g.width * g.rows * 2, 2.0 * (g.width / 2) * (g.rows / 2) * 2, 2.0 * (g.width / 2) * (g.rows / 2) * 2};  // read + write
   for (int c0 = first; c0 < first + n; c0 += MAX_BATCH) {
     const int cn = std::min(MAX_BATCH, first + n - c0);
-    // control words of the slots of this chunk, then one compact launch list per kernel (active slots only)
-    uint16_t word[MAX_BATCH];
-    bool on[MAX_BATCH][3];
+    // control words of the slots of this chunk (-1: nothing to do), then one compact launch list per kernel
+    int word[MAX_BATCH];
+    double bytes_of[MAX_BATCH];
     for (int i = 0; i < cn; i++) {
       Slot& s = ctx->slots[c0 + i];
-      unsigned v = 0;
-      const bool mine = !lane_of || lane_of[c0 + i - first] == lane;
+      unsigned v = buf_word(s);
+      bool any = false;
+      bytes_of[i] = 0;
       for (int p = 0; p < 3; p++) {
-        on[i][p] = mine && (stage == 0 ? (p == 0 || s.db_chroma) : (stage == 1 ? s.sao_on[p] : s.alf_on[p]));
-        v |= (unsigned)s.result_buf[p] << (2 * p);
-        if (!on[i][p]) { v |= 1u << (6 + p); continue; }   // (a slot of another lane is not launched at all: compact() below)
+        const bool on = lane_of[c0 + i - first] == lane && (stage == 0 ? (p == 0 || s.db_chroma) : (stage == 1 ? s.sao_on[p] : s.alf_on[p]));
+        if (!on) { v |= 1u << (6 + p); continue; }
+        any = true;
+        bytes_of[i] += plane_bytes[p];
         s.result_buf[p] = s.result_buf[p] == 1 ? 2 : 1;
       }
       if (stage == 2) v |= ((s.dev.alf_mode & 1) ? CTL_ALF_DOT_Y : 0) | (s.alf_is7 ? CTL_ALF_7X7 : 0) | ((s.dev.alf_mode & 4) ? CTL_ALF_HIC_Y : 0) |
                        ((s.dev.alf_mode & 2) ? CTL_ALF_DOT_C : 0) | ((s.dev.alf_mode & 8) ? CTL_ALF_HIC_C : 0);
-      word[i] = (uint16_t)v;
+      word[i] = any ? (int)v : -1;
     }
-    auto compact = [&](bool use_y, bool use_c, BatchCtl& ctl, double& bytes, int mv_mode = -1) {
-      int m = 0;
-      bytes = 0;
-      for (int i = 0; i < cn; i++) {
-        const bool y = use_y && on[i][0], c = use_c && (on[i][1] || on[i][2]);
-        if (!y && !c) continue;
-        if (mv_mode >= 0 && ctx->slots[c0 + i].mv_mode != mv_mode) continue;
-        ctl.v[m] = word[i];
-        ctl.slot[m] = (uint8_t)i;
-        m++;
-        if (y) bytes += plane_bytes[0];
-        if (use_c) bytes += (on[i][1] ? plane_bytes[1] : 0) + (on[i][2] ? plane_bytes[2] : 0);
-      }
-      return m;
+    // one launch of `kernel_launch` over the active slots (of motion-vector representation mv_mode when >= 0)
+    auto stage_launch = [&](int mv_mode, auto kernel_launch) -> int {
+      BatchCtl ctl;
+      const int m = compact(ctx, c0, cn, mv_mode, ctl, [&](int i) { return word[i]; });
+      if (!m) return ILF_OK;
+      double bytes = 0;
+      for (int j = 0; j < m; j++) bytes += bytes_of[ctl.slot[j]];
+      return launch(ctx, stage, bytes, 1, [&] { kernel_launch(ctl, m); });
     };
-    if (ctx->timed.size() >= 4096) if (int rc = timed_collect(ctx)) return rc;
-    BatchCtl ctl;
-    double bytes = 0;
     if (stage == 0) {
-      // one launch per motion-vector representation present in the batch (none / int16 / int32 are different kernels)
-      for (int mode = 0; mode < 3; mode++) {
-        const int m = compact(true, true, ctl, bytes, mode);
-        if (!m) continue;
-        if (int rc = timed_begin(ctx, stage, bytes)) return rc;
-        launch_deblock(g, ctx->slots_dev, c0, m, ctl, mode, ctx->db_work + 2 * stream_index(ctx, stream), stream);
-        if (int rc = timed_end(ctx)) return rc;
-        ctx->launches++;
-      }
+      for (int mode = 0; mode < 3; mode++)
+        if (int rc = stage_launch(mode, [&](const BatchCtl& ctl, int m) { launch_deblock(g, ctx->slots_dev, c0, m, ctl, mode, ctx->db_work + 2 * ring, st); })) return rc;
     } else if (stage == 1) {
-      const int m = compact(true, true, ctl, bytes);
-      if (m) {
-        if (int rc = timed_begin(ctx, stage, bytes)) return rc;
-        launch_sao(g, ctx->slots_dev, c0, m, ctl, stream);
-        if (int rc = timed_end(ctx)) return rc;
-        ctx->launches++;
-      }
+      if (int rc = stage_launch(-1, [&](const BatchCtl& ctl, int m) { launch_sao(g, ctx->slots_dev, c0, m, ctl, st); })) return rc;
     } else {
-      // One launch for luma and chroma (their CTAs share the SMs); ILF_ALF_SPLIT=1 launches them one after the other, which
-      // is how the per-plane durations of DESIGN.md were measured.  Merged, the whole stage is accounted under ALF_LUMA.
-      static const bool split = getenv("ILF_ALF_SPLIT") && atoi(getenv("ILF_ALF_SPLIT")) != 0;
-      if (!split) {
-        const int m = compact(true, true, ctl, bytes);
-        if (m) {
-          if (int rc = timed_begin(ctx, ILF_KERNEL_ALF_LUMA, bytes)) return rc;
-          launch_alf(g, ctx->slots_dev, c0, m, ctl, 3, stream);
-          if (int rc = timed_end(ctx)) return rc;
-          ctx->launches++;
-        }
-      } else {
-        int m = compact(true, false, ctl, bytes);
-        if (m) {
-          if (int rc = timed_begin(ctx, ILF_KERNEL_ALF_LUMA, bytes)) return rc;
-          launch_alf(g, ctx->slots_dev, c0, m, ctl, 1, stream);
-          if (int rc = timed_end(ctx)) return rc;
-          ctx->launches++;
-        }
-        m = compact(false, true, ctl, bytes);
-        if (m) {
-          if (int rc = timed_begin(ctx, ILF_KERNEL_ALF_CHROMA, bytes)) return rc;
-          launch_alf(g, ctx->slots_dev, c0, m, ctl, 2, stream);
-          if (int rc = timed_end(ctx)) return rc;
-          ctx->launches++;
-        }
-      }
+      // luma and chroma bands are CTAs of one launch (they share the SMs), accounted under ILF_KERNEL_ALF_LUMA
+      if (int rc = stage_launch(-1, [&](const BatchCtl& ctl, int m) { launch_alf(g, ctx->slots_dev, c0, m, ctl, st); })) return rc;
     }
-    CU(ctx, cudaGetLastError());
   }
   return ILF_OK;
 }
 
 int ilf_run(ilf_ctx* ctx, int first_slot, int num_slots, unsigned stages) {
-  if (!ctx) return ILF_ERR_ARG;
-  if (first_slot < 0 || num_slots < 1 || first_slot + num_slots > (int)ctx->slots.size()) return fail(ctx, ILF_ERR_ARG, "slot range [%d,+%d) out of range", first_slot, num_slots);
+  if (int rc = check_range(ctx, first_slot, num_slots)) return rc;
   if (!(stages & ILF_STAGE_ALL)) return fail(ctx, ILF_ERR_ARG, "empty stage mask");
   // validate every requested stage of every slot before anything is launched or any buffer rotation is recorded
   for (int i = first_slot; i < first_slot + num_slots; i++) {
@@ -1209,61 +1209,51 @@ int ilf_run(ilf_ctx* ctx, int first_slot, int num_slots, unsigned stages) {
   // A full run always restarts from the uploaded input.
   if (stages & ILF_STAGE_DEBLOCK)
     for (int i = first_slot; i < first_slot + num_slots; i++) ctx->slots[i].result_buf[0] = ctx->slots[i].result_buf[1] = ctx->slots[i].result_buf[2] = 0;
-  // A chain over a large batch is dealt to the lanes (contiguous groups of slots, each group's stages on its own stream): the
-  // groups are independent, so one group's kernel fills the SMs that another group's draining kernel leaves idle.  Per-kernel
-  // timing keeps everything on the compute stream (serial kernels are what it measures).
+  // A chain over a large batch is dealt to the lanes (groups of slots, each group's stages on its own stream): the groups are
+  // independent, so one group's kernel fills the SMs that another group's draining kernel leaves idle.  Slots are dealt by estimated
+  // cost (planes x stages that run, ALF counted double), heaviest first to the least loaded lane, so that every lane carries a
+  // similar mix of kernels.  Per-kernel timing keeps everything on the compute stream (serial kernels are what it measures).
   const bool chain = (stages & (stages - 1)) != 0;
   const int lanes = (ctx->num_lanes > 1 && chain && !ctx->timing && num_slots >= ctx->lane_min_slots) ? ctx->num_lanes : 1;
-  // slot -> lane.  Policy 0: contiguous groups of equal size.  Policy 1: slots dealt by estimated cost (planes x stages that run,
-  // ALF counted double), heaviest first to the least loaded lane, so that every lane carries a similar mix of kernels.
   std::vector<uint8_t> lane_of(num_slots, 0);
   if (lanes > 1) {
-    if (ctx->lane_policy == 0) {
-      for (int i = 0; i < num_slots; i++) lane_of[i] = (uint8_t)((long long)i * lanes / num_slots);
-    } else {
-      std::vector<std::pair<int, int>> cost(num_slots);
-      for (int i = 0; i < num_slots; i++) {
-        const Slot& s = ctx->slots[first_slot + i];
-        int c = 0;
-        for (int p = 0; p < 3; p++) {
-          const int w = p == 0 ? 4 : 1;
-          if ((stages & ILF_STAGE_DEBLOCK) && (p == 0 || s.db_chroma)) c += w;
-          if ((stages & ILF_STAGE_SAO) && s.sao_on[p]) c += w;
-          if ((stages & ILF_STAGE_ALF) && s.alf_on[p]) c += 2 * w;
-        }
-        cost[i] = {-c, i};
+    std::vector<std::pair<int, int>> cost(num_slots);
+    for (int i = 0; i < num_slots; i++) {
+      const Slot& s = ctx->slots[first_slot + i];
+      int c = 0;
+      for (int p = 0; p < 3; p++) {
+        const int w = p == 0 ? 4 : 1;
+        if ((stages & ILF_STAGE_DEBLOCK) && (p == 0 || s.db_chroma)) c += w;
+        if ((stages & ILF_STAGE_SAO) && s.sao_on[p]) c += w;
+        if ((stages & ILF_STAGE_ALF) && s.alf_on[p]) c += 2 * w;
       }
-      std::sort(cost.begin(), cost.end());
-      int load[ilf_ctx::MAX_LANES] = {};
-      for (auto& ci : cost) {
-        int best = 0;
-        for (int l = 1; l < lanes; l++) if (load[l] < load[best]) best = l;
-        lane_of[ci.second] = (uint8_t)best;
-        load[best] -= ci.first;
-      }
+      cost[i] = {-c, i};
+    }
+    std::sort(cost.begin(), cost.end());
+    int load[ilf_ctx::MAX_LANES] = {};
+    for (auto& ci : cost) {
+      int best = 0;
+      for (int l = 1; l < lanes; l++) if (load[l] < load[best]) best = l;
+      lane_of[ci.second] = (uint8_t)best;
+      load[best] -= ci.first;
     }
   }
   int rc = ILF_OK;
   for (int gi = 0; gi < lanes; gi++) {
+    const int ring = lanes == 1 ? 0 : 1 + gi;
     cudaStream_t st = lanes == 1 ? ctx->stream : ctx->lane[gi];
-    int members = 0;
+    int member = -1;
     for (int i = 0; i < num_slots; i++) {
       if (lane_of[i] != gi) continue;
-      members++;
-      Slot& s = ctx->slots[first_slot + i];
-      if (s.h2d_pending) { CU(ctx, cudaStreamWaitEvent(st, s.ev_up, 0)); s.h2d_pending = false; }
-      if (s.d2h_pending) { CU(ctx, cudaStreamWaitEvent(st, s.ev_down, 0)); s.d2h_pending = false; }  // a download may still read the buffer this run overwrites
-      if (int rc2 = order_after_run(ctx, s, st)) return rc2;
+      member = first_slot + i;
+      if (int rc2 = join(ctx, ctx->slots[member], st, true)) return rc2;
     }
-    if (!members) continue;
+    if (member < 0) continue;
     for (int k = 0; k < 3 && rc == ILF_OK; k++)
-      if (stages & (1u << k)) rc = run_stage(ctx, first_slot, num_slots, k, st, lanes == 1 ? nullptr : lane_of.data(), gi);
-    // whatever was launched is fenced by the run event, also on an error path: later uploads / downloads of these slots wait for it
-    cudaEvent_t done = ctx->next_run_event(lanes == 1 ? 0 : 1 + gi);
-    CU(ctx, cudaEventRecord(done, st));
-    for (int i = 0; i < num_slots; i++)
-      if (lane_of[i] == gi) { ctx->slots[first_slot + i].ev_run = done; ctx->slots[first_slot + i].run_stream = st; }
-    if (lanes > 1) CU(ctx, cudaStreamWaitEvent(ctx->stream, done, 0));   // the compute stream joins the lane (the lane does not wait for anything)
+      if (stages & (1u << k)) rc = run_stage(ctx, first_slot, num_slots, k, st, ring, lane_of.data(), gi);
+    // whatever was launched is fenced, also on an error path: later uploads / downloads of these slots wait for it
+    if (int rc2 = fence(ctx, first_slot, num_slots, st, ring, lane_of.data(), gi)) return rc2;
+    if (lanes > 1) CU(ctx, cudaStreamWaitEvent(ctx->stream, ctx->slots[member].ev_run, 0));   // the compute stream joins the lane (the lane does not wait for anything)
   }
   return rc;
 }
@@ -1278,14 +1268,11 @@ int ilf_alf_classify(ilf_ctx* ctx, int slot, uint8_t* out) {
   Slot& s = ctx->slots[slot];
   if (!s.uploaded) return fail(ctx, ILF_ERR_STATE, "slot %d: classify before upload", slot);
   CU(ctx, cudaSetDevice(ctx->cfg.device));
-  if (s.h2d_pending) { CU(ctx, cudaStreamWaitEvent(ctx->stream, s.ev_up, 0)); s.h2d_pending = false; }
-  if (int rc = order_after_run(ctx, s, ctx->stream)) return rc;
+  if (int rc = join(ctx, s, ctx->stream, false)) return rc;
   BatchCtl ctl;
-  ctl.v[0] = (uint16_t)s.result_buf[0];
+  ctl.v[0] = (uint16_t)buf_word(s);
   ctl.slot[0] = 0;
-  launch_alf_classify(ctx->g, ctx->slots_dev, slot, 1, ctl, ctx->stream);
-  ctx->launches += 1;
-  CU(ctx, cudaGetLastError());
+  if (int rc = launch(ctx, -1, 0, 1, [&] { launch_alf_classify(ctx->g, ctx->slots_dev, slot, 1, ctl, ctx->stream); })) return rc;
   CU(ctx, cudaMemcpyAsync(out, s.alf_class, (size_t)ctx->g.units_w * ctx->g.units_h, cudaMemcpyDeviceToHost, ctx->stream));
   CU(ctx, cudaStreamSynchronize(ctx->stream));
   return ILF_OK;
@@ -1314,9 +1301,9 @@ static int set_original_rows(ilf_ctx* ctx, int slot, const int16_t* y, ptrdiff_t
   const int16_t* srcs[3] = {y, cb, cr};
   const ptrdiff_t strides[3] = {sy, scb, scr};
   for (int p = 0; p < 3; p++) {
-    const int sh = p ? 1 : 0, w = g.width >> sh, h = n >> sh, pitch = p ? g.pitch_c : g.pitch_y;
+    const PlaneRows pr = plane_rows(g, p, first, n);
     // pageable sources are staged by the runtime (the call returns when the source may be reused); page-locked ones are asynchronous
-    CU(ctx, cudaMemcpy2DAsync(const_cast<int16_t*>(s.dev.org[p]) + (size_t)(first >> sh) * pitch, (size_t)pitch * 2, srcs[p], (size_t)strides[p] * 2, (size_t)w * 2, h,
+    CU(ctx, cudaMemcpy2DAsync(const_cast<int16_t*>(s.dev.org[p]) + (size_t)pr.r0 * pr.pitch, (size_t)pr.pitch * 2, srcs[p], (size_t)strides[p] * 2, (size_t)pr.w * 2, pr.h,
                               cudaMemcpyHostToDevice, ctx->s_up));
   }
   CU(ctx, cudaMemcpyAsync(s.stats_avail, ctu_avail, ctx->num_ctus, cudaMemcpyHostToDevice, ctx->s_up));
@@ -1348,35 +1335,23 @@ static int own_ctus(const ilf_ctx* ctx) { return ctx->is_band ? ctx->band.num_ct
 static bool band_org_missing(const ilf_ctx* ctx, const Slot& s) { return ctx->is_band && !s.org_since_upload; }
 
 int ilf_sao_stats(ilf_ctx* ctx, int first_slot, int num_slots) {
-  if (!ctx) return ILF_ERR_ARG;
-  if (first_slot < 0 || num_slots < 1 || first_slot + num_slots > (int)ctx->slots.size()) return fail(ctx, ILF_ERR_ARG, "slot range [%d,+%d) out of range", first_slot, num_slots);
+  if (int rc = check_range(ctx, first_slot, num_slots)) return rc;
+  for (int i = first_slot; i < first_slot + num_slots; i++) {
+    const Slot& s = ctx->slots[i];
+    if (!s.uploaded || !s.has_org || band_org_missing(ctx, s)) return fail(ctx, ILF_ERR_STATE, "slot %d: statistics need ilf_upload and ilf_set_original", i);
+  }
   CU(ctx, cudaSetDevice(ctx->cfg.device));
   const Geom& g = ctx->g;
-  for (int i = first_slot; i < first_slot + num_slots; i++) {
-    Slot& s = ctx->slots[i];
-    if (!s.uploaded || !s.has_org || band_org_missing(ctx, s)) return fail(ctx, ILF_ERR_STATE, "slot %d: statistics need ilf_upload and ilf_set_original", i);
-    if (s.h2d_pending) { CU(ctx, cudaStreamWaitEvent(ctx->stream, s.ev_up, 0)); s.h2d_pending = false; }
-    if (int rc = order_after_run(ctx, s, ctx->stream)) return rc;
-  }
+  for (int i = first_slot; i < first_slot + num_slots; i++)
+    if (int rc = join(ctx, ctx->slots[i], ctx->stream, false)) return rc;
   for (int c0 = first_slot; c0 < first_slot + num_slots; c0 += MAX_BATCH) {
     const int cn = std::min(MAX_BATCH, first_slot + num_slots - c0);
     BatchCtl ctl;
-    for (int i = 0; i < cn; i++) {
-      const Slot& s = ctx->slots[c0 + i];
-      ctl.v[i] = (uint16_t)(s.result_buf[0] | (s.result_buf[1] << 2) | (s.result_buf[2] << 4));
-      ctl.slot[i] = (uint8_t)i;
-    }
+    compact(ctx, c0, cn, -1, ctl, [&](int i) { return (int)buf_word(ctx->slots[c0 + i]); });
     // algorithmic bytes: the deblocked and the original picture (own rows) are read once (2 B x 1.5 samples x 2 pictures per luma pixel)
-    if (int rc = timed_begin(ctx, ILF_KERNEL_SAO_STATS, 6.0 * g.width * g.out_rows * cn)) return rc;
-    launch_sao_stats(g, ctx->slots_dev, c0, cn, ctl, ctx->stream);
-    if (int rc = timed_end(ctx)) return rc;
-    ctx->launches++;
-    CU(ctx, cudaGetLastError());
+    if (int rc = launch(ctx, ILF_KERNEL_SAO_STATS, 6.0 * g.width * g.out_rows * cn, 1, [&] { launch_sao_stats(g, ctx->slots_dev, c0, cn, ctl, ctx->stream); })) return rc;
   }
-  cudaEvent_t done = ctx->next_run_event(0);
-  CU(ctx, cudaEventRecord(done, ctx->stream));
-  for (int i = first_slot; i < first_slot + num_slots; i++) { ctx->slots[i].ev_run = done; ctx->slots[i].run_stream = ctx->stream; }
-  return ILF_OK;
+  return fence(ctx, first_slot, num_slots, ctx->stream, 0);
 }
 
 int ilf_get_sao_stats(ilf_ctx* ctx, int slot, int64_t* out) {
@@ -1392,45 +1367,38 @@ int ilf_get_sao_stats(ilf_ctx* ctx, int slot, int64_t* out) {
 
 // Encoder ALF statistics: block classification of the slots' current pictures, then the covariance launches (ilf_alf_stats.cu).
 int ilf_alf_stats(ilf_ctx* ctx, int first_slot, int num_slots) {
-  if (!ctx) return ILF_ERR_ARG;
-  if (first_slot < 0 || num_slots < 1 || first_slot + num_slots > (int)ctx->slots.size()) return fail(ctx, ILF_ERR_ARG, "slot range [%d,+%d) out of range", first_slot, num_slots);
+  if (int rc = check_range(ctx, first_slot, num_slots)) return rc;
   for (int i = first_slot; i < first_slot + num_slots; i++)
     if (band_org_missing(ctx, ctx->slots[i])) return fail(ctx, ILF_ERR_STATE, "not available on band contexts");
+  for (int i = first_slot; i < first_slot + num_slots; i++) {
+    const Slot& s = ctx->slots[i];
+    if (!s.uploaded || !s.has_org) return fail(ctx, ILF_ERR_STATE, "slot %d: statistics need ilf_upload and ilf_set_original", i);
+  }
   CU(ctx, cudaSetDevice(ctx->cfg.device));
   const Geom& g = ctx->g;
   const size_t bytes = (size_t)own_ctus(ctx) * ILF_ALF_STATS_WORDS * sizeof(long long);
   for (int i = first_slot; i < first_slot + num_slots; i++) {
     Slot& s = ctx->slots[i];
-    if (!s.uploaded || !s.has_org) return fail(ctx, ILF_ERR_STATE, "slot %d: statistics need ilf_upload and ilf_set_original", i);
     if (!s.alf_stats) {
       CU(ctx, cudaMalloc(&s.alf_stats, bytes));
       s.dev.alf_stats = s.alf_stats;
       if (int rc = push_desc(ctx, i)) return rc;
     }
-    if (s.h2d_pending) { CU(ctx, cudaStreamWaitEvent(ctx->stream, s.ev_up, 0)); s.h2d_pending = false; }
-    if (int rc = order_after_run(ctx, s, ctx->stream)) return rc;
+    if (int rc = join(ctx, s, ctx->stream, false)) return rc;
     CU(ctx, cudaMemsetAsync(s.alf_stats, 0, bytes, ctx->stream));
   }
   for (int c0 = first_slot; c0 < first_slot + num_slots; c0 += MAX_BATCH) {
     const int cn = std::min(MAX_BATCH, first_slot + num_slots - c0);
     BatchCtl ctl;
-    for (int i = 0; i < cn; i++) {
-      const Slot& s = ctx->slots[c0 + i];
-      ctl.v[i] = (uint16_t)(s.result_buf[0] | (s.result_buf[1] << 2) | (s.result_buf[2] << 4));
-      ctl.slot[i] = (uint8_t)i;
-    }
+    compact(ctx, c0, cn, -1, ctl, [&](int i) { return (int)buf_word(ctx->slots[c0 + i]); });
     // algorithmic bytes: the reconstructed and the original picture (own rows) are read once (2 B x 1.5 samples x 2 pictures per luma pixel)
-    if (int rc = timed_begin(ctx, ILF_KERNEL_ALF_STATS, 6.0 * g.width * g.out_rows * cn)) return rc;
-    launch_alf_classify(g, ctx->slots_dev, c0, cn, ctl, ctx->stream);
-    launch_alf_stats(g, ctx->slots_dev, c0, cn, ctl, ctx->stream);
-    if (int rc = timed_end(ctx)) return rc;
-    ctx->launches += 4;
-    CU(ctx, cudaGetLastError());
+    if (int rc = launch(ctx, ILF_KERNEL_ALF_STATS, 6.0 * g.width * g.out_rows * cn, 4, [&] {
+          launch_alf_classify(g, ctx->slots_dev, c0, cn, ctl, ctx->stream);
+          launch_alf_stats(g, ctx->slots_dev, c0, cn, ctl, ctx->stream);
+        }))
+      return rc;
   }
-  cudaEvent_t done = ctx->next_run_event(0);
-  CU(ctx, cudaEventRecord(done, ctx->stream));
-  for (int i = first_slot; i < first_slot + num_slots; i++) { ctx->slots[i].ev_run = done; ctx->slots[i].run_stream = ctx->stream; }
-  return ILF_OK;
+  return fence(ctx, first_slot, num_slots, ctx->stream, 0);
 }
 
 int ilf_get_alf_stats(ilf_ctx* ctx, int slot, int64_t* out) {
@@ -1448,8 +1416,7 @@ int ilf_get_alf_stats(ilf_ctx* ctx, int slot, int64_t* out) {
 // Encoder deblocking parameter search (include/ilf_b200.h; EncGOP::applyDeblockingFilterParameterSelection)
 // ---------------------------------------------------------------------------------------------------------------
 int ilf_deblock_search(ilf_ctx* ctx, int first_slot, int num_slots, const ilf_deblock_candidate* cands, int num_cands, const int32_t shift[2]) {
-  if (!ctx) return ILF_ERR_ARG;
-  if (first_slot < 0 || num_slots < 1 || first_slot + num_slots > (int)ctx->slots.size()) return fail(ctx, ILF_ERR_ARG, "slot range [%d,+%d) out of range", first_slot, num_slots);
+  if (int rc = check_range(ctx, first_slot, num_slots)) return rc;
   if (!cands || !shift) return fail(ctx, ILF_ERR_ARG, "null pointer");
   if (num_cands < 1 || num_cands > ILF_DEBLOCK_SEARCH_MAX) return fail(ctx, ILF_ERR_ARG, "num_cands %d outside 1..%d", num_cands, ILF_DEBLOCK_SEARCH_MAX);
   if (shift[0] < 0 || shift[0] > 31 || shift[1] < 0 || shift[1] > 31) return fail(ctx, ILF_ERR_ARG, "shift (%d, %d) outside 0..31", shift[0], shift[1]);
@@ -1463,37 +1430,23 @@ int ilf_deblock_search(ilf_ctx* ctx, int first_slot, int num_slots, const ilf_de
   CU(ctx, cudaSetDevice(ctx->cfg.device));
   constexpr size_t ROW = (size_t)ILF_DEBLOCK_SEARCH_MAX * 3;
   if (!ctx->search_out) CU(ctx, cudaMalloc(&ctx->search_out, ctx->slots.size() * ROW * sizeof(unsigned long long)));
-  for (int i = first_slot; i < first_slot + num_slots; i++) {
-    Slot& s = ctx->slots[i];
-    if (s.h2d_pending) { CU(ctx, cudaStreamWaitEvent(ctx->stream, s.ev_up, 0)); s.h2d_pending = false; }
-    if (int rc = order_after_run(ctx, s, ctx->stream)) return rc;
-  }
+  for (int i = first_slot; i < first_slot + num_slots; i++)
+    if (int rc = join(ctx, ctx->slots[i], ctx->stream, false)) return rc;
   CU(ctx, cudaMemsetAsync(ctx->search_out + first_slot * ROW, 0, num_slots * ROW * sizeof(unsigned long long), ctx->stream));
   for (int c0 = first_slot; c0 < first_slot + num_slots; c0 += MAX_BATCH) {
     const int cn = std::min(MAX_BATCH, first_slot + num_slots - c0);
-    // one launch per motion-vector representation present (none / int16 / int32 are different kernels)
     for (int mode = 0; mode < 3; mode++) {
       BatchCtl ctl;
-      int m = 0;
-      for (int i = 0; i < cn; i++) {
-        if (ctx->slots[c0 + i].mv_mode != mode) continue;
-        ctl.v[m] = 0;   // every plane from buffer 0, the uploaded picture
-        ctl.slot[m] = (uint8_t)i;
-        m++;
-      }
-      if (!m) continue;
-      launch_deblock_search(ctx->g, ctx->slots_dev, c0, m, ctl, mode, cands, num_cands, shift[0], shift[1], ctx->search_out, ctx->stream);
-      ctx->launches++;
-      CU(ctx, cudaGetLastError());
+      const int m = compact(ctx, c0, cn, mode, ctl, [](int) { return 0; });   // every plane from buffer 0, the uploaded picture
+      if (m)
+        if (int rc = launch(ctx, -1, 0, 1, [&] {
+              launch_deblock_search(ctx->g, ctx->slots_dev, c0, m, ctl, mode, cands, num_cands, shift[0], shift[1], ctx->search_out, ctx->stream);
+            }))
+          return rc;
     }
   }
-  cudaEvent_t done = ctx->next_run_event(0);
-  CU(ctx, cudaEventRecord(done, ctx->stream));
-  for (int i = first_slot; i < first_slot + num_slots; i++) {
-    ctx->slots[i].ev_run = done;
-    ctx->slots[i].run_stream = ctx->stream;
-    ctx->slots[i].search_k = num_cands;
-  }
+  if (int rc = fence(ctx, first_slot, num_slots, ctx->stream, 0)) return rc;
+  for (int i = first_slot; i < first_slot + num_slots; i++) ctx->slots[i].search_k = num_cands;
   return ILF_OK;
 }
 

@@ -162,7 +162,7 @@ void launch_deblock(const Geom& g, const SlotDev* slots, int first_slot, int num
 void launch_deblock_search(const Geom& g, const SlotDev* slots, int first_slot, int num_slots, const BatchCtl& ctl, int mv_mode, const ilf_deblock_candidate* cands,
                            int num_cands, int shift_luma, int shift_chroma, unsigned long long* out, cudaStream_t st);
 void launch_sao(const Geom& g, const SlotDev* slots, int first_slot, int num_slots, const BatchCtl& ctl, cudaStream_t st);
-void launch_alf(const Geom& g, const SlotDev* slots, int first_slot, int num_slots, const BatchCtl& ctl, int planes /* bit 0 luma, bit 1 chroma */, cudaStream_t st);
+void launch_alf(const Geom& g, const SlotDev* slots, int first_slot, int num_slots, const BatchCtl& ctl, cudaStream_t st);
 void launch_sao_stats(const Geom& g, const SlotDev* slots, int first_slot, int num_slots, const BatchCtl& ctl, cudaStream_t st);
 cudaError_t picture_hash(const Geom& g, const int16_t* const planes[3], uint32_t* scratch, cudaStream_t st, uint32_t out_crc[3], uint32_t out_sum[3]);
 // The same kernels over luma rows [first, first + n) of the held planes (chroma halved), y0 = their first picture row: the CRC register

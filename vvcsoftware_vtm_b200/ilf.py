@@ -349,7 +349,7 @@ class InLoopFilter:
     def set_timing(self, on):
         self._ck(self._lib.ilf_set_timing(self._h, int(on)))
 
-    KERNELS = ("deblock", "sao", "alf", "alf_chroma", "sao_stats", "alf_stats")   # "alf" = the whole ALF stage (one launch); with ILF_ALF_SPLIT=1: luma only, "alf_chroma" the second launch
+    KERNELS = ("deblock", "sao", "alf", "alf_chroma", "sao_stats", "alf_stats")   # "alf" = the whole ALF stage (one launch); "alf_chroma" is reserved, always zero
 
     def kernel_times(self):
         """{kernel: (total ms, launches, algorithmic bytes)} since set_timing(True); synchronises the context's stream."""
