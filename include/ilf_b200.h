@@ -103,6 +103,56 @@ int ilf_host_register(void* p, size_t bytes);   /* page-lock an existing allocat
 int ilf_host_unregister(void* p);
 
 /* ---------------------------------------------------------------------------------------------
+ * Pictures in device memory.  A caller whose picture is already on the GPU (a GPU decoder's reconstruction, an encoder's source
+ * frames, a GPU consumer of the filtered picture) hands its planes over without a trip through host memory.  The planes are
+ * plain device memory (cudaMalloc, a torch CUDA tensor, ...) of the context's device: managed memory, host memory and memory of
+ * another device are refused.  Strides are in SAMPLES.  On a whole-picture context a call covers the whole picture; on a band
+ * context the band's OWN rows (ilf_get_band_rows), as ilf_upload_band / ilf_download_band / ilf_set_original_band do -- the halo
+ * rows still come from ilf_band_exchange.
+ *
+ *   ilf_upload_device        as ilf_upload: side information must be set again, every plane's current picture is the upload
+ *   ilf_set_original_device  as ilf_set_original, or on a band context as ilf_set_original_band (ILF_ERR_STATE before the slot's
+ *                            upload); ctu_avail is HOST memory, read as ilf_set_original reads it (a pageable array is copied before
+ *                            the call returns)
+ *   ilf_download_device      writes what ilf_download returns (each plane from the buffer its last stage left it in); ILF_ERR_STATE
+ *                            before an upload
+ *
+ * Samples (fmt, NULL = int16 at the context's depths).  The conversion is per plane: b = the context's depth of the plane's channel,
+ * c = the caller's; upload and original go c -> b, download b -> c.  With d = destination depth - source depth, computed in int32
+ * and stored as the destination type:
+ *   d > 0   v << d                                               (no clipping)
+ *   d < 0   clip3(0, 2^dst_depth - 1, (v + (1 << (-d - 1))) >> -d)
+ *   d = 0   v, bit for bit: int16 at the context's depth is exactly what ilf_upload / ilf_download move
+ * An int16 container holds an unsigned sample (so a 16-bit sample of 65535 is the int16 -1).  This is the scaling of VTM's YUV
+ * reader and writer: 8-bit frames for a 10-bit context are shifted left by 2, a 10-bit picture downloaded as uint8 is rounded and
+ * clipped.
+ *
+ * Ordering.  The call returns without waiting.  The transfer runs after all work issued to `stream` before the call and before all
+ * work issued to `stream` after it, so the caller may overwrite its source, or read its destination, on `stream` at once.  Inside
+ * the context the transfer is ordered as its host twin: an upload or original waits for the slot's last run and download, a
+ * download for the slot's last run and upload, and the slot's next run or upload waits for the download.  ilf_wait(slot) and
+ * ilf_sync cover these transfers.  `stream` is a cudaStream_t on the context's device (NULL: the legacy default stream).
+ *
+ * Errors.  ILF_ERR_ARG, before anything is enqueued (the slot is left as it was), for: a NULL pointer, a slot out of range, a plane
+ * that is not device memory of the context's device, a stride shorter than the plane's width, an int16 plane that is not 2-byte
+ * aligned, an unknown type, a depth outside the ranges below.  The host calls (ilf_upload, ilf_download_async, ilf_set_original
+ * and their band twins) return ILF_ERR_ARG for device memory.
+ * ------------------------------------------------------------------------------------------- */
+#define ILF_SAMPLES_I16 0   /* int16, as every host transfer takes it */
+#define ILF_SAMPLES_U8 1    /* one byte per sample                    */
+typedef struct {
+  int32_t type;          /* ILF_SAMPLES_*                                                                     */
+  int32_t bit_depth[2];  /* luma, chroma depth of the CALLER's samples.  I16: 8..16, 0 = the context's; U8: 8 (0 means 8) */
+} ilf_samples;
+
+int ilf_upload_device(ilf_ctx* ctx, int slot, const void* y, ptrdiff_t stride_y, const void* cb, ptrdiff_t stride_cb, const void* cr,
+                      ptrdiff_t stride_cr, const ilf_samples* fmt, void* stream);
+int ilf_download_device(ilf_ctx* ctx, int slot, void* y, ptrdiff_t stride_y, void* cb, ptrdiff_t stride_cb, void* cr, ptrdiff_t stride_cr,
+                        const ilf_samples* fmt, void* stream);
+int ilf_set_original_device(ilf_ctx* ctx, int slot, const void* y, ptrdiff_t stride_y, const void* cb, ptrdiff_t stride_cb, const void* cr,
+                            ptrdiff_t stride_cr, const uint8_t* ctu_avail /* HOST, [ctus_h*ctus_w] */, const ilf_samples* fmt, void* stream);
+
+/* ---------------------------------------------------------------------------------------------
  * Deblocking side information: the packed per-4x4 CU/TU metadata grid.
  *
  * One uint32 per 4x4 luma unit, raster order, units_w = width/4 (what the reference looks up per
@@ -308,9 +358,11 @@ int ilf_download_extended(ilf_ctx* ctx, int slot, int16_t* y, ptrdiff_t stride_y
 /* ---------------------------------------------------------------------------------------------
  * Measurement helpers (bench.py).  Accumulated device time per kernel in milliseconds since
  * ilf_set_timing(ctx, 1) (CUDA event pairs around every launch on the context's stream, collected
- * without synchronising inside ilf_run), number of kernel launches issued since ilf_create, and
- * raw device pointers of a slot's input planes so that synthetic pictures can be generated on the
- * device. planes[0..2] = Y, Cb, Cr; pitch in samples.
+ * without synchronising inside ilf_run), number of kernel launches issued since ilf_create (the
+ * conversion kernel of the device transfers included; it has no timing slot), and raw device
+ * pointers of a slot's input planes so that synthetic pictures can be generated on the device.
+ * planes[0..2] = Y, Cb, Cr; pitch in samples.  These pointers carry no ordering: a caller's
+ * picture enters and leaves through the device transfers above.
  * ------------------------------------------------------------------------------------------- */
 #define ILF_KERNEL_DEBLOCK 0
 #define ILF_KERNEL_SAO 1

@@ -166,6 +166,7 @@ struct ilf_ctx {
   int* db_work = nullptr;             // tile queues of the deblocking kernel: two ints per stream (the compute stream, then the lanes)
   unsigned long long* search_out = nullptr;   // ilf_deblock_search: [num_slots][ILF_DEBLOCK_SEARCH_MAX][3], allocated by the first search
   cudaEvent_t chunk_ev[COPY_CHUNKS_MAX] = {};   // download: chunk i has reached the staging buffer
+  cudaEvent_t ev_caller = nullptr;   // device transfers: the caller's stream up to the call (recorded, then waited for at once)
 };
 
 namespace {
@@ -355,12 +356,27 @@ int push_desc(ilf_ctx* ctx, int slot) {
   return ILF_OK;
 }
 
+// What a pointer addresses: cudaMemoryTypeUnregistered (pageable host memory), cudaMemoryTypeHost (page-locked), cudaMemoryTypeDevice
+// or cudaMemoryTypeManaged.  `device` (when given) receives the device of device memory.
+cudaMemoryType mem_type(const void* p, int* device = nullptr) {
+  cudaPointerAttributes at;
+  if (cudaPointerGetAttributes(&at, p) != cudaSuccess) { cudaGetLastError(); return cudaMemoryTypeUnregistered; }
+  if (device) *device = at.device;
+  return at.type;
+}
+
 // Page-locked (cudaHostAlloc / cudaHostRegister / ilf_host_alloc) host memory can be the source or target of an
 // asynchronous copy directly; pageable memory goes through the slot's pinned staging buffer.
-bool is_pinned(const void* p) {
-  cudaPointerAttributes at;
-  if (cudaPointerGetAttributes(&at, p) != cudaSuccess) { cudaGetLastError(); return false; }
-  return at.type == cudaMemoryTypeHost;
+bool is_pinned(const void* p) { return mem_type(p) == cudaMemoryTypeHost; }
+
+// The host transfers copy with host memcpy or as host <-> device copies: a plane in device memory is refused (its twin is `device_call`).
+int refuse_device_planes(ilf_ctx* ctx, const void* y, const void* cb, const void* cr, cudaMemoryType types[3], const char* device_call) {
+  const void* planes[3] = {y, cb, cr};
+  for (int p = 0; p < 3; p++) {
+    types[p] = mem_type(planes[p]);
+    if (types[p] == cudaMemoryTypeDevice) return fail(ctx, ILF_ERR_ARG, "plane %d is device memory: use %s", p, device_call);
+  }
+  return ILF_OK;
 }
 
 // A side-information setter stages its arrays between side_begin and side_end: host -> pinned staging region k of the slot ->
@@ -466,6 +482,7 @@ int create_impl(ilf_ctx** out, const ilf_config* cfg, const ilf_band* band) {
   *out = ctx;  // from here on errors are reported through ctx->err and the caller destroys
 
   CU(ctx, cudaSetDevice(cfg->device));
+  CU(ctx, cudaEventCreateWithFlags(&ctx->ev_caller, cudaEventDisableTiming));
   CU(ctx, cudaStreamCreateWithFlags(&ctx->stream, cudaStreamNonBlocking));
   CU(ctx, cudaStreamCreateWithFlags(&ctx->s_up, cudaStreamNonBlocking));
   CU(ctx, cudaStreamCreateWithFlags(&ctx->s_down, cudaStreamNonBlocking));
@@ -583,6 +600,7 @@ int ilf_destroy(ilf_ctx* ctx) {
   for (auto& ring : ctx->run_ring)
     for (cudaEvent_t e : ring) if (e) cudaEventDestroy(e);
   for (cudaEvent_t e : ctx->chunk_ev) if (e) cudaEventDestroy(e);
+  if (ctx->ev_caller) cudaEventDestroy(ctx->ev_caller);
   cudaFree(ctx->slots_dev);
   cudaFree(ctx->hash_scratch);
   cudaFree(ctx->db_work);
@@ -627,19 +645,54 @@ static int make_chunks(const Geom& g, int first, int n, CopyChunk* out) {
   return k;
 }
 
+// The state changes of a transfer, shared by the host calls and the device calls (ilf_*_device).
+// Before a new picture is written into buffer 0: that buffer may still be read by kernels of the slot's previous picture, or by its
+// download when no stage ran on a plane.
+static int upload_begin(ilf_ctx* ctx, Slot& s) {
+  CU(ctx, cudaStreamWaitEvent(ctx->s_up, s.ev_run, 0));
+  CU(ctx, cudaStreamWaitEvent(ctx->s_up, s.ev_down, 0));
+  return ILF_OK;
+}
+
+// After the copies of a new picture are issued on the upload stream: the side information must be set again, the original is
+// stale for the deblocking search, and every plane's current picture is the upload.
+static int upload_end(ilf_ctx* ctx, Slot& s) {
+  CU(ctx, cudaEventRecord(s.ev_up, ctx->s_up));
+  s.h2d_pending = true;
+  s.uploaded = true;
+  s.has_db = s.has_sao = s.has_alf = false;
+  s.org_since_upload = false;
+  s.result_buf[0] = s.result_buf[1] = s.result_buf[2] = 0;
+  return ILF_OK;
+}
+
+// A download reads each plane's current buffer: after the slot's last kernels, and after its upload when no stage ran on a plane.
+static int download_begin(ilf_ctx* ctx, Slot& s) {
+  CU(ctx, cudaStreamWaitEvent(ctx->s_down, s.ev_run, 0));
+  CU(ctx, cudaStreamWaitEvent(ctx->s_down, s.ev_up, 0));
+  return ILF_OK;
+}
+
+// An asynchronous download is pending: ilf_wait waits for it, the slot's next run and upload are ordered after it.
+static int download_end(ilf_ctx* ctx, Slot& s) {
+  CU(ctx, cudaEventRecord(s.ev_down, ctx->s_down));
+  s.d2h_pending = true;
+  return ILF_OK;
+}
+
 // Copies host rows [first, first + n) (LOCAL luma rows of the held region; chroma rows first/2 ..) into the slot's input buffer.
 static int upload_rows(ilf_ctx* ctx, int slot, const int16_t* y, ptrdiff_t sy, const int16_t* cb, ptrdiff_t scb, const int16_t* cr, ptrdiff_t scr, int first, int n) {
   if (int rc = check_slot(ctx, slot)) return rc;
   if (!y || !cb || !cr) return fail(ctx, ILF_ERR_ARG, "null plane pointer");
+  cudaMemoryType types[3];
+  if (int rc = refuse_device_planes(ctx, y, cb, cr, types, "ilf_upload_device")) return rc;
   Slot& s = ctx->slots[slot];
   const Geom& g = ctx->g;
   CU(ctx, cudaSetDevice(ctx->cfg.device));
-  // buffer 0 may still be read by kernels of the slot's previous picture, or by its download when no stage ran on a plane
-  CU(ctx, cudaStreamWaitEvent(ctx->s_up, s.ev_run, 0));
-  CU(ctx, cudaStreamWaitEvent(ctx->s_up, s.ev_down, 0));
+  if (int rc = upload_begin(ctx, s)) return rc;
   const int16_t* srcs[3] = {y, cb, cr};
   const ptrdiff_t strides[3] = {sy, scb, scr};
-  if (is_pinned(y) && is_pinned(cb) && is_pinned(cr)) {
+  if (types[0] == cudaMemoryTypeHost && types[1] == cudaMemoryTypeHost && types[2] == cudaMemoryTypeHost) {
     for (int p = 0; p < 3; p++) {
       const PlaneRows pr = plane_rows(g, p, first, n);
       CU(ctx, cudaMemcpy2DAsync(plane_ptr(ctx, s, 0, p) + (size_t)pr.r0 * pr.pitch, (size_t)pr.pitch * 2, srcs[p], (size_t)strides[p] * 2, (size_t)pr.w * 2, pr.h, cudaMemcpyHostToDevice, ctx->s_up));
@@ -676,13 +729,7 @@ static int upload_rows(ilf_ctx* ctx, int slot, const int16_t* y, ptrdiff_t sy, c
     if (par) ctx->copy_pool.wait();
     CU(ctx, err);
   }
-  CU(ctx, cudaEventRecord(s.ev_up, ctx->s_up));
-  s.h2d_pending = true;
-  s.uploaded = true;
-  s.has_db = s.has_sao = s.has_alf = false;
-  s.org_since_upload = false;
-  s.result_buf[0] = s.result_buf[1] = s.result_buf[2] = 0;
-  return ILF_OK;
+  return upload_end(ctx, s);
 }
 
 // Host planes cover the rows the context HOLDS: the whole picture, or for a band context picture rows
@@ -703,22 +750,21 @@ int ilf_upload_band(ilf_ctx* ctx, int slot, const int16_t* y, ptrdiff_t sy, cons
 static int download_rows(ilf_ctx* ctx, int slot, int16_t* y, ptrdiff_t sy, int16_t* cb, ptrdiff_t scb, int16_t* cr, ptrdiff_t scr, int first, int n) {
   if (int rc = check_slot(ctx, slot)) return rc;
   if (!y || !cb || !cr) return fail(ctx, ILF_ERR_ARG, "null plane pointer");
+  cudaMemoryType types[3];
+  if (int rc = refuse_device_planes(ctx, y, cb, cr, types, "ilf_download_device")) return rc;
   Slot& s = ctx->slots[slot];
   if (!s.uploaded) return fail(ctx, ILF_ERR_STATE, "slot %d: download before upload", slot);
   const Geom& g = ctx->g;
   CU(ctx, cudaSetDevice(ctx->cfg.device));
-  CU(ctx, cudaStreamWaitEvent(ctx->s_down, s.ev_run, 0));
-  CU(ctx, cudaStreamWaitEvent(ctx->s_down, s.ev_up, 0));  // a picture that no stage touched is read from the upload buffer
+  if (int rc = download_begin(ctx, s)) return rc;
   int16_t* dsts[3] = {y, cb, cr};
   const ptrdiff_t strides[3] = {sy, scb, scr};
-  if (is_pinned(y) && is_pinned(cb) && is_pinned(cr)) {
+  if (types[0] == cudaMemoryTypeHost && types[1] == cudaMemoryTypeHost && types[2] == cudaMemoryTypeHost) {
     for (int p = 0; p < 3; p++) {
       const PlaneRows pr = plane_rows(g, p, first, n);
       CU(ctx, cudaMemcpy2DAsync(dsts[p], (size_t)strides[p] * 2, plane_ptr(ctx, s, s.result_buf[p], p) + (size_t)pr.r0 * pr.pitch, (size_t)pr.pitch * 2, (size_t)pr.w * 2, pr.h, cudaMemcpyDeviceToHost, ctx->s_down));
     }
-    CU(ctx, cudaEventRecord(s.ev_down, ctx->s_down));
-    s.d2h_pending = true;
-    return ILF_OK;
+    return download_end(ctx, s);
   }
   // staged: the DMA engine delivers row chunks into the page-locked buffer, helper threads (and this one) copy every chunk on to
   // the caller's planes as soon as its event has fired
@@ -1283,12 +1329,9 @@ int ilf_alf_classify(ilf_ctx* ctx, int slot, uint8_t* out) {
 // ---------------------------------------------------------------------------------------------------------------
 // Copies the source picture's LOCAL luma rows [first, first + n) of the held region (chroma rows halved) and the full picture's
 // ctu_avail.  The original lives in the held-row layout of the slot's buffers, so the kernels address it as they address the picture.
-static int set_original_rows(ilf_ctx* ctx, int slot, const int16_t* y, ptrdiff_t sy, const int16_t* cb, ptrdiff_t scb, const int16_t* cr, ptrdiff_t scr,
-                             const uint8_t* ctu_avail, int first, int n) {
-  if (!y || !cb || !cr || !ctu_avail) return fail(ctx, ILF_ERR_ARG, "null pointer");
-  Slot& s = ctx->slots[slot];
-  const Geom& g = ctx->g;
-  CU(ctx, cudaSetDevice(ctx->cfg.device));
+// The original's buffers (allocated on first use), and the upload stream ordered after the slot's kernels: a statistics kernel of the
+// previous picture may still read the planes and ctu_avail.
+static int original_begin(ilf_ctx* ctx, Slot& s) {
   if (!s.org) {
     CU(ctx, cudaMalloc(&s.org, ctx->buf_elems * sizeof(int16_t)));
     CU(ctx, cudaMalloc(&s.stats_avail, ctx->num_ctus));
@@ -1297,7 +1340,42 @@ static int set_original_rows(ilf_ctx* ctx, int slot, const int16_t* y, ptrdiff_t
     s.dev.stats_avail = s.stats_avail;
     s.dev.stats = s.stats;
   }
-  CU(ctx, cudaStreamWaitEvent(ctx->s_up, s.ev_run, 0));  // a statistics kernel of the previous picture may still read the planes
+  CU(ctx, cudaStreamWaitEvent(ctx->s_up, s.ev_run, 0));
+  return ILF_OK;
+}
+
+// The full picture's ctu_avail from host memory; a pageable array is copied before the call returns (the caller may reuse it).
+static int original_avail(ilf_ctx* ctx, Slot& s, const uint8_t* ctu_avail) {
+  CU(ctx, cudaMemcpyAsync(s.stats_avail, ctu_avail, ctx->num_ctus, cudaMemcpyHostToDevice, ctx->s_up));
+  if (!is_pinned(ctu_avail)) CU(ctx, cudaStreamSynchronize(ctx->s_up));
+  return ILF_OK;
+}
+
+// After the original's copies are issued: the statistics and the search of the slot may run.
+static int original_end(ilf_ctx* ctx, int slot) {
+  Slot& s = ctx->slots[slot];
+  s.has_org = true;
+  s.org_since_upload = true;
+  return push_desc(ctx, slot);
+}
+
+// A whole-picture context takes the original at any time; a band context after the slot's upload (ilf_set_original_band).
+static int check_original(ilf_ctx* ctx, int slot, bool band_call) {
+  if (ctx->is_band != band_call)
+    return fail(ctx, ILF_ERR_STATE, band_call ? "not a band context (ilf_set_original takes the whole picture)" : "SAO statistics are not available on band contexts");
+  if (band_call && !ctx->slots[slot].uploaded) return fail(ctx, ILF_ERR_STATE, "slot %d: ilf_set_original_band before the slot's upload", slot);
+  return ILF_OK;
+}
+
+static int set_original_rows(ilf_ctx* ctx, int slot, const int16_t* y, ptrdiff_t sy, const int16_t* cb, ptrdiff_t scb, const int16_t* cr, ptrdiff_t scr,
+                             const uint8_t* ctu_avail, int first, int n) {
+  if (!y || !cb || !cr || !ctu_avail) return fail(ctx, ILF_ERR_ARG, "null pointer");
+  cudaMemoryType types[3];
+  if (int rc = refuse_device_planes(ctx, y, cb, cr, types, "ilf_set_original_device")) return rc;
+  Slot& s = ctx->slots[slot];
+  const Geom& g = ctx->g;
+  CU(ctx, cudaSetDevice(ctx->cfg.device));
+  if (int rc = original_begin(ctx, s)) return rc;
   const int16_t* srcs[3] = {y, cb, cr};
   const ptrdiff_t strides[3] = {sy, scb, scr};
   for (int p = 0; p < 3; p++) {
@@ -1306,16 +1384,13 @@ static int set_original_rows(ilf_ctx* ctx, int slot, const int16_t* y, ptrdiff_t
     CU(ctx, cudaMemcpy2DAsync(const_cast<int16_t*>(s.dev.org[p]) + (size_t)pr.r0 * pr.pitch, (size_t)pr.pitch * 2, srcs[p], (size_t)strides[p] * 2, (size_t)pr.w * 2, pr.h,
                               cudaMemcpyHostToDevice, ctx->s_up));
   }
-  CU(ctx, cudaMemcpyAsync(s.stats_avail, ctu_avail, ctx->num_ctus, cudaMemcpyHostToDevice, ctx->s_up));
-  if (!is_pinned(ctu_avail)) CU(ctx, cudaStreamSynchronize(ctx->s_up));  // the caller may reuse ctu_avail
-  s.has_org = true;
-  s.org_since_upload = true;
-  return push_desc(ctx, slot);
+  if (int rc = original_avail(ctx, s, ctu_avail)) return rc;
+  return original_end(ctx, slot);
 }
 
 int ilf_set_original(ilf_ctx* ctx, int slot, const int16_t* y, ptrdiff_t sy, const int16_t* cb, ptrdiff_t scb, const int16_t* cr, ptrdiff_t scr, const uint8_t* ctu_avail) {
   if (int rc = check_slot(ctx, slot)) return rc;
-  if (ctx->is_band) return fail(ctx, ILF_ERR_STATE, "SAO statistics are not available on band contexts");
+  if (int rc = check_original(ctx, slot, false)) return rc;
   return set_original_rows(ctx, slot, y, sy, cb, scb, cr, scr, ctu_avail, 0, ctx->g.height);
 }
 
@@ -1323,9 +1398,136 @@ int ilf_set_original(ilf_ctx* ctx, int slot, const int16_t* y, ptrdiff_t sy, con
 int ilf_set_original_band(ilf_ctx* ctx, int slot, const int16_t* y, ptrdiff_t sy, const int16_t* cb, ptrdiff_t scb, const int16_t* cr, ptrdiff_t scr,
                           const uint8_t* ctu_avail) {
   if (int rc = check_slot(ctx, slot)) return rc;
-  if (!ctx->is_band) return fail(ctx, ILF_ERR_STATE, "not a band context (ilf_set_original takes the whole picture)");
-  if (!ctx->slots[slot].uploaded) return fail(ctx, ILF_ERR_STATE, "slot %d: ilf_set_original_band before the slot's upload", slot);
+  if (int rc = check_original(ctx, slot, true)) return rc;
   return set_original_rows(ctx, slot, y, sy, cb, scb, cr, scr, ctu_avail, ctx->g.out_row0 - ctx->g.row0, ctx->g.out_rows);
+}
+
+// ---------------------------------------------------------------------------------------------------------------
+// Pictures in device memory (include/ilf_b200.h): one conversion kernel per call (ilf_io.cu) on the upload or download stream,
+// bridged to the caller's stream with an event in each direction; the slot's state changes are those of the host calls.
+// ---------------------------------------------------------------------------------------------------------------
+// The caller's planes and format, validated before anything is enqueued: `depth` receives the caller's luma / chroma depths,
+// `bytes` its sample size.
+struct DevicePlanes { const void* p[3]; ptrdiff_t stride[3]; int depth[2], bytes; };
+static int check_device_planes(ilf_ctx* ctx, DevicePlanes& d, const ilf_samples* fmt) {
+  const Geom& g = ctx->g;
+  const ilf_samples dflt = {ILF_SAMPLES_I16, {0, 0}};
+  if (!fmt) fmt = &dflt;
+  if (fmt->type != ILF_SAMPLES_I16 && fmt->type != ILF_SAMPLES_U8) return fail(ctx, ILF_ERR_ARG, "unknown sample type %d", (int)fmt->type);
+  const bool i16 = fmt->type == ILF_SAMPLES_I16;
+  for (int c = 0; c < 2; c++) {
+    const int v = fmt->bit_depth[c];
+    if (i16 ? (v != 0 && (v < 8 || v > 16)) : (v != 0 && v != 8))
+      return fail(ctx, ILF_ERR_ARG, "%s depth %d outside %s", c ? "chroma" : "luma", v, i16 ? "8..16 (0: the context's)" : "8 (uint8 samples)");
+    d.depth[c] = v ? v : (i16 ? (c ? g.bd_chroma : g.bd_luma) : 8);
+  }
+  d.bytes = i16 ? 2 : 1;
+  for (int p = 0; p < 3; p++) {
+    if (!d.p[p]) return fail(ctx, ILF_ERR_ARG, "null plane pointer");
+    int dev = -1;
+    const cudaMemoryType t = mem_type(d.p[p], &dev);
+    if (t != cudaMemoryTypeDevice || dev != ctx->cfg.device)
+      return fail(ctx, ILF_ERR_ARG, "plane %d is %s, not device memory of the context's device %d", p,
+                  t == cudaMemoryTypeDevice ? "memory of another device" : (t == cudaMemoryTypeManaged ? "managed memory" : "host memory"), ctx->cfg.device);
+    if (i16 && ((uintptr_t)d.p[p] & 1)) return fail(ctx, ILF_ERR_ARG, "int16 plane %d is not 2-byte aligned", p);
+    const int w = p ? g.width / 2 : g.width;
+    if (d.stride[p] < w) return fail(ctx, ILF_ERR_ARG, "plane %d: stride %lld shorter than the plane's width %d", p, (long long)d.stride[p], w);
+  }
+  return ILF_OK;
+}
+
+// The copy between the caller's planes and the context's planes `mine` (held-row layout, first row = LOCAL row 0) over the rows a device
+// transfer covers: to_ctx = caller -> context (upload, original), else context -> caller (download).
+static IoBatch device_batch(const ilf_ctx* ctx, const DevicePlanes& d, int16_t* const mine[3], bool to_ctx) {
+  const Geom& g = ctx->g;
+  const int first = g.out_row0 - g.row0, n = g.out_rows;   // a whole picture, or a band's own rows
+  IoBatch b;
+  for (int p = 0; p < 3; p++) {
+    const PlaneRows pr = plane_rows(g, p, first, n);
+    const int c = p ? 1 : 0, ctx_depth = c ? g.bd_chroma : g.bd_luma;
+    const int diff = to_ctx ? ctx_depth - d.depth[c] : d.depth[c] - ctx_depth;
+    int16_t* rows = mine[p] + (size_t)pr.r0 * pr.pitch;
+    const long long caller_pitch = (long long)d.stride[p] * d.bytes, ctx_pitch = (long long)pr.pitch * 2;
+    IoPlane& io = b.p[p];
+    io.src = to_ctx ? d.p[p] : rows;
+    io.dst = to_ctx ? (void*)rows : const_cast<void*>(d.p[p]);
+    io.src_pitch = to_ctx ? caller_pitch : ctx_pitch;
+    io.dst_pitch = to_ctx ? ctx_pitch : caller_pitch;
+    io.w = pr.w; io.h = pr.h;
+    io.up = std::max(diff, 0); io.down = std::max(-diff, 0);
+    io.maxv = (1 << (to_ctx ? ctx_depth : d.depth[c])) - 1;
+  }
+  b.src_bytes = to_ctx ? d.bytes : 2;
+  b.dst_bytes = to_ctx ? 2 : d.bytes;
+  return b;
+}
+
+// Records the caller's stream up to this call.  First thing enqueued: a stream the context cannot wait for (another device's) fails
+// before anything of the transfer is issued.
+static int caller_mark(ilf_ctx* ctx, void* stream) {
+  CU(ctx, cudaEventRecord(ctx->ev_caller, (cudaStream_t)stream));
+  return ILF_OK;
+}
+
+int ilf_upload_device(ilf_ctx* ctx, int slot, const void* y, ptrdiff_t sy, const void* cb, ptrdiff_t scb, const void* cr, ptrdiff_t scr,
+                      const ilf_samples* fmt, void* stream) {
+  if (int rc = check_slot(ctx, slot)) return rc;
+  DevicePlanes d = {{y, cb, cr}, {sy, scb, scr}};
+  CU(ctx, cudaSetDevice(ctx->cfg.device));
+  if (int rc = check_device_planes(ctx, d, fmt)) return rc;
+  Slot& s = ctx->slots[slot];
+  int16_t* const mine[3] = {plane_ptr(ctx, s, 0, 0), plane_ptr(ctx, s, 0, 1), plane_ptr(ctx, s, 0, 2)};
+  const IoBatch b = device_batch(ctx, d, mine, true);
+  if (int rc = caller_mark(ctx, stream)) return rc;
+  CU(ctx, cudaStreamWaitEvent(ctx->s_up, ctx->ev_caller, 0));
+  if (int rc = upload_begin(ctx, s)) return rc;
+  if (int rc = launch(ctx, -1, 0, 1, [&] { launch_io_convert(b, ctx->s_up); })) return rc;
+  if (int rc = upload_end(ctx, s)) return rc;
+  CU(ctx, cudaStreamWaitEvent((cudaStream_t)stream, s.ev_up, 0));
+  return ILF_OK;
+}
+
+int ilf_set_original_device(ilf_ctx* ctx, int slot, const void* y, ptrdiff_t sy, const void* cb, ptrdiff_t scb, const void* cr, ptrdiff_t scr,
+                            const uint8_t* ctu_avail, const ilf_samples* fmt, void* stream) {
+  if (int rc = check_slot(ctx, slot)) return rc;
+  if (!ctu_avail) return fail(ctx, ILF_ERR_ARG, "null pointer");
+  if (mem_type(ctu_avail) == cudaMemoryTypeDevice) return fail(ctx, ILF_ERR_ARG, "ctu_avail is device memory: it is read from the host");
+  DevicePlanes d = {{y, cb, cr}, {sy, scb, scr}};
+  CU(ctx, cudaSetDevice(ctx->cfg.device));
+  if (int rc = check_device_planes(ctx, d, fmt)) return rc;
+  if (int rc = check_original(ctx, slot, ctx->is_band)) return rc;   // ilf_set_original, or ilf_set_original_band on a band context
+  Slot& s = ctx->slots[slot];
+  if (int rc = caller_mark(ctx, stream)) return rc;
+  if (int rc = original_begin(ctx, s)) return rc;
+  // ctu_avail is not ordered after the caller's stream: a pageable array is copied, and waited for, without waiting for the caller's work
+  if (int rc = original_avail(ctx, s, ctu_avail)) return rc;
+  int16_t* const org[3] = {const_cast<int16_t*>(s.dev.org[0]), const_cast<int16_t*>(s.dev.org[1]), const_cast<int16_t*>(s.dev.org[2])};
+  const IoBatch b = device_batch(ctx, d, org, true);
+  CU(ctx, cudaStreamWaitEvent(ctx->s_up, ctx->ev_caller, 0));
+  if (int rc = launch(ctx, -1, 0, 1, [&] { launch_io_convert(b, ctx->s_up); })) return rc;
+  if (int rc = original_end(ctx, slot)) return rc;
+  CU(ctx, cudaStreamWaitEvent((cudaStream_t)stream, s.ev_up, 0));
+  return ILF_OK;
+}
+
+int ilf_download_device(ilf_ctx* ctx, int slot, void* y, ptrdiff_t sy, void* cb, ptrdiff_t scb, void* cr, ptrdiff_t scr, const ilf_samples* fmt,
+                        void* stream) {
+  if (int rc = check_slot(ctx, slot)) return rc;
+  DevicePlanes d = {{y, cb, cr}, {sy, scb, scr}};
+  CU(ctx, cudaSetDevice(ctx->cfg.device));
+  if (int rc = check_device_planes(ctx, d, fmt)) return rc;
+  Slot& s = ctx->slots[slot];
+  if (!s.uploaded) return fail(ctx, ILF_ERR_STATE, "slot %d: download before upload", slot);
+  // each plane from the buffer its last stage left it in
+  int16_t* const cur[3] = {plane_ptr(ctx, s, s.result_buf[0], 0), plane_ptr(ctx, s, s.result_buf[1], 1), plane_ptr(ctx, s, s.result_buf[2], 2)};
+  const IoBatch b = device_batch(ctx, d, cur, false);
+  if (int rc = caller_mark(ctx, stream)) return rc;
+  CU(ctx, cudaStreamWaitEvent(ctx->s_down, ctx->ev_caller, 0));
+  if (int rc = download_begin(ctx, s)) return rc;
+  if (int rc = launch(ctx, -1, 0, 1, [&] { launch_io_convert(b, ctx->s_down); })) return rc;
+  if (int rc = download_end(ctx, s)) return rc;
+  CU(ctx, cudaStreamWaitEvent((cudaStream_t)stream, s.ev_down, 0));
+  return ILF_OK;
 }
 
 // CTUs whose statistics records a slot produces: the picture's, or a band's own (num_ctu_rows x ctus_w).

@@ -171,4 +171,10 @@ cudaError_t hash_rows(const Geom& g, const int16_t* const planes[3], uint32_t* s
 void launch_alf_stats(const Geom& g, const SlotDev* slots, int first_slot, int num_slots, const BatchCtl& ctl, cudaStream_t st);
 void launch_alf_classify(const Geom& g, const SlotDev* slots, int first_slot, int num_slots, const BatchCtl& ctl, cudaStream_t st);
 
+// Pictures in the caller's device memory (ilf_io.cu): plane p of `src` -> plane p of `dst`, w x h samples, pitches in BYTES, with
+// the depth conversion of ilf_upload_device / ilf_download_device (up: left shift; down > 0: round, shift right, clip to maxv).
+struct IoPlane { const void* src; void* dst; long long src_pitch, dst_pitch; int w, h, up, down, maxv; };
+struct IoBatch { IoPlane p[3]; int src_bytes, dst_bytes; };   // sample sizes: 2 (int16) or 1 (uint8)
+void launch_io_convert(const IoBatch& b, cudaStream_t st);
+
 }  // namespace ilf

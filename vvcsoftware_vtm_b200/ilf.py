@@ -1,7 +1,8 @@
 """ctypes binding of libilf_b200.so (include/ilf_b200.h).
 
 No fallback of any kind: if the CUDA library is missing or no GPU is present the calls raise.  numpy arrays
-in, numpy arrays out; device memory stays inside the library.  Method names follow the reference entry points:
+in, numpy arrays out; pictures that are already on the GPU go in and out as torch CUDA tensors (upload_device,
+set_original_device, download_device), on the caller's current torch stream.  Method names follow the reference entry points:
 ``loop_filter_pic`` = LoopFilter::loopFilterPic, ``sao_process`` = SampleAdaptiveOffset::SAOProcess,
 ``alf_process`` = AdaptiveLoopFilter::ALFProcess (DecLib.cpp:516-530).
 """
@@ -28,6 +29,14 @@ class IlfConfig(C.Structure):
 
 class IlfBand(C.Structure):
     _fields_ = [("first_ctu_row", C.c_int32), ("num_ctu_rows", C.c_int32)]
+
+
+class IlfSamples(C.Structure):
+    """ilf_samples: sample type and the caller's (luma, chroma) bit depths of a device transfer."""
+    _fields_ = [("type", C.c_int32), ("bit_depth", C.c_int32 * 2)]
+
+
+SAMPLES_I16, SAMPLES_U8 = 0, 1   # ILF_SAMPLES_*
 
 
 class IlfHashPart(C.Structure):
@@ -76,6 +85,9 @@ def load_library():
     lib.ilf_sync.argtypes = [vp]
     lib.ilf_download_async.argtypes = [vp, i, vp, pd, vp, pd, vp, pd]
     lib.ilf_wait.argtypes = [vp, i]
+    lib.ilf_upload_device.argtypes = [vp, i, vp, pd, vp, pd, vp, pd, C.POINTER(IlfSamples), vp]
+    lib.ilf_download_device.argtypes = [vp, i, vp, pd, vp, pd, vp, pd, C.POINTER(IlfSamples), vp]
+    lib.ilf_set_original_device.argtypes = [vp, i, vp, pd, vp, pd, vp, pd, vp, C.POINTER(IlfSamples), vp]
     lib.ilf_host_alloc.argtypes = [C.c_size_t]
     lib.ilf_host_alloc.restype = vp
     lib.ilf_host_free.argtypes = [vp]
@@ -230,6 +242,61 @@ class InLoopFilter:
 
     def sync(self):
         self._ck(self._lib.ilf_sync(self._h))
+
+    # ---- pictures in device memory (torch CUDA tensors) -----------------------------------------------
+    # Planes are 2-D CUDA tensors on the context's device with stride(-1) == 1, all int16 or all uint8 (which selects the sample
+    # type), of the shapes of the rows the context produces (own_rows x width, chroma halved): the whole picture, or a band's own
+    # rows.  bit_depth = the caller's depth: None (int16: the context's; uint8: 8), one int, or a (luma, chroma) pair.  Every call is
+    # ordered on torch.cuda.current_stream of the context's device and returns without waiting.
+    def _device_planes(self, planes, bit_depth):
+        import torch
+        shapes = ((self.own_rows, self.width), (self.own_rows // 2, self.width // 2), (self.own_rows // 2, self.width // 2))
+        dtype = planes[0].dtype if isinstance(planes[0], torch.Tensor) else None
+        if dtype not in (torch.int16, torch.uint8):
+            raise IlfError("device planes are torch.int16 or torch.uint8 CUDA tensors")
+        args = []
+        for name, t, shape in zip(("y", "cb", "cr"), planes, shapes):
+            if not isinstance(t, torch.Tensor) or not t.is_cuda or t.dtype != dtype:
+                raise IlfError(f"plane {name}: a CUDA tensor of dtype {dtype} is expected")
+            if t.dim() != 2 or tuple(t.shape) != shape or t.stride(-1) != 1:
+                raise IlfError(f"plane {name}: shape {tuple(t.shape)} strides {t.stride()}, expected shape {shape} with stride(-1) == 1")
+            args += [C.c_void_p(t.data_ptr()), t.stride(0)]
+        if bit_depth is None:
+            bd = (0, 0)
+        elif isinstance(bit_depth, int):
+            bd = (bit_depth, bit_depth)
+        else:
+            bd = tuple(bit_depth)
+        fmt = IlfSamples(SAMPLES_I16 if dtype == torch.int16 else SAMPLES_U8, (C.c_int32 * 2)(*bd))
+        stream = torch.cuda.current_stream(torch.device("cuda", self.cfg.device)).cuda_stream
+        return args, fmt, C.c_void_p(stream)
+
+    def upload_device(self, slot, y, cb, cr, bit_depth=None):
+        """ilf_upload_device: the picture (a band: its own rows) from CUDA tensors; side information must be set again after it."""
+        args, fmt, stream = self._device_planes((y, cb, cr), bit_depth)
+        self._ck(self._lib.ilf_upload_device(self._h, slot, *args, C.byref(fmt), stream))
+
+    def set_original_device(self, slot, y, cb, cr, ctu_avail, bit_depth=None):
+        """ilf_set_original_device: the encoder's source picture (a band: its own rows) from CUDA tensors, e.g. 8-bit frames
+        (uint8) for a 10-bit context; ctu_avail (host, every CTU of the picture) as in set_original."""
+        args, fmt, stream = self._device_planes((y, cb, cr), bit_depth)
+        av = _arr(ctu_avail, np.uint8)
+        assert av.size == self.ctus_w * self.ctus_h
+        self._ck(self._lib.ilf_set_original_device(self._h, slot, *args, _ptr(av), C.byref(fmt), stream))
+
+    def download_device(self, slot, dtype=None, bit_depth=None, out=None):
+        """ilf_download_device: the slot's current picture (a band: its own rows) as {"y","cb","cr"} CUDA tensors of `dtype`
+        (torch.int16, the default, or torch.uint8); `out` = such a dict to fill instead."""
+        import torch
+        if out is None:
+            dev = torch.device("cuda", self.cfg.device)
+            dt = torch.int16 if dtype is None else dtype
+            out = {"y": torch.empty((self.own_rows, self.width), dtype=dt, device=dev)}
+            out["cb"] = torch.empty((self.own_rows // 2, self.width // 2), dtype=dt, device=dev)
+            out["cr"] = torch.empty_like(out["cb"])
+        args, fmt, stream = self._device_planes((out["y"], out["cb"], out["cr"]), bit_depth)
+        self._ck(self._lib.ilf_download_device(self._h, slot, *args, C.byref(fmt), stream))
+        return out
 
     # ---- CTU-row band mode (one picture across several GPUs) ---------------------------------------
     def upload_band(self, slot, y, cb, cr):
