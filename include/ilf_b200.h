@@ -263,7 +263,8 @@ int ilf_set_alf_params(ilf_ctx* ctx, int slot, const ilf_alf_params* params,
  * whose side information was not set since the last upload is an error.  The result of a slot is
  * what ilf_download returns; the uploaded input is preserved, so ilf_run can be repeated.
  * Every requested stage of every slot is validated before anything is launched.  The slots of a batch may mix the motion-vector
- * representations (none / mv16 / mv32): the deblocking stage then takes one launch per representation present.
+ * representations (none / mv16 / mv32) and grids with or without a chroma-tree layer: the deblocking stage reads the edge
+ * records ilf_set_deblock_info derived and is still one launch (ilf_deblock_search takes one launch per representation present).
  * ilf_deblock / ilf_sao / ilf_alf are the per-class entry points of the shim (one stage, one slot;
  * each consumes the previous stage's output).
  * ------------------------------------------------------------------------------------------- */
@@ -359,7 +360,9 @@ int ilf_download_extended(ilf_ctx* ctx, int slot, int16_t* y, ptrdiff_t stride_y
  * Measurement helpers (bench.py).  Accumulated device time per kernel in milliseconds since
  * ilf_set_timing(ctx, 1) (CUDA event pairs around every launch on the context's stream, collected
  * without synchronising inside ilf_run), number of kernel launches issued since ilf_create (the
- * conversion kernel of the device transfers included; it has no timing slot), and raw device
+ * conversion kernel of the device transfers included; it has no timing slot; the edge-record pass
+ * of ilf_set_deblock_info is not counted: the count since ilf_create stays the number of transfer
+ * and filter launches, which callers and tests compare against the stages they ran), and raw device
  * pointers of a slot's input planes so that synthetic pictures can be generated on the device.
  * planes[0..2] = Y, Cb, Cr; pitch in samples.  These pointers carry no ordering: a caller's
  * picture enters and leaves through the device transfers above.

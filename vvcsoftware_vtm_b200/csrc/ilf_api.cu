@@ -87,6 +87,7 @@ struct Slot {
   uint32_t* info = nullptr;
   uint32_t* info_c = nullptr;
   void* mv = nullptr;          // int16x4 or int32x4 per unit
+  void* db_rec = nullptr;      // deblocking edge records (db_rec_layout), derived by ilf_set_deblock_info
   uint8_t* ctu_slice = nullptr;
   ilf_deblock_params* db_params = nullptr;
   ilf_sao_ctu* sao = nullptr;
@@ -118,6 +119,8 @@ struct Slot {
   bool alf_is7 = false;            // luma filter shape of the slot's ALF parameters
   // ordering of the slot's copies and kernels (see "Per-slot ordering" above join())
   cudaEvent_t ev_up = nullptr, ev_run = nullptr, ev_down = nullptr;
+  cudaEvent_t ev_rec = nullptr;    // the slot's last deblocking record pass is done; rec_pending: issued since a stream last waited for it
+  bool rec_pending = false;
   cudaStream_t run_stream = nullptr;
   cudaEvent_t ev_side[3] = {nullptr, nullptr, nullptr};
   size_t side_off[4] = {0, 0, 0, 0};                       // regions of pinned_side per stage
@@ -136,6 +139,7 @@ struct ilf_ctx {
   cudaStream_t stream = nullptr;   // compute stream (kernels)
   cudaStream_t s_up = nullptr;     // host -> device copies
   cudaStream_t s_down = nullptr;   // device -> host copies
+  cudaStream_t s_rec = nullptr;    // deblocking record passes (ilf_set_deblock_info): off the upload stream, so copies queued behind one do not wait for it
   // Lanes: a chain over a large batch is dealt to `num_lanes` extra compute streams (ilf_run), so that the drain of one lane's
   // kernel overlaps another lane's kernels; the compute stream joins them (waits for their run events) without holding them up.
   static constexpr int MAX_LANES = 4;
@@ -210,6 +214,8 @@ int check_range(ilf_ctx* ctx, int first, int n) {
 //                kernel reads (uploads, side information, originals, halo rows) and downloads wait for it.
 //   ev_down      the last D2H copy of the slot is done (uploads wait for it); d2h_pending: a download was issued since ilf_run last
 //                waited for ev_down.
+//   ev_rec       the slot's last deblocking record pass (ilf_set_deblock_info, on s_rec after the side-information copies it reads) is
+//                done; kernels and the next setter call wait for it while rec_pending.
 // A batched entry point validates every slot before it issues anything, then joins each slot to the stream it launches on,
 // launches, and fences.
 
@@ -220,6 +226,7 @@ int check_range(ilf_ctx* ctx, int first, int n) {
 // buffers that a download may still read.
 int join(ilf_ctx* ctx, Slot& s, cudaStream_t st, bool overwrites_buffers) {
   if (s.h2d_pending) { CU(ctx, cudaStreamWaitEvent(st, s.ev_up, 0)); s.h2d_pending = false; }
+  if (s.rec_pending) { CU(ctx, cudaStreamWaitEvent(st, s.ev_rec, 0)); s.rec_pending = false; }
   if (overwrites_buffers && s.d2h_pending) { CU(ctx, cudaStreamWaitEvent(st, s.ev_down, 0)); s.d2h_pending = false; }
   if (s.run_stream && s.run_stream != st) CU(ctx, cudaStreamWaitEvent(st, s.ev_run, 0));
   return ILF_OK;
@@ -240,7 +247,7 @@ unsigned buf_word(const Slot& s) { return s.result_buf[0] | s.result_buf[1] << 2
 
 // Compact launch list of the chunk of slots [c0, c0 + cn): grid layer m works on slot c0 + ctl.slot[m] under control word ctl.v[m].
 // word(i) gives the control word of slot c0 + i, or < 0 to leave it out; mv_mode >= 0 keeps the slots of that motion-vector
-// representation only (none / int16 / int32 are different deblocking kernels).
+// representation only (none / int16 / int32 are different deblocking search kernels).
 template <typename Word>
 int compact(const ilf_ctx* ctx, int c0, int cn, int mv_mode, BatchCtl& ctl, Word word) {
   int m = 0;
@@ -385,6 +392,7 @@ int side_begin(ilf_ctx* ctx, Slot& s, int k, size_t& cursor) {
   CU(ctx, cudaSetDevice(ctx->cfg.device));
   CU(ctx, cudaEventSynchronize(s.ev_side[k]));  // the previous copy out of this staging region is done
   CU(ctx, cudaStreamWaitEvent(ctx->s_up, s.ev_run, 0));  // kernels of the slot's previous picture may still read the device arrays
+  if (s.rec_pending) CU(ctx, cudaStreamWaitEvent(ctx->s_up, s.ev_rec, 0));  // ... and so may its record pass (the grids, motion, slice map)
   cursor = s.side_off[k];
   return ILF_OK;
 }
@@ -486,6 +494,7 @@ int create_impl(ilf_ctx** out, const ilf_config* cfg, const ilf_band* band) {
   CU(ctx, cudaStreamCreateWithFlags(&ctx->stream, cudaStreamNonBlocking));
   CU(ctx, cudaStreamCreateWithFlags(&ctx->s_up, cudaStreamNonBlocking));
   CU(ctx, cudaStreamCreateWithFlags(&ctx->s_down, cudaStreamNonBlocking));
+  CU(ctx, cudaStreamCreateWithFlags(&ctx->s_rec, cudaStreamNonBlocking));
   ctx->num_lanes = std::max(1, std::min((int)ilf_ctx::MAX_LANES, env_int("ILF_RUN_LANES", 2)));
   ctx->lane_min_slots = std::max(2, env_int("ILF_RUN_LANE_MIN", 8));
   if (ctx->num_lanes > 1)
@@ -497,6 +506,7 @@ int create_impl(ilf_ctx** out, const ilf_config* cfg, const ilf_band* band) {
   ctx->slots.resize(cfg->num_slots);
   CU(ctx, cudaMalloc(&ctx->slots_dev, sizeof(SlotDev) * cfg->num_slots));
   const size_t units = (size_t)g.units_pitch * g.units_h;  // device grids are pitched
+  const DbRecLayout rec = db_rec_layout(g);
   for (int i = 0; i < cfg->num_slots; i++) {
     Slot& s = ctx->slots[i];
     CU(ctx, cudaMalloc(&s.planes, 3 * ctx->buf_elems * sizeof(int16_t)));
@@ -507,6 +517,8 @@ int create_impl(ilf_ctx** out, const ilf_config* cfg, const ilf_band* band) {
     CU(ctx, cudaMemsetAsync(s.info, 0, units * 4, ctx->s_up));
     CU(ctx, cudaMemsetAsync(s.info_c, 0, units * 4, ctx->s_up));
     CU(ctx, cudaMemsetAsync(s.mv, 0, units * 16, ctx->s_up));
+    CU(ctx, cudaMalloc(&s.db_rec, rec.bytes));
+    CU(ctx, cudaMemsetAsync(s.db_rec, 0, rec.bytes, ctx->s_up));
     CU(ctx, cudaMalloc(&s.ctu_slice, ctx->num_ctus));
     CU(ctx, cudaMalloc(&s.db_params, sizeof(ilf_deblock_params)));
     CU(ctx, cudaMalloc(&s.sao, sizeof(ilf_sao_ctu) * ctx->num_ctus));
@@ -525,6 +537,7 @@ int create_impl(ilf_ctx** out, const ilf_config* cfg, const ilf_band* band) {
     CU(ctx, cudaEventCreateWithFlags(&s.ev_up, cudaEventDisableTiming));
     s.ev_run = ctx->run_ring[0][0];  // never recorded yet: waiting on it is a no-op
     CU(ctx, cudaEventCreateWithFlags(&s.ev_down, cudaEventDisableTiming));
+    CU(ctx, cudaEventCreateWithFlags(&s.ev_rec, cudaEventDisableTiming));
     for (int k = 0; k < 3; k++) CU(ctx, cudaEventCreateWithFlags(&s.ev_side[k], cudaEventDisableTiming));
     memset(&s.dev, 0, sizeof(s.dev));
     for (int b = 0; b < 3; b++)
@@ -536,6 +549,11 @@ int create_impl(ilf_ctx** out, const ilf_config* cfg, const ilf_band* band) {
       if (int rc = make_map3(ctx, &s.dev.tm_info_c, CU_TENSOR_MAP_DATA_TYPE_UINT32, s.info_c, g.units_w, g.units_h, 1, (size_t)g.units_pitch * 4, grid_bytes, DB_BOX_UNITS, 8)) return rc;
       if (int rc = make_map3(ctx, &s.dev.tm_mv16, CU_TENSOR_MAP_DATA_TYPE_UINT32, s.mv, g.units_w * 2, g.units_h, 1, (size_t)g.units_pitch * 8, units * 8, DB_BOX_MV16_WORDS, 8)) return rc;
       if (int rc = make_map3(ctx, &s.dev.tm_mv32, CU_TENSOR_MAP_DATA_TYPE_UINT32, s.mv, g.units_w * 4, g.units_h, 1, (size_t)g.units_pitch * 16, units * 16, DB_BOX_MV32_WORDS, 8)) return rc;
+      const int box_w[DB_REC_KINDS] = {DB_REC_LV_W, DB_REC_LH_W, DB_REC_CV_W, DB_REC_CH_W}, box_h[DB_REC_KINDS] = {DB_REC_LV_H, DB_REC_LH_H, DB_REC_CV_H, DB_REC_CH_H};
+      for (int k = 0; k < DB_REC_KINDS; k++)
+        if (int rc = make_map3(ctx, &s.dev.tm_rec[k], rec.elem[k] == 2 ? CU_TENSOR_MAP_DATA_TYPE_UINT16 : CU_TENSOR_MAP_DATA_TYPE_UINT32, static_cast<char*>(s.db_rec) + rec.off[k],
+                               rec.cols[k], rec.rows[k], 1, (size_t)rec.pitch[k] * rec.elem[k], (size_t)rec.pitch[k] * rec.elem[k] * rec.rows[k], box_w[k], box_h[k]))
+          return rc;
     }
     for (int p = 0; p < 3; p++) {
       const PlaneRows pr = plane_rows(g, p, 0, g.rows);
@@ -558,6 +576,7 @@ int create_impl(ilf_ctx** out, const ilf_config* cfg, const ilf_band* band) {
 
 int sync_all(ilf_ctx* ctx) {
   CU(ctx, cudaStreamSynchronize(ctx->s_up));
+  CU(ctx, cudaStreamSynchronize(ctx->s_rec));
   CU(ctx, cudaStreamSynchronize(ctx->stream));
   CU(ctx, cudaStreamSynchronize(ctx->s_down));
   return ILF_OK;
@@ -585,17 +604,17 @@ int ilf_create_band(ilf_ctx** out, const ilf_config* cfg, const ilf_band* band) 
 int ilf_destroy(ilf_ctx* ctx) {
   if (!ctx) return ILF_OK;
   cudaSetDevice(ctx->cfg.device);
-  const auto streams = {ctx->s_up, ctx->stream, ctx->s_down, ctx->lane[0], ctx->lane[1], ctx->lane[2], ctx->lane[3]};
+  const auto streams = {ctx->s_up, ctx->s_rec, ctx->stream, ctx->s_down, ctx->lane[0], ctx->lane[1], ctx->lane[2], ctx->lane[3]};
   for (cudaStream_t st : streams) if (st) cudaStreamSynchronize(st);
   for (Slot& s : ctx->slots) {
     for (auto& nb : s.nb) if (nb.ipc_base) cudaIpcCloseMemHandle(nb.ipc_base);
-    cudaFree(s.planes); cudaFree(s.info); cudaFree(s.info_c); cudaFree(s.mv); cudaFree(s.ctu_slice); cudaFree(s.db_params);
+    cudaFree(s.planes); cudaFree(s.info); cudaFree(s.info_c); cudaFree(s.mv); cudaFree(s.db_rec); cudaFree(s.ctu_slice); cudaFree(s.db_params);
     cudaFree(s.sao); cudaFree(s.alf); cudaFree(s.alf_coef); cudaFree(s.alf_coef_dp); cudaFree(s.alf_ctu_enable); cudaFree(s.alf_class);
     cudaFree(s.org); cudaFree(s.stats_avail); cudaFree(s.stats); cudaFree(s.alf_stats);
     if (s.pinned) cudaFreeHost(s.pinned);
     if (s.pinned_down) cudaFreeHost(s.pinned_down);
     if (s.pinned_side) cudaFreeHost(s.pinned_side);
-    for (cudaEvent_t e : {s.ev_up, s.ev_down, s.ev_side[0], s.ev_side[1], s.ev_side[2]}) if (e) cudaEventDestroy(e);
+    for (cudaEvent_t e : {s.ev_up, s.ev_down, s.ev_rec, s.ev_side[0], s.ev_side[1], s.ev_side[2]}) if (e) cudaEventDestroy(e);
   }
   for (auto& ring : ctx->run_ring)
     for (cudaEvent_t e : ring) if (e) cudaEventDestroy(e);
@@ -1105,6 +1124,14 @@ int ilf_set_deblock_info(ilf_ctx* ctx, int slot, const ilf_deblock_params* param
   s.dev.mv32 = mv32 ? (const int32_t*)s.mv : nullptr;
   s.dev.ctu_slice = ctu_slice ? s.ctu_slice : nullptr;
   s.dev.db_params = s.db_params;
+  // The edge records the deblocking kernel reads, derived on s_rec behind the copies just issued (while those arrays are in L2) and
+  // behind the slot's previous kernels (side_begin ordered s_up after them); later kernels of the slot wait for ev_rec (join).
+  CU(ctx, cudaEventRecord(s.ev_side[0], ctx->s_up));
+  CU(ctx, cudaStreamWaitEvent(ctx->s_rec, s.ev_side[0], 0));
+  launch_deblock_records(ctx->g, s.db_params, s.info, s.dev.info_c, s.dev.mv16, s.dev.mv32, params->num_slices > 1 ? s.dev.ctu_slice : nullptr, s.db_rec, ctx->s_rec);
+  CU(ctx, cudaGetLastError());
+  CU(ctx, cudaEventRecord(s.ev_rec, ctx->s_rec));
+  s.rec_pending = true;
   // A chroma edge is filtered only when a side is intra (bS == 2, LoopFilter.cpp:769): without an intra unit in the layer the
   // chroma decisions read, deblocking leaves both chroma planes as uploaded, and run_stage skips them.
   s.db_chroma = any_intra(info_chroma ? info_chroma : info, (size_t)ctx->g.units_w * ctx->g.units_h);
@@ -1216,23 +1243,22 @@ static int run_stage(ilf_ctx* ctx, int first, int n, int stage, cudaStream_t st,
                        ((s.dev.alf_mode & 2) ? CTL_ALF_DOT_C : 0) | ((s.dev.alf_mode & 8) ? CTL_ALF_HIC_C : 0);
       word[i] = any ? (int)v : -1;
     }
-    // one launch of `kernel_launch` over the active slots (of motion-vector representation mv_mode when >= 0)
-    auto stage_launch = [&](int mv_mode, auto kernel_launch) -> int {
+    // one launch of `kernel_launch` over the active slots
+    auto stage_launch = [&](auto kernel_launch) -> int {
       BatchCtl ctl;
-      const int m = compact(ctx, c0, cn, mv_mode, ctl, [&](int i) { return word[i]; });
+      const int m = compact(ctx, c0, cn, -1, ctl, [&](int i) { return word[i]; });
       if (!m) return ILF_OK;
       double bytes = 0;
       for (int j = 0; j < m; j++) bytes += bytes_of[ctl.slot[j]];
       return launch(ctx, stage, bytes, 1, [&] { kernel_launch(ctl, m); });
     };
     if (stage == 0) {
-      for (int mode = 0; mode < 3; mode++)
-        if (int rc = stage_launch(mode, [&](const BatchCtl& ctl, int m) { launch_deblock(g, ctx->slots_dev, c0, m, ctl, mode, ctx->db_work + 2 * ring, st); })) return rc;
+      if (int rc = stage_launch([&](const BatchCtl& ctl, int m) { launch_deblock(g, ctx->slots_dev, c0, m, ctl, ctx->db_work + 2 * ring, st); })) return rc;
     } else if (stage == 1) {
-      if (int rc = stage_launch(-1, [&](const BatchCtl& ctl, int m) { launch_sao(g, ctx->slots_dev, c0, m, ctl, st); })) return rc;
+      if (int rc = stage_launch([&](const BatchCtl& ctl, int m) { launch_sao(g, ctx->slots_dev, c0, m, ctl, st); })) return rc;
     } else {
       // luma and chroma bands are CTAs of one launch (they share the SMs), accounted under ILF_KERNEL_ALF_LUMA
-      if (int rc = stage_launch(-1, [&](const BatchCtl& ctl, int m) { launch_alf(g, ctx->slots_dev, c0, m, ctl, st); })) return rc;
+      if (int rc = stage_launch([&](const BatchCtl& ctl, int m) { launch_alf(g, ctx->slots_dev, c0, m, ctl, st); })) return rc;
     }
   }
   return ILF_OK;

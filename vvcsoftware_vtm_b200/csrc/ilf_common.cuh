@@ -48,6 +48,39 @@ constexpr int DB_BAND_ROWS = 32;   // luma rows a deblocking CTA owns (shifted u
 // units left of the tile and are counted in 32-bit words (2 / 4 per unit; rows are multiples of 16 bytes).
 constexpr int DB_BOX_W = RING_TILE_W + 16, DB_BOX_CW = RING_TILE_W / 2 + 16, DB_BOX_UNITS = RING_TILE_W / 4 + 8;
 constexpr int DB_BOX_MV16_WORDS = (RING_TILE_W / 4 + 4) * 2, DB_BOX_MV32_WORDS = (RING_TILE_W / 4 + 2) * 4;
+// Deblocking edge records: what ilf_set_deblock_info derives per 4-line edge segment (deblock_records_kernel) and deblock_kernel
+// reads instead of the unit grid and the motion vectors.  Four dense arrays per slot, [row][column], rows `pitch` elements apart
+// (16-byte multiples: TMA rows), covering the held rows; a zero record = nothing to filter:
+//   DB_REC_LV  luma vertical      uint16  rows: unit rows                  columns: edges x = 8 e, e = 0 .. width / 8
+//   DB_REC_LH  luma horizontal    uint16  rows: edges y = 8 j              columns: unit columns
+//   DB_REC_CV  chroma vertical    uint32  rows: unit rows                  columns: chroma edges cx = 8 m, m = 0 .. width / 16
+//   DB_REC_CH  chroma horizontal  uint32  rows: chroma edges cy = 8 j      columns: unit columns
+// (chroma: Cb record | Cr record << 16).  A tile's records are one box per array: DB_REC_BOX_W x DB_REC_BOX_H from column
+// 16 tx / 32 tx / 8 tx / 32 tx, row 8 ty - 1 / 4 ty / 8 ty - 1 / 2 ty (17 / 9 of the vertical box columns are used).
+enum { DB_REC_LV, DB_REC_LH, DB_REC_CV, DB_REC_CH, DB_REC_KINDS };
+constexpr int DB_REC_LV_W = 24, DB_REC_LH_W = RING_TILE_W / 4, DB_REC_CV_W = 16, DB_REC_CH_W = RING_TILE_W / 4;
+constexpr int DB_REC_LV_H = DB_BAND_ROWS / 4, DB_REC_LH_H = DB_BAND_ROWS / 8, DB_REC_CV_H = DB_BAND_ROWS / 4, DB_REC_CH_H = DB_BAND_ROWS / 16;
+struct DbRecLayout {
+  int cols[DB_REC_KINDS], rows[DB_REC_KINDS], pitch[DB_REC_KINDS], elem[DB_REC_KINDS];  // elem: bytes per record
+  size_t off[DB_REC_KINDS], bytes;                                                       // offsets in the slot's allocation
+};
+inline DbRecLayout db_rec_layout(const Geom& g) {
+  DbRecLayout L;
+  const int cols[4] = {g.width / 8 + 1, g.units_w, g.width / 16 + 1, g.units_w}, rows[4] = {g.rows / 4, g.rows / 8, g.rows / 4, (g.rows + 15) / 16};
+  size_t at = 0;
+  for (int k = 0; k < DB_REC_KINDS; k++) {
+    L.cols[k] = cols[k];
+    L.rows[k] = rows[k];
+    L.elem[k] = k < DB_REC_CV ? 2 : 4;
+    const int per16 = 16 / L.elem[k];
+    L.pitch[k] = (cols[k] + per16 - 1) / per16 * per16;
+    L.off[k] = at;
+    at += ((size_t)L.pitch[k] * rows[k] * L.elem[k] + 255) & ~size_t(255);
+  }
+  L.bytes = at;
+  return L;
+}
+
 constexpr int SAO_BAND_ROWS = 32;  // rows a SAO CTA owns; the box adds one halo row above and below
 constexpr int ALF_BAND_ROWS = 32;  // rows an ALF CTA owns; the box adds 3 (luma, 7x7 + classification) or 2 (chroma, 5x5) halo rows on each side
 constexpr int ALF_HALO_Y = 3, ALF_HALO_C = 2;
@@ -57,6 +90,7 @@ struct alignas(64) SlotDev {
   CUtensorMap tm_db[3];     // box DB_BOX_W x DB_BAND_ROWS (luma), DB_BOX_CW x DB_BAND_ROWS/2 (chroma)
   CUtensorMap tm_info, tm_info_c;  // unit grids, tensor (unit x, unit y, 1) of uint32: box DB_BOX_UNITS x 8
   CUtensorMap tm_mv16, tm_mv32;    // motion vectors as uint32 words (2 / 4 per unit): box DB_BOX_MV16_WORDS x 8 / DB_BOX_MV32_WORDS x 8
+  CUtensorMap tm_rec[DB_REC_KINDS];  // deblocking edge records (DB_REC_*), tensor (column, row, 1): box DB_REC_*_W x DB_REC_*_H
   CUtensorMap tm_sao[3];    // box SAO_TILE x (SAO_BAND_ROWS + 2)
   CUtensorMap tm_alf[3];    // box (ALF_TILE + 16) x (ALF_BAND_ROWS + 2 * halo), loaded 8 samples left of the tile
   int16_t* buf[3][3];       // [buffer: 0 = input, 1, 2 = work][plane]
@@ -157,7 +191,11 @@ inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, s
 }
 
 // One launch covers `num_slots` <= MAX_BATCH grid layers; layer z works on slot first_slot + ctl.slot[z] under control word ctl.v[z].
-void launch_deblock(const Geom& g, const SlotDev* slots, int first_slot, int num_slots, const BatchCtl& ctl, int mv_mode, int* work, cudaStream_t st);
+void launch_deblock(const Geom& g, const SlotDev* slots, int first_slot, int num_slots, const BatchCtl& ctl, int* work, cudaStream_t st);
+// The edge records of one slot (layout db_rec_layout(g), at `rec`) from its deblocking side information in device memory (mv16 /
+// mv32 / info_c may be null; ctu_slice null: every CTU in slice 0).
+void launch_deblock_records(const Geom& g, const ilf_deblock_params* params, const uint32_t* info, const uint32_t* info_c, const int16_t* mv16,
+                            const int32_t* mv32, const uint8_t* ctu_slice, void* rec, cudaStream_t st);
 // ilf_deblock_search: adds sum((D_k - O)^2 >> shift) of every candidate k and plane to out[(first_slot + ctl.slot[z]) * 192 + 3 k + plane].
 void launch_deblock_search(const Geom& g, const SlotDev* slots, int first_slot, int num_slots, const BatchCtl& ctl, int mv_mode, const ilf_deblock_candidate* cands,
                            int num_cands, int shift_luma, int shift_chroma, unsigned long long* out, cudaStream_t st);

@@ -13,8 +13,8 @@
 // inside a picture (tile of a band, band: rows [32 ty - 4, 32 ty + 28), chroma [16 ty - 2, 16 ty + 14), units [8 ty - 1, 8 ty + 7)),
 // picture after picture; 148 x 6 CTAs draw tile numbers from one device counter (atomicAdd; the last CTA to leave resets it for
 // the next launch on the stream) and each keeps a ring of DB_STAGES shared-memory stages: the TMA boxes of a tile -- luma 144 x 32
-// from x0 - 8, Cb and Cr 80 x 16 from cx0 - 8, the unit grid 40 x 8 from unit ux0 - 4 (and its chroma-tree layer), motion vectors of
-// units ux0 - 2 .. ux0 + 33 -- land in one stage while the tile of the other stage is filtered.  Because the queue hands tiles out in
+// from x0 - 8, Cb and Cr 80 x 16 from cx0 - 8, and the tile's edge records (ilf_common.cuh DB_REC_*: 24 x 8 + 32 x 4 uint16 for luma,
+// 16 x 8 + 32 x 2 uint32 for chroma, 1.4 KB) -- land in one stage while the tile of the other stage is filtered.  Because the queue hands tiles out in
 // raster order whatever the CTAs' relative progress, the CTAs resident at any moment cover a compact window of the picture.
 // That order is what the memory system rewards (profiles/r02_ring_vs_copy.txt, tools/ubench/tma_ring.cu): the same boxes moved by
 // persistent CTAs that each walk a band -- the design of round 1 -- copy at 4.7 TB/s, handed out in raster order 5.7 TB/s, because
@@ -29,16 +29,21 @@
 // Every sample crosses HBM once in and once out (the reference makes two picture passes); the 16 halo columns of a box are
 // L2 hits (the neighbouring tiles are in flight at the same time).
 //
-// Per-edge derivation on the device (xGetBoundaryStrengthSingle :419-541, QP/tc/beta :626-634, chroma QP
-// :811-829) from the packed per-4x4 grid described in include/ilf_b200.h.
+// Edge records.  Everything about a segment that does not depend on the samples -- edge flag and bS (xGetBoundaryStrengthSingle
+// :419-541), the no-filter sides, the QP with the slice's beta / tc offsets applied as table indices (:626-634), for chroma the
+// plane's QP offset and mapping (:811-829) -- is fixed once the picture's side information is: deblock_records_kernel derives it
+// from the packed per-4x4 grid and motion vectors (include/ilf_b200.h) when ilf_set_deblock_info copies them, on a stream of its own,
+// into a 16-bit record per segment.  deblock_kernel reads the records instead of the grid and the motion vectors (about 1.4 KB per
+// tile instead of 3.6 KB), so it does not depend on the motion-vector representation: one launch per batch.
 //
 // Work split: the unit of deblocking work is a SEGMENT (4 lines of one edge).  The 160 threads of a CTA take one
 // segment each in four phases -- luma vertical (17 edge columns x 8 = 136 tasks), chroma vertical (2 planes x 9 x 8 = 144),
-// luma horizontal (4 edge rows x 32 = 128), chroma horizontal (2 x 2 x 32 = 128) -- so edge flag, bS, QP, tc and beta are
-// derived once per segment and segments without an edge cost a few instructions.  The fifth warp has vertical tasks only: its
-// first thread draws the next tile from the queue while the other four run the horizontal pass.
+// luma horizontal (4 edge rows x 32 = 128), chroma horizontal (2 x 2 x 32 = 128) -- and a segment without an edge (zero record)
+// costs a few instructions.  The fifth warp has vertical tasks only: its first thread draws the next tile from the queue while the
+// other four run the horizontal pass.
 // A chroma plane with the skip bit in its picture's control word (ilf_set_deblock_info found no intra unit: chroma is filtered
-// for bS == 2 only, so the plane would come out unchanged) is not loaded, filtered or stored; it stays in the upload buffer.
+// for bS == 2 only, so the plane would come out unchanged) is not loaded, filtered or stored; it stays in the upload buffer.  When
+// both are skipped the chroma records are not loaded either.
 #include <algorithm>
 #include <cstdlib>
 
@@ -65,12 +70,14 @@ constexpr int MV16_UNITS = DB_BOX_MV16_WORDS / 2, MV32_UNITS = DB_BOX_MV32_WORDS
 constexpr int NTHREADS = ILF_DB_WIDE ? 288 : 160;   // 136 / 144 vertical-edge tasks in one round; the horizontal passes use 128 of them
 constexpr int VC0 = ILF_DB_WIDE ? 136 : 0, HC0 = ILF_DB_WIDE ? 128 : 0;   // first thread of the chroma tasks of the vertical / horizontal phase
 // Ring depth and residency (measured, 17 4K pictures): 3 stages x 3 CTAs per SM 0.237 ms, 2 x 4 0.206 ms, 2 x 5 0.194 ms -- the kernel
-// is bound by the latency of a tile's dependent phases, so more, smaller CTAs win over deeper prefetch; 67 registers at 5 CTAs.
+// is bound by the latency of a tile's dependent phases, so more, smaller CTAs win over deeper prefetch.  With edge records instead of
+// grid and motion boxes (15.4 KB stages, ra_4k stream decisions, B200): 2 x 5 0.1328 ms (66 registers), 2 x 6 0.1286 ms (59 registers,
+// no spills), 3 x 5 0.1412 ms, 3 stages at a bound of 6 (4 fit by shared memory) 0.1414 ms.
 #ifndef ILF_DB_STAGES
 #define ILF_DB_STAGES 2
 #endif
 #ifndef ILF_DB_MIN_CTAS
-#define ILF_DB_MIN_CTAS 5
+#define ILF_DB_MIN_CTAS 6
 #endif
 constexpr int DB_STAGES = ILF_DB_STAGES;            // ring depth: the tile being filtered + DB_STAGES - 1 in flight (>= 2)
 static_assert(DB_STAGES >= 2 && DB_STAGES <= 8, "a stage's next tile id is read one step after it was written only behind a barrier when there are two or more stages");
@@ -93,8 +100,15 @@ template <int MV> struct MvBox { static constexpr int UNITS = 1, OFF = 0; };
 template <> struct MvBox<1> { static constexpr int UNITS = MV16_UNITS, OFF = 2; };
 template <> struct MvBox<2> { static constexpr int UNITS = MV32_UNITS, OFF = 1; };
 
-// One stage = what the TMA unit delivers for a tile (dense boxes, each 128-byte aligned): sample column c of the tile is
-// box column c + 8, unit column c is box column c + 4 (motion: c + 2 / c + 1).
+template <int MV> __device__ __forceinline__ void mv_get(const MvT<MV>& v, int m[4]);
+template <> __device__ __forceinline__ void mv_get<0>(const MvT<0>&, int m[4]) { m[0] = m[1] = m[2] = m[3] = 0; }
+template <> __device__ __forceinline__ void mv_get<1>(const MvT<1>& t, int m[4]) {
+  m[0] = (int)(int16_t)(t.v.x & 0xFFFF); m[1] = (int)(int16_t)(t.v.x >> 16); m[2] = (int)(int16_t)(t.v.y & 0xFFFF); m[3] = (int)(int16_t)(t.v.y >> 16);
+}
+template <> __device__ __forceinline__ void mv_get<2>(const MvT<2>& t, int m[4]) { m[0] = t.v.x; m[1] = t.v.y; m[2] = t.v.z; m[3] = t.v.w; }
+
+// A stage of the offset search = what the TMA unit delivers for a tile (dense boxes, each 128-byte aligned): sample column c of the
+// tile is box column c + 8, unit column c is box column c + 4 (motion: c + 2 / c + 1).
 template <int MV>
 struct Stage {
   int16_t y[TH][BW];
@@ -117,27 +131,42 @@ struct Tile {
   bool ctree;
   __device__ __forceinline__ uint32_t info(int r, int c) const { return st->info[r][c + 4]; }
   __device__ __forceinline__ uint32_t cinfo(int r, int c) const { return ctree ? st->info_c[r][c + 4] : st->info[r][c + 4]; }
-  __device__ __forceinline__ MvT<MV> mv(int r, int c) const { return st->mv[MV ? r : 0][MV ? c + MvBox<MV>::OFF : 0]; }
+  __device__ __forceinline__ void mvs(int r, int c, int m[4]) const { mv_get<MV>(st->mv[MV ? r : 0][MV ? c + MvBox<MV>::OFF : 0], m); }
   __device__ __forceinline__ int16_t* y(int r, int c) const { return &st->y[r][c + 8]; }
   __device__ __forceinline__ int16_t* ch(int pl, int r, int c) const { return &st->c[pl][r][c + 8]; }
 };
 
-template <int MV> __device__ __forceinline__ void mv_get(const MvT<MV>& v, int m[4]);
-template <> __device__ __forceinline__ void mv_get<0>(const MvT<0>&, int m[4]) { m[0] = m[1] = m[2] = m[3] = 0; }
-template <> __device__ __forceinline__ void mv_get<1>(const MvT<1>& t, int m[4]) {
-  m[0] = (int)(int16_t)(t.v.x & 0xFFFF); m[1] = (int)(int16_t)(t.v.x >> 16); m[2] = (int)(int16_t)(t.v.y & 0xFFFF); m[3] = (int)(int16_t)(t.v.y >> 16);
-}
-template <> __device__ __forceinline__ void mv_get<2>(const MvT<2>& t, int m[4]) { m[0] = t.v.x; m[1] = t.v.y; m[2] = t.v.z; m[3] = t.v.w; }
+// The same accessors over the slot's side information in device memory (the record pass): unit (r, c) of the held rows; what
+// lies outside them reads as zeros, as outside the picture in a TMA box.
+struct Grid {
+  const uint32_t* units;
+  const uint32_t* units_c;  // chroma-tree layer or nullptr
+  const int16_t* mv16;      // at most one of the two; neither: every unit intra, no vector is read
+  const int32_t* mv32;
+  int units_w, units_h, pitch;
+  __device__ __forceinline__ bool in(int r, int c) const { return r >= 0 && r < units_h && c >= 0 && c < units_w; }
+  __device__ __forceinline__ uint32_t info(int r, int c) const { return in(r, c) ? __ldg(units + (size_t)r * pitch + c) : 0u; }
+  __device__ __forceinline__ uint32_t cinfo(int r, int c) const { return in(r, c) ? __ldg((units_c ? units_c : units) + (size_t)r * pitch + c) : 0u; }
+  __device__ __forceinline__ void mvs(int r, int c, int m[4]) const {
+    MvT<2> v = {make_int4(0, 0, 0, 0)};
+    if (in(r, c) && mv32) v.v = __ldg(reinterpret_cast<const int4*>(mv32) + (size_t)r * pitch + c);
+    if (in(r, c) && mv16) {
+      const uint2 w = __ldg(reinterpret_cast<const uint2*>(mv16) + (size_t)r * pitch + c);
+      v.v = make_int4((int16_t)(w.x & 0xFFFF), (int16_t)(w.x >> 16), (int16_t)(w.y & 0xFFFF), (int16_t)(w.y >> 16));
+    }
+    mv_get<2>(v, m);
+  }
+};
 
-// bS of one 4-sample segment (xGetBoundaryStrengthSingle, LoopFilter.cpp:419-541).  q, p index the staged window.
-template <int MV>
-__device__ __forceinline__ int boundary_strength(const Tile<MV>& t, uint32_t iq, uint32_t ip, int qr, int qc, int pr, int pc, uint32_t tu_bit, int thr) {
+// bS of one 4-sample segment (xGetBoundaryStrengthSingle, LoopFilter.cpp:419-541).  q, p index the view (Tile or Grid).
+template <class View>
+__device__ __forceinline__ int boundary_strength(const View& t, uint32_t iq, uint32_t ip, int qr, int qc, int pr, int pc, uint32_t tu_bit, int thr) {
   if ((iq | ip) & ILF_BI_INTRA) return 2;
   if ((iq & tu_bit) && ((iq | ip) & ILF_BI_CBF)) return 1;
   const int rq0 = (iq >> 16) & 0xFF, rq1 = iq >> 24, rp0 = (ip >> 16) & 0xFF, rp1 = ip >> 24;
   int mq[4], mp[4];
-  mv_get<MV>(t.mv(qr, qc), mq);
-  mv_get<MV>(t.mv(pr, pc), mp);
+  t.mvs(qr, qc, mq);
+  t.mvs(pr, pc, mp);
   const bool d00 = abs(mq[0] - mp[0]) >= thr || abs(mq[1] - mp[1]) >= thr;
   if ((iq | ip) & ILF_BI_BSLICE) {
     if ((rp0 == rq0 && rp1 == rq1) || (rp0 == rq1 && rp1 == rq0)) {
@@ -179,49 +208,106 @@ __device__ __forceinline__ void filter_luma_line(int v[8], int tc, bool sw, bool
   if (no_q) { v[4] = m4; v[5] = m5; v[6] = m6; }
 }
 
-// Per-picture parameters and the tc / beta / chroma-QP tables, copied to shared memory once per CTA: the per-segment
-// derivations index them with per-thread values (constant memory would serialise) and must not wait on global loads.
-struct DbShared {
-  int tile[8];               // tile in (or on its way into) every stage of the ring: tx | ty << 8 | z << 20, -1 = the queue is empty
-  int cur_slot;              // grid layer whose parameters are in prm
-  int next;                  // tile drawn for the stage that is being emptied
-  int16_t* dst[3];           // destination planes, control word and chroma-tree flag of grid layer cur_slot
-  unsigned ctl;
-  int ctree;
-  ilf_deblock_params prm;
-  const uint8_t* ctu_slice;  // nullptr: every CTU in slice 0
-  uint8_t tc[66 + 2], beta[64], chroma_scale[70 + 2];
-};
-
 struct EdgeParams {
   int bs;        // 0 = leave the segment alone
   int tc, beta;
   bool no_p, no_q;
 };
 
-__device__ __forceinline__ int slice_of(const Geom& g, const DbShared& sh, int xg, int yg_local) {
-  return sh.ctu_slice ? (int)__ldg(sh.ctu_slice + (size_t)((yg_local + g.row0) >> g.ctu_log2) * g.ctus_w + (xg >> g.ctu_log2)) : 0;
+// Offset-independent part of a luma segment (xEdgeFilterLuma, LoopFilter.cpp:543-634, up to the tables): 0 = not filtered, else
+// bS | no_p << 2 | no_q << 3 | (QP & 0xFF) << 8.  (qr, qc) / (pr, pc) = unit row and column of the Q / P unit in the view.
+template <class View>
+__device__ __forceinline__ uint32_t luma_edge_record(const View& t, int thr, int qr, int qc, int pr, int pc, bool vertical) {
+  const uint32_t iq = t.info(qr, qc), ip = t.info(pr, pc);
+  if (!(iq & (vertical ? ILF_BI_EDGE_V : ILF_BI_EDGE_H))) return 0;
+  const int bs = boundary_strength(t, iq, ip, qr, qc, pr, pc, vertical ? ILF_BI_TU_V : ILF_BI_TU_H, thr);
+  if (!bs) return 0;
+  const int qp = ((int)(int8_t)(ip >> 8) + (int)(int8_t)(iq >> 8) + 1) >> 1;
+  return (uint32_t)bs | ((ip & ILF_BI_NOFILT) ? 4u : 0u) | ((iq & ILF_BI_NOFILT) ? 8u : 0u) | ((uint32_t)(qp & 0xFF) << 8);
 }
 
-// Parameters of one luma segment (xEdgeFilterLuma, LoopFilter.cpp:543-634): edge flag, bS, QP, tc, beta.  (xg, yg) = first Q sample.
-// (qr, qc) / (pr, pc) = unit row and column of the Q / P unit in the tile's window.
-template <int MV>
-__device__ __forceinline__ EdgeParams luma_edge_params(const Tile<MV>& t, const Geom& g, const DbShared& sh, int qr, int qc, int pr, int pc, bool vertical, int xg, int yg) {
+// Offset-independent part of a chroma segment (xEdgeFilterChroma, LoopFilter.cpp:684-838, up to the table): 0 = not filtered, else
+// 1 | no_p << 1 | no_q << 2 | (chroma QP after the mapping) << 16.
+__device__ __forceinline__ uint32_t chroma_edge_record(uint32_t iq, uint32_t ip, const ilf_deblock_params& prm, const uint8_t* chroma_scale, bool vertical, int comp) {
+  if (!(iq & (vertical ? ILF_BI_EDGE_V : ILF_BI_EDGE_H))) return 0;
+  if (!((iq | ip) & ILF_BI_INTRA)) return 0;  // chroma is filtered for bS == 2 only (:769)
+  int qp = (((int)(int8_t)(ip >> 8) + (int)(int8_t)(iq >> 8) + 1) >> 1) + (comp == 0 ? prm.cb_qp_offset : prm.cr_qp_offset);
+  if (qp >= 70) qp -= 6;
+  else if (qp >= 0) qp = chroma_scale[qp];
+  return 1u | ((ip & ILF_BI_NOFILT) ? 2u : 0u) | ((iq & ILF_BI_NOFILT) ? 4u : 0u) | ((uint32_t)qp << 16);
+}
+
+// ---------------------------------------------------------------------------------------------------------------------------
+// Record pass (ilf_set_deblock_info).  A segment's 16-bit record, 0 = nothing to filter:
+//   luma    1 | no_p << 1 | no_q << 2 | tc index << 3 | beta index << 10   (indices into c_tc / c_beta, slice offsets applied)
+//   chroma  1 | no_p << 1 | no_q << 2 | tc index << 3                      (per plane: QP offset and mapping applied)
+// deblock_kernel multiplies the table values by the bit-depth scale.
+__device__ __forceinline__ uint32_t luma_record(uint32_t r, const ilf_slice_params& sl) {
+  if (!r) return 0;
+  const int bs = r & 3, qp = (int)(int8_t)(r >> 8);
+  const int tci = clip3i(0, 65, qp + 2 * (bs - 1) + 2 * sl.tc_offset_div2), bi = clip3i(0, 63, qp + 2 * sl.beta_offset_div2);
+  return 1u | ((r & 4) ? 2u : 0u) | ((r & 8) ? 4u : 0u) | (uint32_t)tci << 3 | (uint32_t)bi << 10;
+}
+__device__ __forceinline__ uint32_t chroma_record(uint32_t r, const ilf_slice_params& sl) {
+  if (!r) return 0;
+  return 1u | (r & 6u) | (uint32_t)clip3i(0, 65, ((int)r >> 16) + 2 + 2 * sl.tc_offset_div2) << 3;
+}
+
+// One thread per record; blockIdx.y = DB_REC_* kind.  Coordinates: unit rows / columns of the held rows, slices looked up at the
+// full-picture position of the segment's first Q sample.
+__global__ void __launch_bounds__(256) deblock_records_kernel(Geom g, Grid grid, const ilf_deblock_params* __restrict__ params, const uint8_t* __restrict__ ctu_slice,
+                                                              const __grid_constant__ DbRecLayout L, unsigned char* __restrict__ rec) {
+  __shared__ ilf_deblock_params prm;
+  __shared__ uint8_t chroma_scale[70 + 2];
+  for (int i = threadIdx.x; i < (int)(sizeof(ilf_deblock_params) / 4); i += blockDim.x) reinterpret_cast<uint32_t*>(&prm)[i] = __ldg(reinterpret_cast<const uint32_t*>(params) + i);
+  if (threadIdx.x < 70) chroma_scale[threadIdx.x] = c_chroma_scale[threadIdx.x];
+  __syncthreads();
+  const int k = blockIdx.y, cols = L.cols[k], n = cols * L.rows[k];
+  auto slice = [&](int xg, int yg) -> const ilf_slice_params& {
+    return prm.slices[ctu_slice ? (int)__ldg(ctu_slice + (size_t)((yg + g.row0) >> g.ctu_log2) * g.ctus_w + (xg >> g.ctu_log2)) : 0];
+  };
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+    const int r = i / cols, c = i - r * cols;
+    unsigned char* out = rec + L.off[k] + ((size_t)r * L.pitch[k] + c) * L.elem[k];
+    if (k == DB_REC_LV) {        // edge x = 8 c, unit row r
+      const uint32_t e = luma_edge_record(grid, prm.mv_threshold, r, 2 * c, r, 2 * c - 1, true);
+      *reinterpret_cast<uint16_t*>(out) = (uint16_t)(e ? luma_record(e, slice(8 * c, 4 * r)) : 0);
+    } else if (k == DB_REC_LH) { // edge y = 8 r, unit column c
+      const uint32_t e = luma_edge_record(grid, prm.mv_threshold, 2 * r, c, 2 * r - 1, c, false);
+      *reinterpret_cast<uint16_t*>(out) = (uint16_t)(e ? luma_record(e, slice(4 * c, 8 * r)) : 0);
+    } else {                     // chroma edge cx = 8 c (luma 16 c), unit row r / cy = 8 r (luma 16 r), unit column c
+      const bool v = k == DB_REC_CV;
+      const int qr = v ? r : 4 * r, qc = v ? 4 * c : c, pr = v ? r : 4 * r - 1, pc = v ? 4 * c - 1 : c;
+      const uint32_t iq = grid.cinfo(qr, qc), ip = grid.cinfo(pr, pc);
+      uint32_t w = 0;
+      for (int pl = 0; pl < 2; pl++) {
+        const uint32_t e = chroma_edge_record(iq, ip, prm, chroma_scale, v, pl);
+        if (e) w |= chroma_record(e, slice(v ? 16 * c : 4 * c, v ? 4 * r : 16 * r)) << (16 * pl);
+      }
+      *reinterpret_cast<uint32_t*>(out) = w;
+    }
+  }
+}
+
+// The tc / beta tables and the per-picture destination, copied to shared memory once per CTA: the segments index the tables with
+// per-thread values (constant memory would serialise).
+struct DbShared {
+  int tile[8];               // tile in (or on its way into) every stage of the ring: tx | ty << 8 | z << 20, -1 = the queue is empty
+  int cur_slot;              // grid layer whose destination is in dst / ctl
+  int next;                  // tile drawn for the stage that is being emptied
+  int16_t* dst[3];           // destination planes and control word of grid layer cur_slot
+  unsigned ctl;
+  uint8_t tc[66 + 2], beta[64];
+};
+
+// A luma record -> the segment's parameters (LoopFilter.cpp:626-634).
+__device__ __forceinline__ EdgeParams luma_edge(uint32_t rec, const DbShared& sh, int scale) {
   EdgeParams ep;
-  ep.bs = 0; ep.tc = 0; ep.beta = 0; ep.no_p = ep.no_q = false;
-  const uint32_t iq = t.info(qr, qc), ip = t.info(pr, pc);
-  if (!(iq & (vertical ? ILF_BI_EDGE_V : ILF_BI_EDGE_H))) return ep;
-  const int bs = boundary_strength<MV>(t, iq, ip, qr, qc, pr, pc, vertical ? ILF_BI_TU_V : ILF_BI_TU_H, sh.prm.mv_threshold);
-  if (!bs) return ep;
-  const int slice = slice_of(g, sh, xg, yg);
-  const int qp = ((int)(int8_t)(ip >> 8) + (int)(int8_t)(iq >> 8) + 1) >> 1;
-  const int tc_off = sh.prm.slices[slice].tc_offset_div2, beta_off = sh.prm.slices[slice].beta_offset_div2;
-  const int scale = 1 << (g.bd_luma - 8);
-  ep.bs = bs;
-  ep.tc = sh.tc[clip3i(0, 65, qp + 2 * (bs - 1) + 2 * tc_off)] * scale;
-  ep.beta = sh.beta[clip3i(0, 63, qp + 2 * beta_off)] * scale;
-  ep.no_p = (ip & ILF_BI_NOFILT) != 0;
-  ep.no_q = (iq & ILF_BI_NOFILT) != 0;
+  ep.bs = 1;
+  ep.tc = sh.tc[(rec >> 3) & 127] * scale;
+  ep.beta = sh.beta[rec >> 10] * scale;
+  ep.no_p = (rec & 2) != 0;
+  ep.no_q = (rec & 4) != 0;
   return ep;
 }
 
@@ -244,65 +330,64 @@ __device__ __forceinline__ bool filter_luma_segment(int (&L)[4][8], const EdgePa
   return true;
 }
 
-// tc of a chroma segment for one component, or -1 when the segment is not filtered (xEdgeFilterChroma, LoopFilter.cpp:684-838).
-__device__ __forceinline__ int chroma_tc(uint32_t iq, uint32_t ip, const Geom& g, const DbShared& sh, bool vertical, int comp, int xg_luma, int yg_luma,
-                                         bool& no_p, bool& no_q) {
-  if (!(iq & (vertical ? ILF_BI_EDGE_V : ILF_BI_EDGE_H))) return -1;
-  if (!((iq | ip) & ILF_BI_INTRA)) return -1;  // chroma is filtered for bS == 2 only (:769)
-  const int slice = slice_of(g, sh, xg_luma, yg_luma);
-  int qp = (((int)(int8_t)(ip >> 8) + (int)(int8_t)(iq >> 8) + 1) >> 1) + (comp == 0 ? sh.prm.cb_qp_offset : sh.prm.cr_qp_offset);
-  if (qp >= 70) qp -= 6;
-  else if (qp >= 0) qp = sh.chroma_scale[qp];
-  no_p = (ip & ILF_BI_NOFILT) != 0;
-  no_q = (iq & ILF_BI_NOFILT) != 0;
-  return sh.tc[clip3i(0, 65, qp + 2 + 2 * sh.prm.slices[slice].tc_offset_div2)] * (1 << (g.bd_chroma - 8));
-}
-
 __device__ __forceinline__ void unpack2(uint32_t w, int& a, int& b) { a = (int)(int16_t)(w & 0xFFFF); b = (int)(int16_t)(w >> 16); }
 __device__ __forceinline__ uint32_t pack2(int a, int b) { return (uint32_t)(uint16_t)a | ((uint32_t)b << 16); }
 
-template <int MV>
+// One stage of deblock_kernel = what the TMA unit delivers for a tile (dense boxes, each 128-byte aligned): sample column c of the
+// tile is box column c + 8; the record boxes start at the tile's first edge column and first segment row (ilf_common.cuh).
+struct DbStage {
+  int16_t y[TH][BW];
+  int16_t c[2][CTH][BCW];
+  uint16_t rec_lv[DB_REC_LV_H][DB_REC_LV_W];   // [segment row sg][edge e]: x0 + 8 e, rows y0 + 4 sg ..
+  uint16_t rec_lh[DB_REC_LH_H][DB_REC_LH_W];   // [edge row h][unit column u]: y0 + 4 + 8 h, columns x0 + 4 u ..
+  uint32_t rec_cv[DB_REC_CV_H][DB_REC_CV_W];   // [segment row sg][edge k]: cx0 + 8 k, chroma rows cy0 + 2 sg .. (Cb | Cr << 16)
+  uint32_t rec_ch[DB_REC_CH_H][DB_REC_CH_W];   // [edge row h][unit column u]: cy0 + 2 + 8 h, chroma columns cx0 + 2 u ..
+};
+static_assert(sizeof(int16_t[TH][BW]) % 128 == 0 && sizeof(int16_t[CTH][BCW]) % 128 == 0 && sizeof(uint16_t[DB_REC_LV_H][DB_REC_LV_W]) % 128 == 0 &&
+              sizeof(uint16_t[DB_REC_LH_H][DB_REC_LH_W]) % 128 == 0 && sizeof(uint32_t[DB_REC_CV_H][DB_REC_CV_W]) % 128 == 0, "TMA destinations are 128-byte aligned");
+static_assert(DB_REC_LV_W >= TW / 8 + 1 && DB_REC_CV_W >= CTW / 8 + 1, "a vertical record box holds the tile's edges and the next tile's first");
+constexpr int DB_STRIDE = (int)((sizeof(DbStage) + 127) & ~size_t(127));
+constexpr int DB_REC_LUMA_BYTES = (int)(sizeof(DbStage::rec_lv) + sizeof(DbStage::rec_lh)), DB_REC_CHROMA_BYTES = (int)(sizeof(DbStage::rec_cv) + sizeof(DbStage::rec_ch));
+
 __global__ void __launch_bounds__(NTHREADS, ILF_DB_MIN_CTAS) deblock_kernel(Geom g, const SlotDev* __restrict__ slots, int first_slot, BatchCtl bc, int num_slots, int* __restrict__ work) {
   extern __shared__ __align__(128) unsigned char smem[];
-  constexpr int STRIDE = stage_stride<MV>();
   constexpr int S = DB_STAGES;
   pdl_launch_dependents();
   const int tid = threadIdx.x;
   const int rows = g.rows, crow = g.rows >> 1, cw = g.width >> 1;
   const int ntx = (g.width + TW - 1) / TW, bands = (g.rows + 4 + TH - 1) / TH;
   const int total = ntx * bands * num_slots;
-  uint64_t* full = reinterpret_cast<uint64_t*>(smem + S * STRIDE);
-  DbShared& sh = *reinterpret_cast<DbShared*>(smem + S * STRIDE + 8 * S);
+  uint64_t* full = reinterpret_cast<uint64_t*>(smem + S * DB_STRIDE);
+  DbShared& sh = *reinterpret_cast<DbShared*>(smem + S * DB_STRIDE + 8 * S);
   // tile id -> (grid layer, band, tile of the band): raster order inside a picture, pictures one after the other
   auto pack_id = [&](int id) { if (id >= total) return -1; const int tx = id % ntx, r = id / ntx; return tx | (r % bands) << 8 | (r / bands) << 20; };
   auto decode = [&](int id, int& z, int& ty, int& tx) { tx = id & 255; ty = (id >> 8) & 4095; z = id >> 20; };
   // The boxes of a tile are issued by the first lanes of the CTA's warps, one part each, so that their descriptor fetches
-  // overlap: part 0 arms the barrier and loads luma, 1 both chroma planes, 2 the unit grids, 3 motion.  A skipped chroma plane
-  // (a picture without an intra unit: no chroma edge is filtered) is neither loaded nor stored.  The tile may belong to another
-  // picture than sh.cur_slot, so its control word is read from bc.
+  // overlap: part 0 arms the barrier and loads luma, 1 both chroma planes, 2 the luma records, 3 the chroma records.  A skipped
+  // chroma plane (a picture without an intra unit: no chroma edge is filtered) is neither loaded nor stored, and with both planes
+  // skipped the chroma records stay behind too.  The tile may belong to another picture than sh.cur_slot, so its control word is
+  // read from bc.
   auto issue_part = [&](int id, int si, int part) {  // tile id into stage si
     int z, ty, tx;
     decode(id, z, ty, tx);
     const SlotDev& sd = slots[first_slot + bc.slot[z]];
     const unsigned c = bc.v[z];
-    const int src_b = ctl_src(c, 0);
-    const int y0 = ty * TH - 4, cy0 = ty * CTH - 2, uy0 = ty * UH - 1;  // band origin (local rows)
-    const bool has_ctree = (part == 0 || part == 2) ? (z == sh.cur_slot ? sh.ctree != 0 : sd.info_c != nullptr) : false;
-    Stage<MV>* st = reinterpret_cast<Stage<MV>*>(smem + si * STRIDE);
+    const bool chroma = !(ctl_skip(c, 1) && ctl_skip(c, 2));
+    DbStage* st = reinterpret_cast<DbStage*>(smem + si * DB_STRIDE);
     uint64_t* bar = &full[si];
     if (part == 0) {
       const int skipped = (int)ctl_skip(c, 1) + (int)ctl_skip(c, 2);
-      ring::mbar_expect_tx(bar, (uint32_t)(stage_tx_bytes<MV>(has_ctree) - skipped * (CTH * BCW * 2)));
-      ring::tma_load_3d(&st->y[0][0], &sd.tm_db[0], bar, tx * TW - 8, y0, src_b);
+      ring::mbar_expect_tx(bar, (uint32_t)(TH * BW * 2 + (2 - skipped) * (CTH * BCW * 2) + DB_REC_LUMA_BYTES + (chroma ? DB_REC_CHROMA_BYTES : 0)));
+      ring::tma_load_3d(&st->y[0][0], &sd.tm_db[0], bar, tx * TW - 8, ty * TH - 4, ctl_src(c, 0));
     } else if (part == 1) {
-      if (!ctl_skip(c, 1)) ring::tma_load_3d(&st->c[0][0][0], &sd.tm_db[1], bar, tx * CTW - 8, cy0, src_b);
-      if (!ctl_skip(c, 2)) ring::tma_load_3d(&st->c[1][0][0], &sd.tm_db[2], bar, tx * CTW - 8, cy0, src_b);
+      if (!ctl_skip(c, 1)) ring::tma_load_3d(&st->c[0][0][0], &sd.tm_db[1], bar, tx * CTW - 8, ty * CTH - 2, ctl_src(c, 0));
+      if (!ctl_skip(c, 2)) ring::tma_load_3d(&st->c[1][0][0], &sd.tm_db[2], bar, tx * CTW - 8, ty * CTH - 2, ctl_src(c, 0));
     } else if (part == 2) {
-      ring::tma_load_3d(&st->info[0][0], &sd.tm_info, bar, tx * UW - 4, uy0, 0);
-      if (has_ctree) ring::tma_load_3d(&st->info_c[0][0], &sd.tm_info_c, bar, tx * UW - 4, uy0, 0);
-    } else {
-      if (MV == 1) ring::tma_load_3d(&st->mv[0][0], &sd.tm_mv16, bar, (tx * UW - MvBox<1>::OFF) * 2, uy0, 0);
-      if (MV == 2) ring::tma_load_3d(&st->mv[0][0], &sd.tm_mv32, bar, (tx * UW - MvBox<2>::OFF) * 4, uy0, 0);
+      ring::tma_load_3d(&st->rec_lv[0][0], &sd.tm_rec[DB_REC_LV], bar, tx * (TW / 8), ty * UH - 1, 0);
+      ring::tma_load_3d(&st->rec_lh[0][0], &sd.tm_rec[DB_REC_LH], bar, tx * UW, ty * (TH / 8), 0);
+    } else if (chroma) {
+      ring::tma_load_3d(&st->rec_cv[0][0], &sd.tm_rec[DB_REC_CV], bar, tx * (CTW / 8), ty * UH - 1, 0);
+      ring::tma_load_3d(&st->rec_ch[0][0], &sd.tm_rec[DB_REC_CH], bar, tx * UW, ty * (TH / 16), 0);
     }
   };
   if (tid == 0) {
@@ -312,7 +397,6 @@ __global__ void __launch_bounds__(NTHREADS, ILF_DB_MIN_CTAS) deblock_kernel(Geom
   }
   if (tid < 66) sh.tc[tid] = c_tc[tid];
   if (tid < 64) sh.beta[tid] = c_beta[tid];
-  if (tid < 70) sh.chroma_scale[tid] = c_chroma_scale[tid];
   pdl_wait();  // the previous chain's last stage has finished with the buffers this stage reads and writes -- and has reset the work counter
   // Work queue: tiles are drawn from one counter in raster order, so the CTAs resident at any moment work on a compact window of
   // the picture whatever their relative progress; a CTA keeps S - 1 tiles in flight ahead of the one it filters.
@@ -323,6 +407,7 @@ __global__ void __launch_bounds__(NTHREADS, ILF_DB_MIN_CTAS) deblock_kernel(Geom
     for (int i = 0; i < S; i++) if (sh.tile[i] >= 0 && tid < 128) issue_part(sh.tile[i], i, tid >> 5);
 
   const int max_y = (1 << g.bd_luma) - 1, max_c = (1 << g.bd_chroma) - 1;
+  const int scale_y = 1 << (g.bd_luma - 8), scale_c = 1 << (g.bd_chroma - 8);
   const bool filt = !(g.debug & 1);
   int si = 0;
   uint32_t phases = 0;   // bit s: parity of stage s's next completion
@@ -331,16 +416,13 @@ __global__ void __launch_bounds__(NTHREADS, ILF_DB_MIN_CTAS) deblock_kernel(Geom
     if (id < 0) break;
     int z, ty, tx;
     decode(id, z, ty, tx);
-    if (sh.cur_slot != z) {   // CTA-uniform: the picture's parameters -> shared memory (once per picture a CTA meets)
+    if (sh.cur_slot != z) {   // CTA-uniform: the picture's destination -> shared memory (once per picture a CTA meets)
       __syncthreads();
-      const SlotDev& sd = slots[first_slot + bc.slot[z]];
-      for (int i = tid; i < (int)(sizeof(ilf_deblock_params) / 4); i += NTHREADS) reinterpret_cast<uint32_t*>(&sh.prm)[i] = __ldg(reinterpret_cast<const uint32_t*>(sd.db_params) + i);
       if (tid == 0) {
-        sh.ctu_slice = __ldg(&sd.db_params->num_slices) == 1 ? nullptr : sd.ctu_slice;  // one slice: no per-CTU lookup
+        const SlotDev& sd = slots[first_slot + bc.slot[z]];
         const unsigned c = bc.v[z];
         const int db = ctl_dst(c, 0);  // deblocking starts from the uploaded picture: all planes in one buffer (skipped planes are not written)
         sh.ctl = c; sh.dst[0] = sd.buf[db][0]; sh.dst[1] = sd.buf[db][1]; sh.dst[2] = sd.buf[db][2];
-        sh.ctree = sd.info_c != nullptr;
         sh.cur_slot = z;
       }
       __syncthreads();
@@ -349,9 +431,7 @@ __global__ void __launch_bounds__(NTHREADS, ILF_DB_MIN_CTAS) deblock_kernel(Geom
     int16_t* __restrict__ dst_y = sh.dst[0];
     int16_t* __restrict__ dst_cb = sh.dst[1];
     int16_t* __restrict__ dst_cr = sh.dst[2];
-    Tile<MV> t;
-    t.st = reinterpret_cast<Stage<MV>*>(smem + si * STRIDE);
-    t.ctree = sh.ctree != 0;
+    DbStage* const st = reinterpret_cast<DbStage*>(smem + si * DB_STRIDE);
     ring::mbar_wait(&full[si], (phases >> si) & 1u);
     phases ^= 1u << si;
     const int x0 = tx * TW, cx0 = tx * CTW;
@@ -361,10 +441,11 @@ __global__ void __launch_bounds__(NTHREADS, ILF_DB_MIN_CTAS) deblock_kernel(Geom
       if (tid < 17 * 8) {
         const int task = tid;
         const int e = task < 128 ? (task & 15) : 16, sg = task < 128 ? (task >> 4) : task - 128;
-        const EdgeParams ep = luma_edge_params<MV>(t, g, sh, sg, 2 * e, sg, 2 * e - 1, true, x0 + 8 * e, y0 + 4 * sg);
-        if (ep.bs) {
-          int16_t* pp = t.y(4 * sg, 8 * e - 4);
-          int16_t* pq = t.y(4 * sg, 8 * e);
+        const uint32_t rec = st->rec_lv[sg][e];
+        if (rec) {
+          const EdgeParams ep = luma_edge(rec, sh, scale_y);
+          int16_t* pp = &st->y[4 * sg][8 * e + 4];
+          int16_t* pq = &st->y[4 * sg][8 * e + 8];
           int L[4][8];
 #pragma unroll
           for (int i = 0; i < 4; i++) {
@@ -385,11 +466,12 @@ __global__ void __launch_bounds__(NTHREADS, ILF_DB_MIN_CTAS) deblock_kernel(Geom
       const int pl = task < 128 ? (task >> 6) : ((task - 128) >> 3);
       if (tid >= VC0 && task < 2 * 9 * 8 && !ctl_skip(sh.ctl, 1 + pl)) {
         const int k = task < 128 ? ((task >> 3) & 7) : 8, sg = task & 7;
-        bool no_p, no_q;
-        const int tc = chroma_tc(t.cinfo(sg, 4 * k), t.cinfo(sg, 4 * k - 1), g, sh, true, pl, 2 * (cx0 + 8 * k), 2 * (cy0 + 2 * sg), no_p, no_q);
-        if (tc >= 0) {
-          int16_t* pp = t.ch(pl, 2 * sg, 8 * k - 2);
-          int16_t* pq = t.ch(pl, 2 * sg, 8 * k);
+        const uint32_t rec = (st->rec_cv[sg][k] >> (16 * pl)) & 0xFFFFu;
+        if (rec) {
+          const int tc = sh.tc[rec >> 3] * scale_c;
+          const bool no_p = rec & 2, no_q = rec & 4;
+          int16_t* pp = &st->c[pl][2 * sg][8 * k + 6];
+          int16_t* pq = &st->c[pl][2 * sg][8 * k + 8];
 #pragma unroll
           for (int i = 0; i < 2; i++) {
             const int m2 = pp[i * BCW], m3 = pp[i * BCW + 1], m4 = pq[i * BCW], m5 = pq[i * BCW + 1];
@@ -409,20 +491,19 @@ __global__ void __launch_bounds__(NTHREADS, ILF_DB_MIN_CTAS) deblock_kernel(Geom
     //      (a warp = one edge row: 256 contiguous bytes per stored row) ----
     if (tid < 128) {
       const int u = tid & 31, h = tid >> 5;
-      const int16_t* sp = t.y(8 * h, 4 * u);
+      const int16_t* sp = &st->y[8 * h][4 * u + 8];
       uint2 raw[8];
 #pragma unroll
       for (int i = 0; i < 8; i++) raw[i] = *reinterpret_cast<const uint2*>(sp + i * BW);
-      if (filt) {
-        const EdgeParams ep = luma_edge_params<MV>(t, g, sh, 2 * h + 1, u, 2 * h, u, false, x0 + 4 * u, y0 + 4 + 8 * h);
-        if (ep.bs) {
-          int L[4][8];
+      const uint32_t rec = st->rec_lh[h][u];
+      if (filt && rec) {
+        const EdgeParams ep = luma_edge(rec, sh, scale_y);
+        int L[4][8];
 #pragma unroll
-          for (int i = 0; i < 8; i++) { unpack2(raw[i].x, L[0][i], L[1][i]); unpack2(raw[i].y, L[2][i], L[3][i]); }
-          if (filter_luma_segment(L, ep, max_y)) {
+        for (int i = 0; i < 8; i++) { unpack2(raw[i].x, L[0][i], L[1][i]); unpack2(raw[i].y, L[2][i], L[3][i]); }
+        if (filter_luma_segment(L, ep, max_y)) {
 #pragma unroll
-            for (int i = 1; i < 7; i++) raw[i] = make_uint2(pack2(L[0][i], L[1][i]), pack2(L[2][i], L[3][i]));
-          }
+          for (int i = 1; i < 7; i++) raw[i] = make_uint2(pack2(L[0][i], L[1][i]), pack2(L[2][i], L[3][i]));
         }
       }
       const int x = x0 + 4 * u;
@@ -446,22 +527,20 @@ __global__ void __launch_bounds__(NTHREADS, ILF_DB_MIN_CTAS) deblock_kernel(Geom
     if (tid >= HC0 && tid < HC0 + 128 && !ctl_skip(sh.ctl, 1 + ((tid - HC0) >> 6))) {
       const int ht = tid - HC0;
       const int pl = ht >> 6, h = (ht >> 5) & 1, u = ht & 31;
-      const int16_t* sp = t.ch(pl, 8 * h, 2 * u);
+      const int16_t* sp = &st->c[pl][8 * h][2 * u + 8];
       uint32_t raw[8];
 #pragma unroll
       for (int i = 0; i < 8; i++) raw[i] = *reinterpret_cast<const uint32_t*>(sp + i * BCW);
-      if (filt) {
-        bool no_p, no_q;
-        const int tc = chroma_tc(t.cinfo(4 * h + 1, u), t.cinfo(4 * h, u), g, sh, false, pl, 2 * (cx0 + 2 * u), 2 * (cy0 + 2 + 8 * h), no_p, no_q);
-        if (tc >= 0) {
-          int a[4], b[4];
+      const uint32_t rec = (st->rec_ch[h][u] >> (16 * pl)) & 0xFFFFu;
+      if (filt && rec) {
+        const int tc = sh.tc[rec >> 3] * scale_c;
+        int a[4], b[4];
 #pragma unroll
-          for (int i = 0; i < 4; i++) unpack2(raw[i], a[i], b[i]);
-          const int da = clip3i(-tc, tc, (((a[2] - a[1]) << 2) + a[0] - a[3] + 4) >> 3);
-          const int db = clip3i(-tc, tc, (((b[2] - b[1]) << 2) + b[0] - b[3] + 4) >> 3);
-          if (!no_p) raw[1] = pack2(clip3i(0, max_c, a[1] + da), clip3i(0, max_c, b[1] + db));
-          if (!no_q) raw[2] = pack2(clip3i(0, max_c, a[2] - da), clip3i(0, max_c, b[2] - db));
-        }
+        for (int i = 0; i < 4; i++) unpack2(raw[i], a[i], b[i]);
+        const int da = clip3i(-tc, tc, (((a[2] - a[1]) << 2) + a[0] - a[3] + 4) >> 3);
+        const int db = clip3i(-tc, tc, (((b[2] - b[1]) << 2) + b[0] - b[3] + 4) >> 3);
+        if (!(rec & 2)) raw[1] = pack2(clip3i(0, max_c, a[1] + da), clip3i(0, max_c, b[1] + db));
+        if (!(rec & 4)) raw[2] = pack2(clip3i(0, max_c, a[2] - da), clip3i(0, max_c, b[2] - db));
       }
       const int x = cx0 + 2 * u;
       if (x < cw) {
@@ -497,12 +576,12 @@ __global__ void __launch_bounds__(NTHREADS, ILF_DB_MIN_CTAS) deblock_kernel(Geom
 
 }  // namespace
 
-template <int MV>
-static void launch_deblock_mv(const Geom& g, const SlotDev* slots, int first_slot, int num_slots, const BatchCtl& ctl, int* work, cudaStream_t st) {
+// work: two ints in device memory, zero before the first launch and owned by the launching stream (the kernel leaves them zero).
+void launch_deblock(const Geom& g, const SlotDev* slots, int first_slot, int num_slots, const BatchCtl& ctl, int* work, cudaStream_t st) {
   static const int pad = env_int("ILF_DB_SMEM_PAD");
-  const int smem = DB_STAGES * stage_stride<MV>() + DB_STAGES * 8 + (int)sizeof(DbShared) + pad;
+  const int smem = DB_STAGES * DB_STRIDE + DB_STAGES * 8 + (int)sizeof(DbShared) + pad;
   static bool attr_set[64] = {};
-  once_per_device(attr_set, [&] { cudaFuncSetAttribute(deblock_kernel<MV>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem); });
+  once_per_device(attr_set, [&] { cudaFuncSetAttribute(deblock_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem); });
   const int bands = (g.rows + 4 + TH - 1) / TH, ntx = (g.width + TW - 1) / TW;
   const long long total = (long long)ntx * bands * num_slots;
   // CTAs drawing tiles from the queue: the resident ones plus a fifth.  Exactly the resident number starves the kernel when
@@ -510,22 +589,26 @@ static void launch_deblock_mv(const Geom& g, const SlotDev* slots, int first_slo
   // non-empty only runs its prologue at the end of the launch (twice the resident number: 0.275 ms; 800 - 1000 CTAs: 0.271 ms).
   static const int ctas = env_int("ILF_DB_CTAS", 148 * (ILF_DB_MIN_CTAS + 1));
   dim3 grid((unsigned)std::min<long long>(total, ctas));
-  launch_pdl(deblock_kernel<MV>, grid, dim3(NTHREADS), smem, st, g, slots, first_slot, ctl, num_slots, work);
+  launch_pdl(deblock_kernel, grid, dim3(NTHREADS), smem, st, g, slots, first_slot, ctl, num_slots, work);
 }
 
-// work: two ints in device memory, zero before the first launch and owned by the launching stream (the kernel leaves them zero).
-void launch_deblock(const Geom& g, const SlotDev* slots, int first_slot, int num_slots, const BatchCtl& ctl, int mv_mode, int* work, cudaStream_t st) {
-  if (mv_mode == 0) launch_deblock_mv<0>(g, slots, first_slot, num_slots, ctl, work, st);
-  else if (mv_mode == 1) launch_deblock_mv<1>(g, slots, first_slot, num_slots, ctl, work, st);
-  else launch_deblock_mv<2>(g, slots, first_slot, num_slots, ctl, work, st);
+void launch_deblock_records(const Geom& g, const ilf_deblock_params* params, const uint32_t* info, const uint32_t* info_c, const int16_t* mv16,
+                            const int32_t* mv32, const uint8_t* ctu_slice, void* rec, cudaStream_t st) {
+  const DbRecLayout L = db_rec_layout(g);
+  const Grid grid = {info, info_c, mv16, mv32, g.units_w, g.units_h, g.units_pitch};
+  int most = 0;
+  for (int k = 0; k < DB_REC_KINDS; k++) most = std::max(most, L.cols[k] * L.rows[k]);
+  const dim3 blocks((unsigned)std::min(std::max(1, (most + 255) / 256), 148 * 8), DB_REC_KINDS);
+  deblock_records_kernel<<<blocks, 256, 0, st>>>(g, grid, params, ctu_slice, L, static_cast<unsigned char*>(rec));
 }
 
 // ---------------------------------------------------------------------------------------------------------------------------
-// Deblocking offset search (ilf_deblock_search; EncGOP::applyDeblockingFilterParameterSelection).  The same tiles, boxes and
-// device functions as deblock_kernel, but a tile is deblocked K times, once per (beta, tc) offset candidate, and nothing is
+// Deblocking offset search (ilf_deblock_search; EncGOP::applyDeblockingFilterParameterSelection).  The same tiles and device
+// functions as deblock_kernel, but a tile is deblocked K times, once per (beta, tc) offset candidate, and nothing is
 // stored: the horizontal-pass tasks compare their filtered block with the original and only sums of squared differences leave.
-//   - per tile, what does not depend on the offsets (edge flag, bS, QP, no-filter sides, chroma QP) is derived once into a
-//     compact record per segment; a thread owns the same four segments (one per phase) for every candidate, so the records stay
+//   - the slot's edge records have the slice offsets applied, so the stage carries the unit grid and the motion vectors instead
+//     (one launch per motion-vector representation), and per tile what does not depend on the offsets (edge flag, bS, QP,
+//     no-filter sides, chroma QP) is derived once into a compact record per segment; a thread owns the same four segments (one per phase) for every candidate, so the records stay
 //     in its registers, and so does the horizontal-pass task's block of the original;
 //   - per candidate: the staged samples are copied into a work buffer (two buffers alternate, so the copy of candidate k + 1 needs
 //     no barrier behind the horizontal pass of k), vertical edges, a barrier, horizontal edges + distortion;
@@ -568,18 +651,6 @@ template <int MV> __host__ __device__ constexpr int search_smem() {
   return stage_stride<MV>() + 2 * (int)sizeof(SearchWork) + (int)sizeof(SearchShared);
 }
 
-// Offset-independent part of a luma segment (luma_edge_params up to the tables): 0 = not filtered, else
-// bS | no_p << 2 | no_q << 3 | (QP & 0xFF) << 8.
-template <int MV>
-__device__ __forceinline__ uint32_t luma_edge_record(const Tile<MV>& t, int thr, int qr, int qc, int pr, int pc, bool vertical) {
-  const uint32_t iq = t.info(qr, qc), ip = t.info(pr, pc);
-  if (!(iq & (vertical ? ILF_BI_EDGE_V : ILF_BI_EDGE_H))) return 0;
-  const int bs = boundary_strength<MV>(t, iq, ip, qr, qc, pr, pc, vertical ? ILF_BI_TU_V : ILF_BI_TU_H, thr);
-  if (!bs) return 0;
-  const int qp = ((int)(int8_t)(ip >> 8) + (int)(int8_t)(iq >> 8) + 1) >> 1;
-  return (uint32_t)bs | ((ip & ILF_BI_NOFILT) ? 4u : 0u) | ((iq & ILF_BI_NOFILT) ? 8u : 0u) | ((uint32_t)(qp & 0xFF) << 8);
-}
-
 // tc / beta of a luma record under one candidate's offsets (LoopFilter.cpp:626-634).
 __device__ __forceinline__ EdgeParams luma_edge_apply(uint32_t rec, const SearchShared& sh, int beta_off, int tc_off, int scale) {
   EdgeParams ep;
@@ -590,17 +661,6 @@ __device__ __forceinline__ EdgeParams luma_edge_apply(uint32_t rec, const Search
   ep.no_p = (rec & 4) != 0;
   ep.no_q = (rec & 8) != 0;
   return ep;
-}
-
-// Offset-independent part of a chroma segment (chroma_tc up to the table): 0 = not filtered, else
-// 1 | no_p << 1 | no_q << 2 | (chroma QP after the mapping) << 16.
-__device__ __forceinline__ uint32_t chroma_edge_record(uint32_t iq, uint32_t ip, const SearchShared& sh, bool vertical, int comp) {
-  if (!(iq & (vertical ? ILF_BI_EDGE_V : ILF_BI_EDGE_H))) return 0;
-  if (!((iq | ip) & ILF_BI_INTRA)) return 0;
-  int qp = (((int)(int8_t)(ip >> 8) + (int)(int8_t)(iq >> 8) + 1) >> 1) + (comp == 0 ? sh.prm.cb_qp_offset : sh.prm.cr_qp_offset);
-  if (qp >= 70) qp -= 6;
-  else if (qp >= 0) qp = sh.chroma_scale[qp];
-  return 1u | ((ip & ILF_BI_NOFILT) ? 2u : 0u) | ((iq & ILF_BI_NOFILT) ? 4u : 0u) | ((uint32_t)qp << 16);
 }
 
 __device__ __forceinline__ int chroma_edge_tc(uint32_t rec, const SearchShared& sh, int tc_off, int bd_chroma) {
@@ -761,11 +821,11 @@ __global__ void __launch_bounds__(SEARCH_THREADS, SEARCH_MIN_CTAS) deblock_searc
     uint32_t rec_lv = 0, rec_cv = 0, rec_lh = 0, rec_ch = 0;
     const int ev = tid < 128 ? (tid & 15) : 16, sgv = tid < 128 ? (tid >> 4) : tid - 128;    // luma vertical task (tid < 136)
     const int plv = tid < 128 ? (tid >> 6) : ((tid - 128) >> 3), kv = tid < 128 ? ((tid >> 3) & 7) : 8, sgc = tid & 7;   // chroma vertical (tid < 144)
-    if (tid < 17 * 8) rec_lv = luma_edge_record<MV>(t, thr, sgv, 2 * ev, sgv, 2 * ev - 1, true);
-    if (tid < 2 * 9 * 8) rec_cv = chroma_edge_record(t.cinfo(sgc, 4 * kv), t.cinfo(sgc, 4 * kv - 1), sh, true, plv);
+    if (tid < 17 * 8) rec_lv = luma_edge_record(t, thr, sgv, 2 * ev, sgv, 2 * ev - 1, true);
+    if (tid < 2 * 9 * 8) rec_cv = chroma_edge_record(t.cinfo(sgc, 4 * kv), t.cinfo(sgc, 4 * kv - 1), sh.prm, sh.chroma_scale, true, plv);
     if (tid < 128) {
-      rec_lh = luma_edge_record<MV>(t, thr, 2 * h + 1, u, 2 * h, u, false);
-      rec_ch = chroma_edge_record(t.cinfo(4 * hc + 1, u), t.cinfo(4 * hc, u), sh, false, pl);
+      rec_lh = luma_edge_record(t, thr, 2 * h + 1, u, 2 * h, u, false);
+      rec_ch = chroma_edge_record(t.cinfo(4 * hc + 1, u), t.cinfo(4 * hc, u), sh.prm, sh.chroma_scale, false, pl);
     }
     if (!__syncthreads_or((int)(rec_lv | rec_cv | rec_lh | rec_ch))) {
       // nothing in the tile is filtered under any candidate: measure the staged samples once
